@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- consistency-loss pixels/s (fwd+bwd) of the Deep Co-Training unlabeled-branch hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one synthetic unlabeled batch (BASELINE.json configs[1]:
 ACDC co-training, K=3 views, C=4 classes, 256x256, batch 32 per GPU, JSD + VAT adversarial):
@@ -187,7 +187,7 @@ def time_cpu(K, C, B, H, W, cin, steps, warmup, with_vat=True, budget_s=None):
 
 
 def reference_staged():
-    """The unmodified reference (baseline/_ref, staged by tools/stage_reference.sh; /root/reference in the build container)."""
+    """The unmodified reference ($DCT_REFERENCE_ROOT, or baseline/_ref staged by tools/stage_reference.sh), if present."""
     try:
         import ref_trainer
         return ref_trainer if ref_trainer.available() else None
@@ -242,6 +242,39 @@ def run_reference(args, wl):
 # ---------------------------------------------------------------------------------------------------
 # GPU arm
 # ---------------------------------------------------------------------------------------------------
+DUMP_BYTES = 48 << 20   # per-pixel outputs are sampled down to this many bytes in all (the rest is a few KB)
+
+
+def dump_outputs(path, step, bufs):
+    """Write what one step left in ``bufs`` -- the arrays a caller of the step receives -- as ``path/<name>.npy``.
+
+    Losses, raw loss sums and Dice counts are written whole.  The per-pixel outputs (gradients, the VAT direction,
+    r_adv, img_adv) are written whole as [B, C, H, W] when they fit DUMP_BYTES together, else as [P, C] rows at P pixels
+    drawn once with a fixed seed (same pixels for every output; ``pixel_index.npy`` holds their flat b*H*W + h*W + w).
+    Integer outputs are stored as float64 (exact)."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    small = {"losses": torch.stack(step.losses(bufs)), "loss_sums": bufs.sums}
+    pix = {f"grad_logits{k}": g for k, g in enumerate(bufs.grad_logits)}
+    if step.with_dice:
+        small["dice_counts"] = bufs.dice_counts.double()
+    if step.with_vat:
+        pix.update(vat_direction=bufs.d, r_adv=bufs.r_adv, img_adv=bufs.img_adv, grad_yhat=bufs.grad_yhat,
+                   grad_adv=bufs.grad_adv)
+    B, _, H, W = bufs.logits[0].shape
+    n = B * H * W
+    per_pixel = sum(t.shape[1] * t.element_size() for t in pix.values())
+    P = min(n, DUMP_BYTES // per_pixel)
+    if P < n:
+        idx = np.sort(np.random.default_rng(20240).choice(n, size=P, replace=False))
+        small["pixel_index"] = torch.from_numpy(idx.astype(np.float64))
+        di = torch.from_numpy(idx).to(bufs.logits[0].device)
+        pix = {k: t.permute(0, 2, 3, 1).reshape(n, t.shape[1]).index_select(0, di) for k, t in pix.items()}
+    for name, t in {**small, **pix}.items():
+        np.save(os.path.join(path, name + ".npy"), t.detach().cpu().numpy())
+
+
 def use_nccl_later(world, px):
     return world > 1 and px is None
 
@@ -384,6 +417,8 @@ def run_ours(args, wl):
     if world > 1:
         dist.barrier()
     torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:   # before anything below runs the step again on these buffers
+        dump_outputs(args.dump_outputs, step, sets[(args.steps - 1) % R])
     ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -789,7 +824,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true",
                     help="skip aten_gpu_baseline / cotrain_it_s / other_workloads (developer A/B runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of the last timed step (rank 0) as DIR/<name>.npy; "
+                         "the same arguments give the same inputs, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, wl)

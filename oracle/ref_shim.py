@@ -1,11 +1,11 @@
 """Import shim for the upstream reference (TEST INFRASTRUCTURE ONLY).
 
-Makes ``import generalframework`` work in the build container, where the
-reference lives read-only at /root/reference and several of its eager imports
-(skimage, tensorboardX, visdom, matplotlib) are absent.  Nothing under
-/root/reference is modified.  This file is only used by
-``oracle/make_golden.py`` and by CPU tests that are skipped when the reference
-tree is not mounted (it never exists on the GPU box).
+Makes ``import generalframework`` work from a read-only copy of the original
+project's source tree, where several of its eager imports (skimage,
+tensorboardX, visdom, matplotlib) may be absent.  Nothing in that tree is
+modified.  This file is only used by ``oracle/make_golden*.py``, by
+``oracle/ref_trainer.py`` and by tests that are skipped when the tree is not
+found (the repository does not contain it).
 
 Why each stub is needed (reference file:line):
   generalframework/utils/__init__.py:1-2  -> utils/utils.py:16 (skimage.io.imsave)
@@ -14,8 +14,8 @@ Why each stub is needed (reference file:line):
   generalframework/utils/utils.py:318,342 + dataset/augment.py:141 (collections.Mapping...)
   generalframework/trainer/mean_teacher_trainer.py:10 (easydict; only when the package is absent)
 
-Where the reference is looked for: $DCT_REFERENCE_ROOT, else /root/reference (the build container), else
-<repo>/baseline/_ref (a staged copy that travels to the GPU box; tools/stage_reference.sh).
+Where the reference is looked for: $DCT_REFERENCE_ROOT, else <repo>/baseline/_ref (a staged copy;
+tools/stage_reference.sh).
 """
 import collections
 import collections.abc
@@ -27,11 +27,11 @@ _REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _find_root() -> str:
-    cands = [os.environ.get("DCT_REFERENCE_ROOT"), "/root/reference", os.path.join(_REPO, "baseline", "_ref")]
+    cands = [os.environ.get("DCT_REFERENCE_ROOT"), os.path.join(_REPO, "baseline", "_ref")]
     for c in cands:
         if c and os.path.isdir(os.path.join(c, "generalframework")):
             return c
-    return cands[0] or "/root/reference"
+    return cands[0] or cands[1]
 
 
 REFERENCE_ROOT = _find_root()

@@ -12,8 +12,8 @@ hard-coded 300 iterations through the module-global ``tqdm_`` and records, witho
   * the tensors ``_train_loop`` returns,
   * wall time per iteration (device-synchronised).
 
-The reference is found through ``oracle/ref_shim.py``: /root/reference in the build container, ``baseline/_ref`` (staged by
-``tools/stage_reference.sh``) on the GPU box.
+The reference is found through ``oracle/ref_shim.py``: ``$DCT_REFERENCE_ROOT``, else ``baseline/_ref`` (staged by
+``tools/stage_reference.sh``).
 """
 import os
 import sys

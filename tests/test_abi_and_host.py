@@ -6,9 +6,14 @@ import re
 
 import numpy as np
 import pytest
+import ref_shim
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+# the original project's source tree is not part of this repository: oracle/ref_shim.py finds it through
+# $DCT_REFERENCE_ROOT or a copy staged into baseline/_ref (tools/stage_reference.sh)
+needs_reference = pytest.mark.skipif(not ref_shim.reference_available(),
+                                     reason="original project's source tree not found ($DCT_REFERENCE_ROOT or baseline/_ref)")
 
 
 def _header_symbols():
@@ -147,7 +152,7 @@ def test_meter_host_logic_matches_reference_structures():
     assert v["Validated_Mean_IoU"] == np.mean([5 / 8, 3 / 6])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/generalframework"), reason="reference tree not mounted")
+@needs_reference
 def test_install_rebinds_reference_call_sites():
     import ref_shim
     ref_shim.install()
@@ -171,7 +176,7 @@ def test_install_rebinds_reference_call_sites():
     assert gl.LOSS["jsd"] is orig and ct.DiceMeter is not dct_b200.DiceMeter
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/generalframework"), reason="reference tree not mounted")
+@needs_reference
 def test_install_keeps_the_metrics2_flavour():
     """generalframework.metrics2.DiceMeter (user: trainer/mean_teacher_trainer.py:18) differs from metrics.DiceMeter on the
     host side (metrics2/dice_meter.py:43,82-84); install() must hand each module its own flavour and uninstall() must
