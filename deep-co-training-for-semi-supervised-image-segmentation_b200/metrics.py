@@ -6,10 +6,15 @@ Mirrors ``generalframework/metrics`` of the reference:
   ConfusionMatrix  metrics/confusionmatrix.py:7-98
   IoU              metrics/iou.py:8-113
 
+plus ``hausdorff`` / ``HausdorffMeter``: the Hausdorff distance Summary.py:25 takes from the external ``deepclustering``
+package, with the definition of ``medpy.metric.binary.hd`` (exact distance transforms on the device).
+
 ``add`` never leaves the device (no one-hot tensors, no ``torch.unique(a.cpu())``, no numpy
 ``bincount``); ``value()`` / ``summary()`` keep the reference's return structures.  Counts are exact
 int64; ``conf`` is exposed as the reference's ``np.int32`` view.
 """
+import ctypes
+
 import numpy as np
 import torch
 
@@ -174,6 +179,122 @@ class DiceMeter2(DiceMeter):
     def summary(self) -> dict:
         _, (means, _) = self.value()
         return {f'DSC{i}': means[i].item() for i in self.report_axis}
+
+
+def _class_map(t, C, what):
+    """int64 ``[B,H,W]`` class map from an integer ``[B,H,W]`` / ``[B,1,H,W]`` tensor."""
+    _runtime.require_cuda(t, what)
+    if t.is_floating_point():
+        raise TypeError(f"{what}: integer class map expected, got {t.dtype}")
+    if t.dim() == 4 and t.shape[1] == 1:
+        t = t[:, 0]
+    assert t.dim() == 3, f"{what}: class map [B,H,W] or [B,1,H,W] expected, got {tuple(t.shape)}"
+    return t.to(torch.int64).contiguous()
+
+
+def hausdorff(pred, gt, C=None, method='2d', voxelspacing=None) -> torch.Tensor:
+    """Hausdorff distance per class, float32 ``[rows, C]`` on the input's device (``rows`` = B for ``'2d'``, 1 for ``'3d'``).
+
+    Definition of ``medpy.metric.binary.hd`` (the ACDC challenge's evaluation code; the reference's Summary.py:25 gets the
+    metric from the external ``deepclustering`` package): the largest distance from a border pixel of ``{pred == c}`` to the
+    border of ``{gt == c}`` and back, borders taken with the cross structuring element and the grid's outside as
+    background, distances scaled by ``voxelspacing``.  ``'2d'`` measures every slice ``[H,W]`` on its own; ``'3d'`` measures
+    the batch as one ``[B,H,W]`` volume (under ``PatientSampler`` one batch is one patient).  A class absent from ``pred``
+    or ``gt`` gives NaN (medpy raises there).
+
+    ``pred``: float32 scores ``[B,C,H,W]`` -- reduced to a class map with the arg-max ``DiceMeter.add`` uses, so the Dice and
+    the HD of one batch describe the same segmentation -- or an integer class map ``[B,H,W]`` / ``[B,1,H,W]`` (e.g.
+    ``ensemble.vote_class(...)``; then ``C`` is required).  ``gt``: integer ``[B,H,W]`` / ``[B,1,H,W]``.
+    ``voxelspacing``: ``(sy, sx)`` for ``'2d'``, ``(sz, sy, sx)`` for ``'3d'``, ``None`` = ones.  Values outside ``[0, C)``
+    belong to no class and raise the label / prediction range checks under the current check mode.
+    """
+    assert method in ('2d', '3d')
+    if pred.is_floating_point():
+        from .utils import _classmap
+        assert pred.dim() == 4, f"hausdorff: scores [B,C,H,W] expected, got {tuple(pred.shape)}"
+        if pred.dtype != torch.float32:
+            raise TypeError(f"hausdorff: float32 scores expected, got {pred.dtype}")
+        assert C is None or C == pred.shape[1], f"C={C} does not match scores {tuple(pred.shape)}"
+        C = pred.shape[1]
+        p = _classmap(pred.detach(), 1, want_cls=True)[0]
+    else:
+        assert C is not None, "hausdorff: C is required for an integer class map"
+        p = _class_map(pred, C, "hausdorff")
+    g = _class_map(gt, C, "hausdorff")
+    assert g.shape == p.shape, f"label shape {tuple(gt.shape)} does not match prediction {tuple(pred.shape)}"
+    B, H, W = p.shape
+    volume = method == '3d'
+    sp = None
+    if voxelspacing is not None:
+        vals = [float(v) for v in voxelspacing]
+        assert len(vals) == (3 if volume else 2), f"voxelspacing for '{method}' has {3 if volume else 2} values, got {vals}"
+        sp = (ctypes.c_double * len(vals))(*vals)
+    h = _lib.lib()
+    nbytes = h.dct_hausdorff_scratch_bytes(C, B, H, W, int(volume))
+    if nbytes == 0:
+        _lib.check(_lib.ERR_UNSUPPORTED, f"dct_hausdorff_scratch_bytes (C={C}, shape {(B, H, W)})")
+    scratch = torch.empty(nbytes, dtype=torch.uint8, device=p.device)
+    out = torch.empty((1 if volume else B, C), dtype=torch.float32, device=p.device)
+    st = _runtime.state(p.device)
+    _lib.check(h.dct_hausdorff_i64(p.data_ptr(), g.data_ptr(), C, B, H, W, int(volume), sp, out.data_ptr(),
+                                   _runtime.flags_ptr(st), scratch.data_ptr(), _runtime.stream_ptr(p.device)),
+               "dct_hausdorff_i64")
+    _runtime.after_call(st)
+    return out
+
+
+def _nan_mean_std(x: torch.Tensor, dim: int):
+    """Mean and unbiased standard deviation along ``dim`` over the non-NaN entries (NaN where fewer than 1 / 2 remain)."""
+    valid = ~torch.isnan(x)
+    n = valid.sum(dim)
+    mean = torch.nanmean(x, dim)
+    dev = torch.where(valid, x - mean.unsqueeze(dim), torch.zeros_like(x))
+    var = (dev * dev).sum(dim) / (n - 1)
+    return mean, torch.where(n > 1, var.sqrt(), torch.full_like(var, float('nan')))
+
+
+class HausdorffMeter(Metric):
+    """Hausdorff distance per class next to ``DiceMeter`` (same ``method`` / ``report_axises`` / ``C``; definition of
+    ``medpy.metric.binary.hd``, see ``hausdorff``).  ``add`` appends one row per image (``'2d'``) or per batch
+    (``'3d'``); the statistics skip the NaN of classes absent from a prediction or a label."""
+
+    def __init__(self, method='2d', report_axises='all', C=4) -> None:
+        super().__init__()
+        assert method in ('2d', '3d')
+        assert report_axises == 'all' or isinstance(report_axises, list)
+        self.method = method
+        self.report_axis = report_axises
+        self.C = C
+        self.hdLog = []
+
+    def reset(self):
+        self.hdLog = []
+
+    def add(self, pred, gt, voxelspacing=None):
+        self.hdLog.append(hausdorff(pred, gt, C=self.C, method=self.method, voxelspacing=voxelspacing))
+
+    @property
+    def log(self):
+        if len(self.hdLog) == 0:
+            return torch.full((1, self.C), float('nan'))
+        return torch.cat(self.hdLog)
+
+    def value(self, **kwargs):
+        """``((mean, std), (means[C], stds[C]))``: per class over the rows, and of the per-row mean over the report
+        axes; NaN entries skipped, unbiased standard deviations."""
+        log = self.log
+        means, stds = _nan_mean_std(log, 0)
+        axes = log if self.report_axis == 'all' else log[:, self.report_axis]
+        report_mean, report_std = _nan_mean_std(torch.nanmean(axes, 1), 0)
+        return (report_mean, report_std), (means, stds)
+
+    def detailed_summary(self) -> dict:
+        _, (means, _) = self.value()
+        return {f'HD{i}': means[i].item() for i in range(len(means))}
+
+    def summary(self) -> dict:
+        (mean, var), _ = self.value()
+        return {'mHD': mean.item(), 'mHDVars': var.item()}
 
 
 class ConfusionMatrix(Metric):

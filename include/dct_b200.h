@@ -359,6 +359,31 @@ DCT_API int dct_vote_f32(const float* const* views, int K, int C, int64_t B, int
                          int64_t* cls, uint8_t* cls_u8, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Boundary distance (evaluation path, Summary.py:25: the reference reports the Hausdorff distance of every view and
+ * ensemble through the external deepclustering package).  Definition: medpy.metric.binary.hd, the ACDC challenge's
+ * evaluation code.  Per class c on a grid -- one H x W slice (volume == 0) or the whole batch as one B x H x W volume
+ * (volume != 0; DiceMeter's '2d' / '3d') -- with A = {pred == c}, G = {labels == c}:
+ *   border(M) = M xor binary_erosion(M), cross structuring element (4 / 6 neighbours), off-grid cells are background;
+ *   d(x, S)   = min over y in S of ||(x - y) * spacing||_2, spacing (sy, sx) or (sz, sy, sx) along the tensor axes;
+ *   hd        = max(max over border(A) of d(., border(G)), max over border(G) of d(., border(A))); NaN if A or G is empty.
+ * Values outside [0,C) belong to no class (a non-c neighbour for every c) and are counted in flags[DCT_FLAG_PRED]
+ * (pred) / flags[DCT_FLAG_LABEL] (labels).  Exact separable Euclidean distance transforms of the 2C border sets:
+ * 4 launches for a slice batch, 5 for a volume; no host synchronisation.  At unit spacing hd is the correctly rounded
+ * square root of the exact squared distance (while that stays below 2^24).
+ * Limits (DCT_ERR_UNSUPPORTED): C <= DCT_MAX_CLASSES; H, W (and B when volume != 0) <= 32768 (each line's envelope stack
+ * keeps 16-bit positions); 2*C*B*max(H,W) (and 2*C*H*W for a volume) <= 2^31 - 1.
+ * ------------------------------------------------------------------------------------------ */
+
+/* bytes of `scratch` dct_hausdorff_i64 needs for this shape (about 4*C + 2 bytes per pixel, 12*C + 2 for a volume);
+ * 0 for a shape it rejects.  Host only. */
+DCT_API size_t dct_hausdorff_scratch_bytes(int C, int64_t B, int64_t H, int64_t W, int volume);
+/* pred, labels int64 [B,H,W]; spacing: HOST array of 2 (volume == 0) or 3 positive finite values, NULL = all ones;
+ * hd float32 [volume ? 1 : B][C], overwritten; scratch: >= dct_hausdorff_scratch_bytes() bytes, 256-byte aligned, no
+ * initial state required, private to the call until the stream reaches its end. */
+DCT_API int dct_hausdorff_i64(const int64_t* pred, const int64_t* labels, int C, int64_t B, int64_t H, int64_t W,
+                              int volume, const double* spacing, float* hd, int32_t* flags, void* scratch, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * bfloat16 twins of the one-pass-over-logits entry points (networks under torch.autocast emit bf16 logits;
  * north_star: "within 1e-2 relative in bf16").  Tensors [B,C,HW] are bfloat16 (2-byte elements, same NCHW
  * layout), gradients are written as bfloat16 (round-to-nearest-even); ALL arithmetic is fp32 in registers and the
