@@ -85,6 +85,7 @@ struct CeArgs {
     Upstream up;
     int32_t* flags;
     Workspace* ws;
+    int64_t B;          // ce_launch_rt: images b = blockIdx.y, blockIdx.y + gridDim.y, ... (image_grid)
 };
 
 // Correctness path for shapes the tile pipeline does not take (C outside {2,3,4,19}, odd HW, misaligned pointers):
@@ -93,38 +94,39 @@ template <bool GRAD>
 __global__ void __launch_bounds__(256) ce_kernel_rt(const CeArgs a) {
     const int C = a.C;
     const int64_t HW = a.HW;
-    const int b = blockIdx.y;
     float gs = 1.0f;
     if constexpr (GRAD) gs = upstream_scalar(a.up);
     double acc = 0.0;
     int nbad = 0;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < HW; i += (int64_t)gridDim.x * blockDim.x) {
-        const float* xb = a.x + (int64_t)b * C * HW + i;
-        const long long t = a.labels[(int64_t)b * HW + i];
-        const bool valid = t >= 0 && t < C, ign = t == a.ignore_index;
-        nbad += (!valid) & (!ign);
-        const bool use = valid & !ign;
-        const float w = use ? (a.class_w != nullptr ? __ldg(a.class_w + t) : 1.0f) : 0.0f;
-        float mx = xb[0];
-        for (int c = 1; c < C; ++c) mx = fmaxf(mx, xb[(int64_t)c * HW]);
-        float Z = 0.0f, sel = 0.0f;
-        for (int c = 0; c < C; ++c) {
-            const float tt = fmaf(xb[(int64_t)c * HW], kLog2e, -mx * kLog2e);
-            Z += ex2_ftz(tt);
-            if (use && c == (int)t) sel = tt;
-        }
-        const float lZ = lg2_ftz(Z);
-        const float loss = use ? w * ((lZ - sel) * kLn2) : 0.0f;
-        acc += (double)loss;
-        if (a.map != nullptr) a.map[(int64_t)b * HW + i] = loss;
-        if constexpr (GRAD) {
-            float g = gs * w;
-            if (a.up.gmap != nullptr) g *= a.up.gmap[(int64_t)b * HW + i];
-            const float inv = rcp_ftz(Z);
-            float* gb = a.grad + (int64_t)b * C * HW + i;
+    for (int64_t b = blockIdx.y; b < a.B; b += gridDim.y) {
+        for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < HW; i += (int64_t)gridDim.x * blockDim.x) {
+            const float* xb = a.x + b * C * HW + i;
+            const long long t = a.labels[b * HW + i];
+            const bool valid = t >= 0 && t < C, ign = t == a.ignore_index;
+            nbad += (!valid) & (!ign);
+            const bool use = valid & !ign;
+            const float w = use ? (a.class_w != nullptr ? __ldg(a.class_w + t) : 1.0f) : 0.0f;
+            float mx = xb[0];
+            for (int c = 1; c < C; ++c) mx = fmaxf(mx, xb[(int64_t)c * HW]);
+            float Z = 0.0f, sel = 0.0f;
             for (int c = 0; c < C; ++c) {
-                const float p = ex2_ftz(fmaf(xb[(int64_t)c * HW], kLog2e, -mx * kLog2e)) * inv;
-                gb[(int64_t)c * HW] = use ? g * (p - ((int)t == c ? 1.0f : 0.0f)) : 0.0f;
+                const float tt = fmaf(xb[(int64_t)c * HW], kLog2e, -mx * kLog2e);
+                Z += ex2_ftz(tt);
+                if (use && c == (int)t) sel = tt;
+            }
+            const float lZ = lg2_ftz(Z);
+            const float loss = use ? w * ((lZ - sel) * kLn2) : 0.0f;
+            acc += (double)loss;
+            if (a.map != nullptr) a.map[b * HW + i] = loss;
+            if constexpr (GRAD) {
+                float g = gs * w;
+                if (a.up.gmap != nullptr) g *= a.up.gmap[b * HW + i];
+                const float inv = rcp_ftz(Z);
+                float* gb = a.grad + b * C * HW + i;
+                for (int c = 0; c < C; ++c) {
+                    const float p = ex2_ftz(fmaf(xb[(int64_t)c * HW], kLog2e, -mx * kLog2e)) * inv;
+                    gb[(int64_t)c * HW] = use ? g * (p - ((int)t == c ? 1.0f : 0.0f)) : 0.0f;
+                }
             }
         }
     }
@@ -157,6 +159,15 @@ static int ce_tile(const CeArgs& c, int64_t B, unsigned long long* counts, cudaS
     if (rc == DCT_ERR_UNSUPPORTED) return DCT_OK;  // not a tile shape: the caller falls back
     done = rc == DCT_OK;
     return rc;
+}
+
+template <bool GRAD>
+static int ce_launch_rt(CeArgs c, int64_t B, cudaStream_t s) {
+    c.B = B;
+    const dim3 grid = image_grid(B, c.HW, 256);
+    if (!fits_partials(grid)) return DCT_ERR_UNSUPPORTED;
+    ce_kernel_rt<GRAD><<<grid, 256, 0, s>>>(c);
+    return check_launch();
 }
 
 static int ce_check(const float* x, const int64_t* labels, int C, int64_t B, int64_t HW) {
@@ -219,8 +230,7 @@ extern "C" int dct_ce_fwd_f32(const float* logits, const int64_t* labels, int C,
     bool done;
     rc = ce_tile<CeOp<false, false, false>>(c, B, nullptr, s, done);
     if (rc != DCT_OK || done) return rc;
-    ce_kernel_rt<false><<<image_grid(B, HW, 256), 256, 0, s>>>(c);
-    return check_launch();
+    return ce_launch_rt<false>(c, B, s);
 }
 
 extern "C" int dct_ce_bwd_f32(const float* logits, const int64_t* labels, int C, int64_t B, int64_t HW,
@@ -236,8 +246,7 @@ extern "C" int dct_ce_bwd_f32(const float* logits, const int64_t* labels, int C,
     bool done;
     rc = ce_tile<CeOp<true, false, true>>(c, B, nullptr, s, done);
     if (rc != DCT_OK || done) return rc;
-    ce_kernel_rt<true><<<image_grid(B, HW, 256), 256, 0, s>>>(c);
-    return check_launch();
+    return ce_launch_rt<true>(c, B, s);
 }
 
 extern "C" int dct_ce_fwdbwd_f32(const float* logits, const int64_t* labels, int C, int64_t B, int64_t HW,
@@ -259,8 +268,7 @@ extern "C" int dct_ce_fwdbwd_f32(const float* logits, const int64_t* labels, int
     rc = ce_tile<CeOp<true, false, false>>(c, B, nullptr, s, done);
     if (rc != DCT_OK) return rc;
     if (!done) {
-        ce_kernel_rt<true><<<image_grid(B, HW, 256), 256, 0, s>>>(c);
-        rc = check_launch();
+        rc = ce_launch_rt<true>(c, B, s);
         if (rc != DCT_OK) return rc;
     }
     if (dice_counts != nullptr)  // Dice counting of the same logits in its own launch (C > 4 or a non-tile shape)

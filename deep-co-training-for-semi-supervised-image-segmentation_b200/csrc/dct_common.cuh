@@ -225,7 +225,8 @@ static __device__ __noinline__ void peer_publish(const double* src, unsigned lon
 
 // Deterministic grid-wide sum of one double per thread.  Every CTA writes its partial to the
 // workspace; the CTA that draws the last ticket adds the partials in index order and writes
-// *out, then re-arms the ticket.  `out` may be null (nothing is done).
+// *out, then re-arms the ticket.  `out` may be null (nothing is done).  num_ctas <= kMaxPartials
+// (image_grid + fits_partials on the host): a larger grid would write past `partials` into the l2 area.
 __device__ __forceinline__ void grid_sum_to(double v, Workspace* ws, double* out, int cta_linear, int num_ctas) {
     if (out == nullptr) return;
     __shared__ double s_warp[32];
@@ -351,16 +352,22 @@ __device__ __forceinline__ void tile_grid_finish(long long acc_fx, bool nonfinit
 // grid geometry: blockIdx.y = image b, blockIdx.x strides over the image's pixel groups, so a CTA
 // never straddles two images (per-image integer counts and per-sample norms stay CTA-local).
 // One pixel group per thread (thousands of small CTAs: the hardware block scheduler balances the
-// tail); B <= 65535 is checked by the callers.
+// tail); B <= 65535 is checked by the callers.  Every CTA of a grid_sum_to launch owns one of the
+// kMaxPartials partial-sum slots, so the grid never has more CTAs than that: for B > max_ctas,
+// gridDim.y = max_ctas and the kernels stride over images (b = blockIdx.y, blockIdx.y + gridDim.y, ...).
+// For B <= max_ctas that loop runs once and the grid is one row per image.
 // ---------------------------------------------------------------------------------------------
 inline dim3 image_grid(int64_t B, int64_t groups_per_image, int threads, int64_t max_ctas = kMaxPartials) {
+    const int64_t gy = B < 1 ? 1 : (B < max_ctas ? B : max_ctas);
     int64_t gx = (groups_per_image + threads - 1) / threads;  // one pixel group per thread ...
-    int64_t cap = max_ctas / (B > 0 ? B : 1);                  // ... unless that exceeds the partial-sum slots
-    if (cap < 1) cap = 1;
+    const int64_t cap = max_ctas / gy;                         // ... unless that exceeds the partial-sum slots (cap >= 1)
     if (gx > cap) gx = cap;                                    // then threads stride over the image
     if (gx < 1) gx = 1;
-    return dim3((unsigned)gx, (unsigned)B, 1);
+    return dim3((unsigned)gx, (unsigned)gy, 1);
 }
+
+// host-side guard in front of every launch that ends in grid_sum_to: one partial-sum slot per CTA
+inline bool fits_partials(dim3 grid) { return (int64_t)grid.x * grid.y * grid.z <= kMaxPartials; }
 
 // ---------------------------------------------------------------------------------------------
 // The pinned softmax arithmetic for the integer (Dice) path -- see DESIGN.md "Dice spec".

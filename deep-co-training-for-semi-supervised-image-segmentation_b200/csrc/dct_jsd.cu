@@ -10,9 +10,10 @@ static int jsd_launch_rt(const JsdCall& c) {
         a.in[k] = k < c.K ? c.views[k] : nullptr;
         a.grad[k] = (k < c.K && c.grads) ? c.grads[k] : nullptr;
     }
-    a.K = c.K; a.C = c.C; a.HW = c.HW; a.map = c.map; a.sum = c.sum; a.up = c.up; a.flags = c.flags; a.ws = c.ws;
+    a.K = c.K; a.C = c.C; a.B = c.B; a.HW = c.HW; a.map = c.map; a.sum = c.sum; a.up = c.up; a.flags = c.flags; a.ws = c.ws;
     const int threads = 256;
     dim3 grid = image_grid(c.B, c.HW, threads);
+    if (!fits_partials(grid)) return DCT_ERR_UNSUPPORTED;
 #define DCT_JSD_RT(LG, MD) jsd_kernel_rt<LG, MD><<<grid, threads, 0, c.stream>>>(a)
     if (c.in_kind == DCT_IN_LOGITS) {
         if (c.mode == kFwd) DCT_JSD_RT(true, kFwd);

@@ -21,7 +21,7 @@ enum JsdMode { kFwd = 0, kBwd = 1, kFwdBwd = 2 };
 template <int K>
 struct JsdArgs {
     Views<K> v;
-    int64_t HW;
+    int64_t B, HW;          // images b = blockIdx.y, blockIdx.y + gridDim.y, ... (image_grid)
     float* map;             // [B,HW] or null
     double* sum;            // or null
     Upstream up;            // kBwd: full upstream; kFwdBwd: gconst only
@@ -33,7 +33,7 @@ struct JsdArgsRt {          // runtime-(K,C) fallback
     const float* in[DCT_MAX_VIEWS];
     float* grad[DCT_MAX_VIEWS];
     int K, C;
-    int64_t HW;
+    int64_t B, HW;
     float* map;
     double* sum;
     Upstream up;
@@ -267,59 +267,60 @@ template <int K, int C, int VEC, bool LOGITS, int MODE, int MINB = 1>
 __global__ void __launch_bounds__(256, MINB) jsd_kernel(const JsdArgs<K> a) {
     const int64_t HW = a.HW;
     const int64_t gpi = HW / VEC;  // pixel groups per image (host guarantees HW % VEC == 0)
-    const int b = blockIdx.y;
-    const int64_t img = (int64_t)b * C * HW;
     float gs = 0.0f;
     if constexpr (MODE == kBwd) gs = upstream_scalar(a.up);
     if constexpr (MODE == kFwdBwd) gs = a.up.gconst;
     gs = div_by_K<K>(gs);
     double acc = 0.0;
     bool bad = false;
-    for (int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; g < gpi; g += (int64_t)gridDim.x * blockDim.x) {
-        const int64_t i = g * VEC;
-        FVec<VEC> xin[K][C];
-#pragma unroll
-        for (int k = 0; k < K; ++k)
-#pragma unroll
-            for (int c = 0; c < C; ++c) xin[k][c] = ld_stream<VEC>(a.v.in[k] + img + (int64_t)c * HW + i);
-        FVec<VEC> gm;
-        if constexpr (MODE == kBwd) {
-            if (a.up.gmap != nullptr) gm = ld_stream<VEC>(a.up.gmap + (int64_t)b * HW + i);
-            else {
-#pragma unroll
-                for (int v = 0; v < VEC; ++v) gm.v[v] = 1.0f;
-            }
-        }
-        FVec<VEC> mapv;
-        float part = 0.0f;
-#pragma unroll
-        for (int v = 0; v < VEC; ++v) {
-            float x[K][C];
+    for (int64_t b = blockIdx.y; b < a.B; b += gridDim.y) {
+        const int64_t img = b * C * HW;
+        for (int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; g < gpi; g += (int64_t)gridDim.x * blockDim.x) {
+            const int64_t i = g * VEC;
+            FVec<VEC> xin[K][C];
 #pragma unroll
             for (int k = 0; k < K; ++k)
 #pragma unroll
-                for (int c = 0; c < C; ++c) x[k][c] = xin[k][c].v[v];
-            float gK = gs;
-            if constexpr (MODE == kBwd) gK *= gm.v[v];
-            float j = jsd_pixel<K, C, LOGITS, MODE != kFwd, float>(x, gK, bad);
-            mapv.v[v] = j;
-            part += j;
+                for (int c = 0; c < C; ++c) xin[k][c] = ld_stream<VEC>(a.v.in[k] + img + (int64_t)c * HW + i);
+            FVec<VEC> gm;
+            if constexpr (MODE == kBwd) {
+                if (a.up.gmap != nullptr) gm = ld_stream<VEC>(a.up.gmap + b * HW + i);
+                else {
+#pragma unroll
+                    for (int v = 0; v < VEC; ++v) gm.v[v] = 1.0f;
+                }
+            }
+            FVec<VEC> mapv;
+            float part = 0.0f;
+#pragma unroll
+            for (int v = 0; v < VEC; ++v) {
+                float x[K][C];
+#pragma unroll
+                for (int k = 0; k < K; ++k)
+#pragma unroll
+                    for (int c = 0; c < C; ++c) x[k][c] = xin[k][c].v[v];
+                float gK = gs;
+                if constexpr (MODE == kBwd) gK *= gm.v[v];
+                float j = jsd_pixel<K, C, LOGITS, MODE != kFwd, float>(x, gK, bad);
+                mapv.v[v] = j;
+                part += j;
+                if constexpr (MODE != kFwd) {
+#pragma unroll
+                    for (int k = 0; k < K; ++k)
+#pragma unroll
+                        for (int c = 0; c < C; ++c) xin[k][c].v[v] = x[k][c];
+                }
+            }
+            acc += (double)part;
+            if constexpr (MODE != kBwd) {
+                if (a.map != nullptr) st_stream<VEC>(a.map + b * HW + i, mapv);
+            }
             if constexpr (MODE != kFwd) {
 #pragma unroll
                 for (int k = 0; k < K; ++k)
 #pragma unroll
-                    for (int c = 0; c < C; ++c) xin[k][c].v[v] = x[k][c];
+                    for (int c = 0; c < C; ++c) st_stream<VEC>(a.v.grad[k] + img + (int64_t)c * HW + i, xin[k][c]);
             }
-        }
-        acc += (double)part;
-        if constexpr (MODE != kBwd) {
-            if (a.map != nullptr) st_stream<VEC>(a.map + (int64_t)b * HW + i, mapv);
-        }
-        if constexpr (MODE != kFwd) {
-#pragma unroll
-            for (int k = 0; k < K; ++k)
-#pragma unroll
-                for (int c = 0; c < C; ++c) st_stream<VEC>(a.v.grad[k] + img + (int64_t)c * HW + i, xin[k][c]);
         }
     }
     if constexpr (MODE != kBwd) {
@@ -341,67 +342,36 @@ template <bool LOGITS, int MODE>
 __global__ void __launch_bounds__(256) jsd_kernel_rt(const JsdArgsRt a) {
     const int K = a.K, C = a.C;
     const int64_t HW = a.HW;
-    const int b = blockIdx.y;
-    const int64_t img = (int64_t)b * C * HW;
     const float invK = 1.0f / (float)K;
     float gs = 0.0f;
     if constexpr (MODE == kBwd) gs = upstream_scalar(a.up);
     if constexpr (MODE == kFwdBwd) gs = a.up.gconst;
     double acc = 0.0;
     bool bad = false;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < HW; i += (int64_t)gridDim.x * blockDim.x) {
-        float mx[DCT_MAX_VIEWS], inv[DCT_MAX_VIEWS], lZ[DCT_MAX_VIEWS], kl[DCT_MAX_VIEWS];
-        float hsum = 0.0f;
-#pragma unroll
-        for (int k = 0; k < DCT_MAX_VIEWS; ++k) {
-            mx[k] = 0.0f; inv[k] = 1.0f; lZ[k] = 0.0f; kl[k] = 0.0f;
-            if (k < K) {
-                const float* xb = a.in[k] + img + i;
-                if constexpr (LOGITS) {
-                    float m = xb[0];
-                    for (int c = 1; c < C; ++c) m = fmaxf(m, xb[(int64_t)c * HW]);
-                    float Z = 0.0f;
-                    for (int c = 0; c < C; ++c) Z += fexp(xb[(int64_t)c * HW] - m);
-                    mx[k] = m; inv[k] = fdiv(1.0f, Z); lZ[k] = flog(Z);
-                } else {
-                    float s = 0.0f;
-                    for (int c = 0; c < C; ++c) s += xb[(int64_t)c * HW];
-                    bad |= !simplex_ok(s);
-                }
-            }
-        }
-        float hm = 0.0f;
-        for (int c = 0; c < C; ++c) {
-            float s = 0.0f;
-            float pv[DCT_MAX_VIEWS], lp[DCT_MAX_VIEWS];
+    for (int64_t b = blockIdx.y; b < a.B; b += gridDim.y) {
+        const int64_t img = b * C * HW;
+        for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < HW; i += (int64_t)gridDim.x * blockDim.x) {
+            float mx[DCT_MAX_VIEWS], inv[DCT_MAX_VIEWS], lZ[DCT_MAX_VIEWS], kl[DCT_MAX_VIEWS];
+            float hsum = 0.0f;
 #pragma unroll
             for (int k = 0; k < DCT_MAX_VIEWS; ++k) {
-                pv[k] = 0.0f; lp[k] = 0.0f;
+                mx[k] = 0.0f; inv[k] = 1.0f; lZ[k] = 0.0f; kl[k] = 0.0f;
                 if (k < K) {
-                    float xv = a.in[k][img + (int64_t)c * HW + i];
-                    if constexpr (LOGITS) { float d = xv - mx[k]; pv[k] = fexp(d) * inv[k]; lp[k] = d - lZ[k]; }
-                    else { pv[k] = xv; lp[k] = flog(xv + kEntEps); }
-                    s = (k == 0) ? pv[k] : s + pv[k];
-                    hsum = fmaf(pv[k], lp[k], hsum);
+                    const float* xb = a.in[k] + img + i;
+                    if constexpr (LOGITS) {
+                        float m = xb[0];
+                        for (int c = 1; c < C; ++c) m = fmaxf(m, xb[(int64_t)c * HW]);
+                        float Z = 0.0f;
+                        for (int c = 0; c < C; ++c) Z += fexp(xb[(int64_t)c * HW] - m);
+                        mx[k] = m; inv[k] = fdiv(1.0f, Z); lZ[k] = flog(Z);
+                    } else {
+                        float s = 0.0f;
+                        for (int c = 0; c < C; ++c) s += xb[(int64_t)c * HW];
+                        bad |= !simplex_ok(s);
+                    }
                 }
             }
-            float m = ((K & (K - 1)) == 0) ? s * invK : s / (float)K;
-            float lm = flog(m + kEntEps);
-            hm = fmaf(m, lm, hm);
-#pragma unroll
-            for (int k = 0; k < DCT_MAX_VIEWS; ++k)
-                if (k < K) kl[k] = fmaf(pv[k], lp[k] - lm, kl[k]);
-        }
-        float hs = ((K & (K - 1)) == 0) ? hsum * invK : hsum / (float)K;
-        const float jsd = hs - hm;
-        acc += (double)jsd;
-        if constexpr (MODE != kBwd) {
-            if (a.map != nullptr) a.map[(int64_t)b * HW + i] = jsd;
-        }
-        if constexpr (MODE != kFwd) {
-            float g = gs;
-            if constexpr (MODE == kBwd) { if (a.up.gmap != nullptr) g *= a.up.gmap[(int64_t)b * HW + i]; }
-            float gK = ((K & (K - 1)) == 0) ? g * invK : g / (float)K;
+            float hm = 0.0f;
             for (int c = 0; c < C; ++c) {
                 float s = 0.0f;
                 float pv[DCT_MAX_VIEWS], lp[DCT_MAX_VIEWS];
@@ -413,18 +383,50 @@ __global__ void __launch_bounds__(256) jsd_kernel_rt(const JsdArgsRt a) {
                         if constexpr (LOGITS) { float d = xv - mx[k]; pv[k] = fexp(d) * inv[k]; lp[k] = d - lZ[k]; }
                         else { pv[k] = xv; lp[k] = flog(xv + kEntEps); }
                         s = (k == 0) ? pv[k] : s + pv[k];
+                        hsum = fmaf(pv[k], lp[k], hsum);
                     }
                 }
                 float m = ((K & (K - 1)) == 0) ? s * invK : s / (float)K;
                 float lm = flog(m + kEntEps);
+                hm = fmaf(m, lm, hm);
 #pragma unroll
                 for (int k = 0; k < DCT_MAX_VIEWS; ++k)
-                    if (k < K) {
-                        float gv;
-                        if constexpr (LOGITS) gv = gK * pv[k] * ((lp[k] - lm) - kl[k]);
-                        else gv = gK * ((lp[k] + fdiv(pv[k], pv[k] + kEntEps)) - (lm + fdiv(m, m + kEntEps)));
-                        a.grad[k][img + (int64_t)c * HW + i] = gv;
+                    if (k < K) kl[k] = fmaf(pv[k], lp[k] - lm, kl[k]);
+            }
+            float hs = ((K & (K - 1)) == 0) ? hsum * invK : hsum / (float)K;
+            const float jsd = hs - hm;
+            acc += (double)jsd;
+            if constexpr (MODE != kBwd) {
+                if (a.map != nullptr) a.map[(int64_t)b * HW + i] = jsd;
+            }
+            if constexpr (MODE != kFwd) {
+                float g = gs;
+                if constexpr (MODE == kBwd) { if (a.up.gmap != nullptr) g *= a.up.gmap[(int64_t)b * HW + i]; }
+                float gK = ((K & (K - 1)) == 0) ? g * invK : g / (float)K;
+                for (int c = 0; c < C; ++c) {
+                    float s = 0.0f;
+                    float pv[DCT_MAX_VIEWS], lp[DCT_MAX_VIEWS];
+#pragma unroll
+                    for (int k = 0; k < DCT_MAX_VIEWS; ++k) {
+                        pv[k] = 0.0f; lp[k] = 0.0f;
+                        if (k < K) {
+                            float xv = a.in[k][img + (int64_t)c * HW + i];
+                            if constexpr (LOGITS) { float d = xv - mx[k]; pv[k] = fexp(d) * inv[k]; lp[k] = d - lZ[k]; }
+                            else { pv[k] = xv; lp[k] = flog(xv + kEntEps); }
+                            s = (k == 0) ? pv[k] : s + pv[k];
+                        }
                     }
+                    float m = ((K & (K - 1)) == 0) ? s * invK : s / (float)K;
+                    float lm = flog(m + kEntEps);
+#pragma unroll
+                    for (int k = 0; k < DCT_MAX_VIEWS; ++k)
+                        if (k < K) {
+                            float gv;
+                            if constexpr (LOGITS) gv = gK * pv[k] * ((lp[k] - lm) - kl[k]);
+                            else gv = gK * ((lp[k] + fdiv(pv[k], pv[k] + kEntEps)) - (lm + fdiv(m, m + kEntEps)));
+                            a.grad[k][img + (int64_t)c * HW + i] = gv;
+                        }
+                }
             }
         }
     }
@@ -556,11 +558,12 @@ int jsd_launch_kc(const JsdCall& c) {
         a.v.grad[k] = c.grads ? c.grads[k] : nullptr;
         al = al && aligned(a.v.in[k], 4 * VEC) && (a.v.grad[k] == nullptr || aligned(a.v.grad[k], 4 * VEC));
     }
-    a.HW = c.HW; a.map = c.map; a.sum = c.sum; a.up = c.up; a.flags = c.flags; a.ws = c.ws;
+    a.B = c.B; a.HW = c.HW; a.map = c.map; a.sum = c.sum; a.up = c.up; a.flags = c.flags; a.ws = c.ws;
     const int threads = 256;
     auto go = [&](auto vec_tag) -> int {
         constexpr int V = decltype(vec_tag)::value;
         dim3 grid = image_grid(c.B, c.HW / V, threads);
+        if (!fits_partials(grid)) return DCT_ERR_UNSUPPORTED;
 #define DCT_JSD_GO(LG, MD) jsd_kernel<K, C, V, LG, MD, (V == 4 ? 3 : 2)><<<grid, threads, 0, c.stream>>>(a)
         if (c.in_kind == DCT_IN_LOGITS) {
             if (c.mode == kFwd) DCT_JSD_GO(true, kFwd);

@@ -14,7 +14,7 @@ struct PixArgs {
     const float* in[2];
     float* out[2];      // each nullable
     int C;
-    int64_t HW;
+    int64_t B, HW;      // images b = blockIdx.y, blockIdx.y + gridDim.y, ... (image_grid)
     float* map;         // nullable
     double* sum;        // nullable
     Upstream up;
@@ -40,56 +40,57 @@ __global__ void __launch_bounds__(256) pix_kernel(const PixArgs a) {
     const int C = CT ? CT : a.C;
     const int64_t HW = a.HW;
     const int64_t gpi = HW / VEC;
-    const int b = blockIdx.y;
-    const int64_t img = (int64_t)b * C * HW;
     float gs = 1.0f;
     if constexpr (Op::USES_UP) gs = upstream_scalar(a.up);
     double acc = 0.0;
     bool bad = false;
-    for (int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; g < gpi; g += (int64_t)gridDim.x * blockDim.x) {
-        const int64_t i = g * VEC;
-        FVec<VEC> xin[NIN][CM];
-#pragma unroll
-        for (int n = 0; n < NIN; ++n)
-#pragma unroll
-            for (int c = 0; c < CM; ++c)
-                if (c < C) xin[n][c] = ld_stream<VEC>(a.in[n] + img + (int64_t)c * HW + i);
-        FVec<VEC> gm;
-#pragma unroll
-        for (int v = 0; v < VEC; ++v) gm.v[v] = 1.0f;
-        if constexpr (Op::USES_UP) {
-            if (a.up.gmap != nullptr) gm = ld_stream<VEC>(a.up.gmap + (int64_t)b * HW + i);
-        }
-        FVec<VEC> mapv;
-        float part = 0.0f;
-#pragma unroll
-        for (int v = 0; v < VEC; ++v) {
-            float x[NIN][CM];
+    for (int64_t b = blockIdx.y; b < a.B; b += gridDim.y) {
+        const int64_t img = b * C * HW;
+        for (int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; g < gpi; g += (int64_t)gridDim.x * blockDim.x) {
+            const int64_t i = g * VEC;
+            FVec<VEC> xin[NIN][CM];
 #pragma unroll
             for (int n = 0; n < NIN; ++n)
 #pragma unroll
                 for (int c = 0; c < CM; ++c)
-                    if (c < C) x[n][c] = xin[n][c].v[v];
-            float mv = Op::template apply<CM, float>(x, C, gs * gm.v[v], a.eps, bad);
-            mapv.v[v] = mv;
-            part += mv;
+                    if (c < C) xin[n][c] = ld_stream<VEC>(a.in[n] + img + (int64_t)c * HW + i);
+            FVec<VEC> gm;
+#pragma unroll
+            for (int v = 0; v < VEC; ++v) gm.v[v] = 1.0f;
+            if constexpr (Op::USES_UP) {
+                if (a.up.gmap != nullptr) gm = ld_stream<VEC>(a.up.gmap + b * HW + i);
+            }
+            FVec<VEC> mapv;
+            float part = 0.0f;
+#pragma unroll
+            for (int v = 0; v < VEC; ++v) {
+                float x[NIN][CM];
+#pragma unroll
+                for (int n = 0; n < NIN; ++n)
+#pragma unroll
+                    for (int c = 0; c < CM; ++c)
+                        if (c < C) x[n][c] = xin[n][c].v[v];
+                float mv = Op::template apply<CM, float>(x, C, gs * gm.v[v], a.eps, bad);
+                mapv.v[v] = mv;
+                part += mv;
+#pragma unroll
+                for (int n = 0; n < NOUT; ++n)
+#pragma unroll
+                    for (int c = 0; c < CM; ++c)
+                        if (c < C) xin[n][c].v[v] = x[n][c];
+            }
+            acc += (double)part;
+            if constexpr (Op::HAS_MAP) {
+                if (a.map != nullptr) st_stream<VEC>(a.map + b * HW + i, mapv);
+            }
 #pragma unroll
             for (int n = 0; n < NOUT; ++n)
+                if (a.out[n] != nullptr) {
 #pragma unroll
-                for (int c = 0; c < CM; ++c)
-                    if (c < C) xin[n][c].v[v] = x[n][c];
+                    for (int c = 0; c < CM; ++c)
+                        if (c < C) st_stream<VEC>(a.out[n] + img + (int64_t)c * HW + i, xin[n][c]);
+                }
         }
-        acc += (double)part;
-        if constexpr (Op::HAS_MAP) {
-            if (a.map != nullptr) st_stream<VEC>(a.map + (int64_t)b * HW + i, mapv);
-        }
-#pragma unroll
-        for (int n = 0; n < NOUT; ++n)
-            if (a.out[n] != nullptr) {
-#pragma unroll
-                for (int c = 0; c < CM; ++c)
-                    if (c < C) st_stream<VEC>(a.out[n] + img + (int64_t)c * HW + i, xin[n][c]);
-            }
     }
     if constexpr (Op::CHECKS_SIMPLEX) {
         if (a.flags != nullptr && __syncthreads_or(bad)) {
@@ -116,7 +117,10 @@ int pix_launch_ct(const PixArgs& a, int64_t B, cudaStream_t stream) {
     if (!al) return DCT_ERR_UNSUPPORTED;
     const int threads = 256;
     dim3 grid = image_grid(B, a.HW / VEC, threads);
-    pix_kernel<Op, CT, VEC><<<grid, threads, 0, stream>>>(a);
+    if (Op::HAS_MAP && !fits_partials(grid)) return DCT_ERR_UNSUPPORTED;
+    PixArgs ab = a;
+    ab.B = B;
+    pix_kernel<Op, CT, VEC><<<grid, threads, 0, stream>>>(ab);
     return check_launch();
 }
 
