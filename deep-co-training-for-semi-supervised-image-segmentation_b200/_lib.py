@@ -70,6 +70,8 @@ _SIGNATURES = {
     "dct_vote_f32": [_p, _i, _i, _i64, _i64, _i, _p, _p, _p, _p],
     "dct_hausdorff_scratch_bytes": [_i, _i64, _i64, _i64, _i],
     "dct_hausdorff_i64": [_p, _p, _i, _i64, _i64, _i64, _i, _p, _p, _p, _p, _p],
+    "dct_surface_distance_scratch_bytes": [_i, _i64, _i64, _i64, _i],
+    "dct_surface_distances_i64": [_p, _p, _i, _i64, _i64, _i64, _i, _p, _p, _p, _p, _p],
     "dct_jsd_fwdbwd_bf16": [_p, _i, _i, _i64, _i64, _f, _p, _p, _p, _p, _p, _i, _p, _p, _p],
     "dct_kl_logit_bf16": [_p, _p, _i, _i64, _i64, _p, _p, _i, _p, _p, _f, _p, _p, _p, _p],
     "dct_kl_from_logits_fwdbwd_bf16": [_p, _p, _i, _i64, _i64, _f, _f, _p, _p, _p, _p, _p, _p],
@@ -85,7 +87,8 @@ _SIGNATURES = {
     "dct_kl_from_logits_fwdbwd_pub_f32": [_p, _p, _i, _i64, _i64, _f, _f, _p, _p, _p, _p, _p, _p, _p],
 }
 _RESTYPES = {"dct_error_string": C.c_char_p, "dct_last_cuda_error": C.c_char_p, "dct_workspace_bytes": C.c_size_t,
-             "dct_peer_pub_bytes": C.c_size_t, "dct_hausdorff_scratch_bytes": C.c_size_t}
+             "dct_peer_pub_bytes": C.c_size_t, "dct_hausdorff_scratch_bytes": C.c_size_t,
+             "dct_surface_distance_scratch_bytes": C.c_size_t}
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 
 _lib = None

@@ -7,7 +7,9 @@ Mirrors ``generalframework/metrics`` of the reference:
   IoU              metrics/iou.py:8-113
 
 plus ``hausdorff`` / ``HausdorffMeter``: the Hausdorff distance Summary.py:25 takes from the external ``deepclustering``
-package, with the definition of ``medpy.metric.binary.hd`` (exact distance transforms on the device).
+package, with the definition of ``medpy.metric.binary.hd`` (exact distance transforms on the device), and
+``surface_distances`` / ``SurfaceDistanceMeter``: HD95, ASD and ASSD (``medpy.metric.binary`` hd95 / asd / assd) from the
+same distance transforms.
 
 ``add`` never leaves the device (no one-hot tensors, no ``torch.unique(a.cpu())``, no numpy
 ``bincount``); ``value()`` / ``summary()`` keep the reference's return structures.  Counts are exact
@@ -192,6 +194,32 @@ def _class_map(t, C, what):
     return t.to(torch.int64).contiguous()
 
 
+def _distance_args(pred, gt, C, method, voxelspacing, what):
+    """Arguments of ``hausdorff`` / ``surface_distances``: int64 class maps ``p``, ``g`` ``[B,H,W]``, ``C``, whether the
+    batch is one volume, and the spacing as a ctypes double array (``None`` = ones)."""
+    assert method in ('2d', '3d')
+    if pred.is_floating_point():
+        from .utils import _classmap
+        assert pred.dim() == 4, f"{what}: scores [B,C,H,W] expected, got {tuple(pred.shape)}"
+        if pred.dtype != torch.float32:
+            raise TypeError(f"{what}: float32 scores expected, got {pred.dtype}")
+        assert C is None or C == pred.shape[1], f"C={C} does not match scores {tuple(pred.shape)}"
+        C = pred.shape[1]
+        p = _classmap(pred.detach(), 1, want_cls=True)[0]
+    else:
+        assert C is not None, f"{what}: C is required for an integer class map"
+        p = _class_map(pred, C, what)
+    g = _class_map(gt, C, what)
+    assert g.shape == p.shape, f"label shape {tuple(gt.shape)} does not match prediction {tuple(pred.shape)}"
+    volume = method == '3d'
+    sp = None
+    if voxelspacing is not None:
+        vals = [float(v) for v in voxelspacing]
+        assert len(vals) == (3 if volume else 2), f"voxelspacing for '{method}' has {3 if volume else 2} values, got {vals}"
+        sp = (ctypes.c_double * len(vals))(*vals)
+    return p, g, C, volume, sp
+
+
 def hausdorff(pred, gt, C=None, method='2d', voxelspacing=None) -> torch.Tensor:
     """Hausdorff distance per class, float32 ``[rows, C]`` on the input's device (``rows`` = B for ``'2d'``, 1 for ``'3d'``).
 
@@ -208,27 +236,8 @@ def hausdorff(pred, gt, C=None, method='2d', voxelspacing=None) -> torch.Tensor:
     ``voxelspacing``: ``(sy, sx)`` for ``'2d'``, ``(sz, sy, sx)`` for ``'3d'``, ``None`` = ones.  Values outside ``[0, C)``
     belong to no class and raise the label / prediction range checks under the current check mode.
     """
-    assert method in ('2d', '3d')
-    if pred.is_floating_point():
-        from .utils import _classmap
-        assert pred.dim() == 4, f"hausdorff: scores [B,C,H,W] expected, got {tuple(pred.shape)}"
-        if pred.dtype != torch.float32:
-            raise TypeError(f"hausdorff: float32 scores expected, got {pred.dtype}")
-        assert C is None or C == pred.shape[1], f"C={C} does not match scores {tuple(pred.shape)}"
-        C = pred.shape[1]
-        p = _classmap(pred.detach(), 1, want_cls=True)[0]
-    else:
-        assert C is not None, "hausdorff: C is required for an integer class map"
-        p = _class_map(pred, C, "hausdorff")
-    g = _class_map(gt, C, "hausdorff")
-    assert g.shape == p.shape, f"label shape {tuple(gt.shape)} does not match prediction {tuple(pred.shape)}"
+    p, g, C, volume, sp = _distance_args(pred, gt, C, method, voxelspacing, "hausdorff")
     B, H, W = p.shape
-    volume = method == '3d'
-    sp = None
-    if voxelspacing is not None:
-        vals = [float(v) for v in voxelspacing]
-        assert len(vals) == (3 if volume else 2), f"voxelspacing for '{method}' has {3 if volume else 2} values, got {vals}"
-        sp = (ctypes.c_double * len(vals))(*vals)
     h = _lib.lib()
     nbytes = h.dct_hausdorff_scratch_bytes(C, B, H, W, int(volume))
     if nbytes == 0:
@@ -243,6 +252,34 @@ def hausdorff(pred, gt, C=None, method='2d', voxelspacing=None) -> torch.Tensor:
     return out
 
 
+_SURFACE_KEYS = ('hd', 'hd95', 'asd', 'assd')
+
+
+def surface_distances(pred, gt, C=None, method='2d', voxelspacing=None) -> dict:
+    """Surface distances per class: ``{'hd', 'hd95', 'asd', 'assd'}``, each float32 ``[rows, C]`` on the input's device,
+    from one device call.  Arguments, borders, grids, spacing and NaN are those of ``hausdorff``.
+
+    With ``S_pg`` the distances from each border pixel of ``{pred == c}`` to the border of ``{gt == c}`` and ``S_gp`` the
+    other direction (``medpy.metric.binary``, connectivity 1): ``hd`` = ``hausdorff(...)`` bit for bit; ``hd95`` =
+    ``np.percentile(np.hstack((S_pg, S_gp)), 95)`` (medpy ``hd95``); ``asd`` = ``mean(S_pg)`` (medpy ``asd(pred, gt)``,
+    directional); ``assd`` = ``(mean(S_pg) + mean(S_gp)) / 2`` (medpy ``assd``).
+    """
+    p, g, C, volume, sp = _distance_args(pred, gt, C, method, voxelspacing, "surface_distances")
+    B, H, W = p.shape
+    h = _lib.lib()
+    nbytes = h.dct_surface_distance_scratch_bytes(C, B, H, W, int(volume))
+    if nbytes == 0:
+        _lib.check(_lib.ERR_UNSUPPORTED, f"dct_surface_distance_scratch_bytes (C={C}, shape {(B, H, W)})")
+    scratch = torch.empty(nbytes, dtype=torch.uint8, device=p.device)
+    out = torch.empty((4, 1 if volume else B, C), dtype=torch.float32, device=p.device)
+    st = _runtime.state(p.device)
+    _lib.check(h.dct_surface_distances_i64(p.data_ptr(), g.data_ptr(), C, B, H, W, int(volume), sp, out.data_ptr(),
+                                           _runtime.flags_ptr(st), scratch.data_ptr(), _runtime.stream_ptr(p.device)),
+               "dct_surface_distances_i64")
+    _runtime.after_call(st)
+    return dict(zip(_SURFACE_KEYS, out.unbind(0)))
+
+
 def _nan_mean_std(x: torch.Tensor, dim: int):
     """Mean and unbiased standard deviation along ``dim`` over the non-NaN entries (NaN where fewer than 1 / 2 remain)."""
     valid = ~torch.isnan(x)
@@ -251,6 +288,14 @@ def _nan_mean_std(x: torch.Tensor, dim: int):
     dev = torch.where(valid, x - mean.unsqueeze(dim), torch.zeros_like(x))
     var = (dev * dev).sum(dim) / (n - 1)
     return mean, torch.where(n > 1, var.sqrt(), torch.full_like(var, float('nan')))
+
+
+def _nan_statistics(log: torch.Tensor, report_axis):
+    """``HausdorffMeter.value`` of a ``[rows, C]`` log."""
+    means, stds = _nan_mean_std(log, 0)
+    axes = log if report_axis == 'all' else log[:, report_axis]
+    report_mean, report_std = _nan_mean_std(torch.nanmean(axes, 1), 0)
+    return (report_mean, report_std), (means, stds)
 
 
 class HausdorffMeter(Metric):
@@ -282,11 +327,7 @@ class HausdorffMeter(Metric):
     def value(self, **kwargs):
         """``((mean, std), (means[C], stds[C]))``: per class over the rows, and of the per-row mean over the report
         axes; NaN entries skipped, unbiased standard deviations."""
-        log = self.log
-        means, stds = _nan_mean_std(log, 0)
-        axes = log if self.report_axis == 'all' else log[:, self.report_axis]
-        report_mean, report_std = _nan_mean_std(torch.nanmean(axes, 1), 0)
-        return (report_mean, report_std), (means, stds)
+        return _nan_statistics(self.log, self.report_axis)
 
     def detailed_summary(self) -> dict:
         _, (means, _) = self.value()
@@ -295,6 +336,55 @@ class HausdorffMeter(Metric):
     def summary(self) -> dict:
         (mean, var), _ = self.value()
         return {'mHD': mean.item(), 'mHDVars': var.item()}
+
+
+class SurfaceDistanceMeter(Metric):
+    """HD, HD95, ASD and ASSD per class next to ``DiceMeter`` (same ``method`` / ``report_axises`` / ``C``; definitions of
+    ``surface_distances``).  ``add`` makes one device call and appends one row per image (``'2d'``) or per batch
+    (``'3d'``) to each metric's log; the statistics are ``HausdorffMeter``'s and skip the NaN of absent classes."""
+
+    _NAMES = (('hd', 'HD', 'HD'), ('hd95', 'HD95', 'HD95_'), ('asd', 'ASD', 'ASD'), ('assd', 'ASSD', 'ASSD'))   # key, summary, detailed
+
+    def __init__(self, method='2d', report_axises='all', C=4) -> None:
+        super().__init__()
+        assert method in ('2d', '3d')
+        assert report_axises == 'all' or isinstance(report_axises, list)
+        self.method = method
+        self.report_axis = report_axises
+        self.C = C
+        self.reset()
+
+    def reset(self):
+        self.logs = {k: [] for k in _SURFACE_KEYS}
+
+    def add(self, pred, gt, voxelspacing=None):
+        r = surface_distances(pred, gt, C=self.C, method=self.method, voxelspacing=voxelspacing)
+        for k in _SURFACE_KEYS:
+            self.logs[k].append(r[k])
+
+    def log(self, metric='hd95') -> torch.Tensor:
+        rows = self.logs[metric]
+        if len(rows) == 0:
+            return torch.full((1, self.C), float('nan'))
+        return torch.cat(rows)
+
+    def value(self, metric='hd95'):
+        """``((mean, std), (means[C], stds[C]))`` of one metric's log, as ``HausdorffMeter.value``."""
+        return _nan_statistics(self.log(metric), self.report_axis)
+
+    def detailed_summary(self) -> dict:
+        out = {}
+        for k, _, prefix in self._NAMES:
+            _, (means, _) = self.value(k)
+            out.update({f'{prefix}{i}': means[i].item() for i in range(len(means))})
+        return out
+
+    def summary(self) -> dict:
+        out = {}
+        for k, name, _ in self._NAMES:
+            (mean, var), _ = self.value(k)
+            out.update({f'm{name}': mean.item(), f'm{name}Vars': var.item()})
+        return out
 
 
 class ConfusionMatrix(Metric):

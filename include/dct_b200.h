@@ -383,6 +383,28 @@ DCT_API size_t dct_hausdorff_scratch_bytes(int C, int64_t B, int64_t H, int64_t 
 DCT_API int dct_hausdorff_i64(const int64_t* pred, const int64_t* labels, int C, int64_t B, int64_t H, int64_t W,
                               int volume, const double* spacing, float* hd, int32_t* flags, void* scratch, void* stream);
 
+/* Surface distances of the same borders, grids and spacing (medpy.metric.binary hd95 / asd / assd, connectivity 1).
+ * Per (row, class): S_pg = d(x, border(G)) for every x in border(A), S_gp = d(y, border(A)) for every y in border(G);
+ *   hd   = max(max S_pg, max S_gp), bit-identical to dct_hausdorff_i64;
+ *   hd95 = numpy.percentile(concat(S_pg, S_gp), 95) with the default 'linear' method: n = |S_pg| + |S_gp|,
+ *          v = (n - 1) * 0.95, lo = floor(v), t = v - lo, a = sorted[lo], b = sorted[min(lo + 1, n - 1)], d = b - a,
+ *          (t >= 0.5 ? b - d * (1 - t) : a + d * t) in double, rounded once to float;
+ *   asd  = mean(S_pg) (directional: prediction border to label border), assd = (mean(S_pg) + mean(S_gp)) / 2.
+ * All four are NaN where A or G is empty.  Same limits, flags, argument checks and error codes as dct_hausdorff_i64.
+ * The last distance pass keeps each border pixel's d^2 and per-line sums; a radix select on the d^2 bits (4 passes of
+ * 8 bits, integer histograms) and a fixed-order reduction of the sums make the result bit-reproducible.  14 launches
+ * for a slice batch, 15 for a volume; no host synchronisation, no allocation. */
+
+/* bytes of `scratch` dct_surface_distances_i64 needs: dct_hausdorff_scratch_bytes() + 8 per pixel (d^2 of the queries
+ * of both sides) + 12 per line of the last pass (2*C*B*H lines for a slice batch, 2*C*H*W for a volume) + 2112 per
+ * (row, class), each region rounded up to 256 bytes; 0 for a shape it rejects.  Host only. */
+DCT_API size_t dct_surface_distance_scratch_bytes(int C, int64_t B, int64_t H, int64_t W, int volume);
+/* pred, labels, spacing, flags, scratch as for dct_hausdorff_i64 (scratch >= dct_surface_distance_scratch_bytes());
+ * out float32 [4][volume ? 1 : B][C] = hd, hd95, asd, assd, overwritten. */
+DCT_API int dct_surface_distances_i64(const int64_t* pred, const int64_t* labels, int C, int64_t B, int64_t H, int64_t W,
+                                      int volume, const double* spacing, float* out, int32_t* flags, void* scratch,
+                                      void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * bfloat16 twins of the one-pass-over-logits entry points (networks under torch.autocast emit bf16 logits;
  * north_star: "within 1e-2 relative in bf16").  Tensors [B,C,HW] are bfloat16 (2-byte elements, same NCHW
