@@ -194,21 +194,25 @@ def _class_map(t, C, what):
     return t.to(torch.int64).contiguous()
 
 
-def _distance_args(pred, gt, C, method, voxelspacing, what):
-    """Arguments of ``hausdorff`` / ``surface_distances``: int64 class maps ``p``, ``g`` ``[B,H,W]``, ``C``, whether the
-    batch is one volume, and the spacing as a ctypes double array (``None`` = ones)."""
-    assert method in ('2d', '3d')
+def _prediction_map(pred, C, what):
+    """int64 class map ``[B,H,W]`` and ``C`` of a prediction: float32 scores ``[B,C,H,W]`` reduced with the arg-max
+    ``DiceMeter.add`` uses, or an integer ``[B,H,W]`` / ``[B,1,H,W]`` class map (then ``C`` is required)."""
     if pred.is_floating_point():
         from .utils import _classmap
         assert pred.dim() == 4, f"{what}: scores [B,C,H,W] expected, got {tuple(pred.shape)}"
         if pred.dtype != torch.float32:
             raise TypeError(f"{what}: float32 scores expected, got {pred.dtype}")
         assert C is None or C == pred.shape[1], f"C={C} does not match scores {tuple(pred.shape)}"
-        C = pred.shape[1]
-        p = _classmap(pred.detach(), 1, want_cls=True)[0]
-    else:
-        assert C is not None, f"{what}: C is required for an integer class map"
-        p = _class_map(pred, C, what)
+        return _classmap(pred.detach(), 1, want_cls=True)[0], pred.shape[1]
+    assert C is not None, f"{what}: C is required for an integer class map"
+    return _class_map(pred, C, what), C
+
+
+def _distance_args(pred, gt, C, method, voxelspacing, what):
+    """Arguments of ``hausdorff`` / ``surface_distances``: int64 class maps ``p``, ``g`` ``[B,H,W]``, ``C``, whether the
+    batch is one volume, and the spacing as a ctypes double array (``None`` = ones)."""
+    assert method in ('2d', '3d')
+    p, C = _prediction_map(pred, C, what)
     g = _class_map(gt, C, what)
     assert g.shape == p.shape, f"label shape {tuple(gt.shape)} does not match prediction {tuple(pred.shape)}"
     volume = method == '3d'

@@ -406,6 +406,34 @@ DCT_API int dct_surface_distances_i64(const int64_t* pred, const int64_t* labels
                                       void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Connected components of a class map (evaluation path: the post-processing in front of the Dice and surface distances;
+ * getLargestCC of the UA-MT / DTC / MC-Net test scripts, nnU-Net's "remove all but the largest component").
+ * Grids as for dct_hausdorff_i64: every H x W slice on its own (volume == 0; adjacency never crosses slices) or the
+ * B x H x W batch as one volume (volume != 0).  Neighbourhood: scipy's generate_binary_structure(rank, connectivity),
+ * offsets in {-1,0,1}^rank with at most `connectivity` non-zero entries (slices: 1 -> 4, 2 -> 8 neighbours; volume:
+ * 1 -> 6, 2 -> 18, 3 -> 26).  Two pixels are in one component when they hold the same class c in [0,C) and are joined
+ * through neighbours holding c; every class, 0 included, is labelled.
+ *   labels      int32 [B,H,W]: the linear index in the batch tensor of the component's first pixel in raster order (its
+ *               smallest index; scipy.ndimage.label numbers components in this order); -1 for a value outside [0,C).
+ *   stats       int64 [volume ? 1 : B][C][2]: number of components, size in pixels of the largest; (0, 0) for an absent class.
+ *   largest_map int64 [B,H,W]: the input with every pixel of a class c >= 1 outside the largest component of c on its
+ *               grid set to 0 (ties: the component with the smallest first-pixel index, np.argmax(np.bincount(...)[1:]) on
+ *               scipy's labels); class 0 is never filtered.
+ * Values outside [0,C) belong to no component, count toward no statistic, are copied unchanged into largest_map and are
+ * counted in flags[DCT_FLAG_PRED].  Union-find that always links the larger root to the smaller (atomicMin), so every
+ * output is a bit-reproducible integer.  5 launches (3 when only labels are asked for); no host synchronisation, no
+ * allocation.  Limits (DCT_ERR_UNSUPPORTED): C <= DCT_MAX_CLASSES, B*H*W <= 2^31 - 1.
+ * ------------------------------------------------------------------------------------------ */
+
+/* bytes of `scratch` dct_components_i64 needs: 9 per pixel + 16 per (row, class), each region rounded up to 256 bytes;
+ * 0 for a shape it rejects.  Host only. */
+DCT_API size_t dct_components_scratch_bytes(int C, int64_t B, int64_t H, int64_t W, int volume);
+/* map int64 [B,H,W]; labels, stats, largest_map each nullable, at least one given, overwritten; largest_map must not
+ * overlap map; connectivity in 1..(volume ? 3 : 2), else DCT_ERR_BAD_ARG; scratch: >= dct_components_scratch_bytes()
+ * bytes, 256-byte aligned, no initial state required, private to the call until the stream reaches its end. */
+DCT_API int dct_components_i64(const int64_t* map, int C, int64_t B, int64_t H, int64_t W, int volume, int connectivity, int32_t* labels, int64_t* stats, int64_t* largest_map, int32_t* flags, void* scratch, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * bfloat16 twins of the one-pass-over-logits entry points (networks under torch.autocast emit bf16 logits;
  * north_star: "within 1e-2 relative in bf16").  Tensors [B,C,HW] are bfloat16 (2-byte elements, same NCHW
  * layout), gradients are written as bfloat16 (round-to-nearest-even); ALL arithmetic is fp32 in registers and the
