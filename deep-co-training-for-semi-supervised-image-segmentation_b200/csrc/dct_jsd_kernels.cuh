@@ -153,92 +153,6 @@ __device__ __forceinline__ T jsd_pixel(T (&x)[K][C], T gK, bool& bad) {
     return jsd;
 }
 
-// K-view JSD forward + backward from logits on a pixel (pair) whose K*C values stay in the shared-memory stage (K*C > 40:
-// a register-resident pair would need > 255 registers and spills).  Four sweeps over the stage, in place:
-//   A  per view: max_c x                                                    (LDS)
-//   B  per view: e = 2^((x - max) log2 e) written over x; Z = sum e; S = sum e*t       -> sum_c p lg p = S/Z - lg Z
-//   C  per class: m = (1/K) sum_k e_k/Z_k; lg m; H(m); per view sum_c e lg m           -> KL(p_k||m) without another pass
-//   D  per class: lg m again (K multiplies + one MUFU), lg p = lg2(e) - lg Z; gradient written over e
-// MUFU per pixel: 2*K*C (ex2, lg2 of e) + 2*C (lg m) + 2*K -- 155 at K=3, 190 at K=4, against ~360-480 issue slots.
-// e underflows to 0 below 2^-126: lg2(0) = -inf is clamped so that 0 * (...) stays 0 (the register path's 0 * finite).
-template <int K, int C, class T>
-__device__ __forceinline__ T jsd_stream_pair(unsigned char* st, size_t row_bytes, int p0, float g) {
-    auto at = [&](int k, int c) -> T* { return reinterpret_cast<T*>(st + (size_t)(k * C + c) * row_bytes + (size_t)p0 * 4); };
-    const float invK = 1.0f / (float)K;
-    T rZ[K], lZ[K], hp[K];
-    T hsum = vset<T>(0.0f);
-#pragma unroll
-    for (int k = 0; k < K; ++k) {
-        T mx = *at(k, 0);
-#pragma unroll
-        for (int c = 1; c < C; ++c) mx = vmax(mx, *at(k, c));
-        const T nmxl = vmuls(mx, -kLog2e);
-        T Z = vset<T>(0.0f), S = vset<T>(0.0f);
-#pragma unroll
-        for (int c = 0; c < C; ++c) {
-            const T t = vfmas(*at(k, c), kLog2e, nmxl);  // (x - max) * log2(e), one rounding
-            const T e = vex2(t);
-            *at(k, c) = e;
-            Z = vadd(Z, e);
-            S = vfma(e, t, S);
-        }
-        rZ[k] = vrcp(Z);
-        lZ[k] = vlg2(Z);
-        hp[k] = vsub(vmul(rZ[k], S), lZ[k]);     // sum_c p lg2 p
-        hsum = vadd(hsum, hp[k]);
-        // compiler barrier: the next sweeps re-read e from the stage instead of keeping K*C pairs in (255) registers
-        // across them -- the point of this body is a small register footprint
-        asm volatile("" ::: "memory");
-    }
-    T hm = vset<T>(0.0f);
-    T plm[K];
-#pragma unroll
-    for (int k = 0; k < K; ++k) plm[k] = vset<T>(0.0f);
-    T rZK[K];                                    // 1 / (K Z_k): m_c = sum_k e_kc * rZK_k
-#pragma unroll
-    for (int k = 0; k < K; ++k) rZK[k] = vmuls(rZ[k], invK);
-#pragma unroll
-    for (int c = 0; c < C; ++c) {
-        T e[K];
-#pragma unroll
-        for (int k = 0; k < K; ++k) e[k] = *at(k, c);
-        T m = vmul(e[0], rZK[0]);
-#pragma unroll
-        for (int k = 1; k < K; ++k) m = vfma(e[k], rZK[k], m);
-        const T lm = vlg2(vadds(m, kEntEps));
-        hm = vfma(m, lm, hm);
-#pragma unroll
-        for (int k = 0; k < K; ++k) plm[k] = vfma(e[k], lm, plm[k]);
-    }
-    const T jsd = vmuls(vsub(vmuls(hsum, invK), hm), kLn2);
-    asm volatile("" ::: "memory");
-    // gradient: (g/K) ln2 * p_kc * ((lg p_kc - lg m_c) - KL_k),  KL_k = hp_k - sum_c p_kc lg m_c  (in lg2 units)
-    T off[K], gr[K];
-    const float g2 = g * invK * kLn2;
-#pragma unroll
-    for (int k = 0; k < K; ++k) {
-        const T kl = vsub(hp[k], vmul(rZ[k], plm[k]));
-        off[k] = vadd(lZ[k], kl);                // (lg2 e - lg Z) - lg m - KL  =  lg2 e - lg m - off
-        gr[k] = vmuls(rZ[k], g2);                // g2 * p = gr * e
-    }
-#pragma unroll
-    for (int c = 0; c < C; ++c) {
-        T e[K];
-#pragma unroll
-        for (int k = 0; k < K; ++k) e[k] = *at(k, c);
-        T m = vmul(e[0], rZK[0]);
-#pragma unroll
-        for (int k = 1; k < K; ++k) m = vfma(e[k], rZK[k], m);
-        const T lm = vlg2(vadds(m, kEntEps));
-#pragma unroll
-        for (int k = 0; k < K; ++k) {
-            const T le = vmax(vlg2(e[k]), vset<T>(-1.0e4f));   // e == 0 (underflow): keep 0 * finite == 0
-            *at(k, c) = vmul(vmul(gr[k], e[k]), vsub(vsub(le, lm), off[k]));
-        }
-    }
-    return jsd;
-}
-
 // JSD as a tile-pipeline Op (dct_tile.cuh): NIN = K views; gradients overwrite the views' rows.
 template <int K, bool LOGITS, int MODE, bool DICEF>
 struct JsdOp {
@@ -246,21 +160,16 @@ struct JsdOp {
     static constexpr bool HAS_MAP = (MODE != kBwd), USES_UP = (MODE != kFwd), CHECKS_SIMPLEX = !LOGITS;
     static constexpr int NDICE = DICEF ? K : 0;
     static constexpr bool GMAP = (MODE == kBwd);
-    // logits in, loss + gradients out, no meters: the shape the shared-memory-resident body (jsd_stream_pair) serves
-    static constexpr bool STREAM_CAPABLE = LOGITS && MODE == kFwdBwd && !DICEF;
-    template <int CM, class T>   // T = f2: a pixel pair per thread (p0 even); T = float: one pixel per thread
-    static __device__ __forceinline__ T stream(unsigned char* st, size_t row_bytes, int p0, float g) {
-        return jsd_stream_pair<K, CM, T>(st, row_bytes, p0, g);
-    }
     template <int CM, class T>
     static __device__ __forceinline__ T apply(T (&x)[K][CM], int, T g, float, bool& bad) {
         return jsd_pixel<K, CM, LOGITS, MODE != kFwd, T>(x, vmuls(g, 1.0f / (float)K), bad);
     }
 };
 
+// (K*C <= 16 has no register-tiled instantiation: the tile pipeline takes every call such a kernel could, see jsd_launch_kc)
 template <int K, int C>
 constexpr int jsd_vec() {
-    return K * C <= 16 ? 4 : (K * C <= 40 ? 2 : 1);
+    return K * C <= 40 ? 2 : 1;
 }
 
 template <int K, int C, int VEC, bool LOGITS, int MODE, int MINB = 1>
@@ -545,7 +454,7 @@ int jsd_launch_kc(const JsdCall& c) {
         return DCT_ERR_UNSUPPORTED;
     }
     if constexpr (K * C <= kTileMaxRows) {
-        // TMA tile pipeline (falls through to the register-tiled kernel when rows are not 16-byte aligned)
+        // TMA tile pipeline (falls through to the register-tiled kernel when rows are not 16-byte aligned and K*C > 16)
         int rc = jsd_launch_tile<K, C>(c);
         if (rc != DCT_ERR_UNSUPPORTED) return rc;
     }
@@ -564,7 +473,7 @@ int jsd_launch_kc(const JsdCall& c) {
         constexpr int V = decltype(vec_tag)::value;
         dim3 grid = image_grid(c.B, c.HW / V, threads);
         if (!fits_partials(grid)) return DCT_ERR_UNSUPPORTED;
-#define DCT_JSD_GO(LG, MD) jsd_kernel<K, C, V, LG, MD, (V == 4 ? 3 : 2)><<<grid, threads, 0, c.stream>>>(a)
+#define DCT_JSD_GO(LG, MD) jsd_kernel<K, C, V, LG, MD, 2><<<grid, threads, 0, c.stream>>>(a)
         if (c.in_kind == DCT_IN_LOGITS) {
             if (c.mode == kFwd) DCT_JSD_GO(true, kFwd);
             else if (c.mode == kBwd) DCT_JSD_GO(true, kBwd);
@@ -577,8 +486,10 @@ int jsd_launch_kc(const JsdCall& c) {
 #undef DCT_JSD_GO
         return check_launch();
     };
-    if (al) return go(std::integral_constant<int, VEC>{});
-    return DCT_ERR_UNSUPPORTED;  // odd HW / misaligned views: the caller falls back to jsd_kernel_rt
+    if constexpr (K * C > 16) {
+        if (al) return go(std::integral_constant<int, VEC>{});
+    }
+    return DCT_ERR_UNSUPPORTED;  // odd HW / misaligned views, or K*C <= 16: the caller falls back to jsd_kernel_rt
 }
 
 }  // namespace dct

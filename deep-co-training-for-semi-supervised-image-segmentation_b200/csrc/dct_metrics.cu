@@ -38,16 +38,13 @@ __device__ __forceinline__ void load_pixels(const float* xb, int C, int64_t HW, 
 }
 
 // ---------------------------------------------------------------------------------------------
-// Dice counts.  grid = (gx, B): a CTA only sees pixels of image blockIdx.y.
-//   C <= 4 : three packed 32-bit registers per thread (8-bit field per class) for I, G, P,
-//            flushed to 32-bit warp sums every <= 252 pixels;  zero atomics in the pixel loop.
-//   C  > 4 : shared-memory histogram over (label row incl. one "invalid" row) x (prediction),
-//            one shared atomic per pixel; I/G/P are its diagonal, row sums and column sums.
+// Dice counts of the shapes the tile pipeline's DiceOp does not take (C > 4, or rows it refuses).  grid = (gx, B): a CTA
+// only sees pixels of image blockIdx.y.  Shared-memory histogram over (label row incl. one "invalid" row) x (prediction),
+// one shared atomic per pixel; I/G/P are its diagonal, row sums and column sums.
 // ---------------------------------------------------------------------------------------------
 template <int CT, int VEC>
 __global__ void __launch_bounds__(256) dice_kernel(const MetricArgs a) {
     constexpr int CM = CT ? CT : DCT_MAX_CLASSES;
-    constexpr bool PACKED = (CT > 0 && CT <= 4);
     const int C = CT ? CT : a.C;
     const int64_t HW = a.HW;
     const int64_t gpi = HW / VEC;
@@ -55,19 +52,12 @@ __global__ void __launch_bounds__(256) dice_kernel(const MetricArgs a) {
     const float* xb = a.x + (int64_t)b * C * HW;
     const int64_t* lb = a.labels + (int64_t)b * HW;
 
-    extern __shared__ int s_hist[];  // PACKED: 3*C ints ; else (C+1)*C ints
-    const int nbins = PACKED ? 3 * C : (C + 1) * C;
+    extern __shared__ int s_hist[];  // (C+1)*C ints
+    const int nbins = (C + 1) * C;
     for (int j = threadIdx.x; j < nbins; j += blockDim.x) s_hist[j] = 0;
     __syncthreads();
 
     int nbad = 0;
-    unsigned int pI = 0, pG = 0, pP = 0;  // packed 8-bit fields (PACKED only)
-    int wI[PACKED ? CM : 1], wG[PACKED ? CM : 1], wP[PACKED ? CM : 1];
-    if constexpr (PACKED) {
-#pragma unroll
-        for (int c = 0; c < CM; ++c) { wI[c] = 0; wG[c] = 0; wP[c] = 0; }
-    }
-    int since_flush = 0;
     for (int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; g < gpi; g += (int64_t)gridDim.x * blockDim.x) {
         const int64_t i = g * VEC;
         FVec<VEC> xin[CM];
@@ -88,64 +78,21 @@ __global__ void __launch_bounds__(256) dice_kernel(const MetricArgs a) {
             const long long gl = lab[v];
             const bool valid = (gl >= 0) & (gl < C);
             nbad += !valid;
-            if constexpr (PACKED) {
-                const unsigned int sh = 8u * (unsigned int)pred;
-                pP += 1u << sh;
-                if (valid) {
-                    pG += 1u << (8u * (unsigned int)gl);
-                    pI += (unsigned int)(gl == pred) << sh;
-                }
-            } else {
-                const int row = valid ? (int)gl : C;
-                atomicAdd(&s_hist[row * C + pred], 1);
-            }
-        }
-        if constexpr (PACKED) {
-            since_flush += VEC;
-            if (since_flush > 255 - VEC) {
-#pragma unroll
-                for (int c = 0; c < CM; ++c) {
-                    wI[c] += (pI >> (8 * c)) & 0xffu; wG[c] += (pG >> (8 * c)) & 0xffu; wP[c] += (pP >> (8 * c)) & 0xffu;
-                }
-                pI = pG = pP = 0; since_flush = 0;
-            }
-        }
-    }
-    if constexpr (PACKED) {
-        const int lane = threadIdx.x & 31;
-#pragma unroll
-        for (int c = 0; c < CM; ++c) {
-            int vI = wI[c] + (int)((pI >> (8 * c)) & 0xffu);
-            int vG = wG[c] + (int)((pG >> (8 * c)) & 0xffu);
-            int vP = wP[c] + (int)((pP >> (8 * c)) & 0xffu);
-            vI = __reduce_add_sync(0xffffffffu, vI);
-            vG = __reduce_add_sync(0xffffffffu, vG);
-            vP = __reduce_add_sync(0xffffffffu, vP);
-            if (lane == 0) {
-                if (vI) atomicAdd(&s_hist[c * 3 + 0], vI);
-                if (vG) atomicAdd(&s_hist[c * 3 + 1], vG);
-                if (vP) atomicAdd(&s_hist[c * 3 + 2], vP);
-            }
+            const int row = valid ? (int)gl : C;
+            atomicAdd(&s_hist[row * C + pred], 1);
         }
     }
     nbad = __reduce_add_sync(0xffffffffu, nbad);
     if ((threadIdx.x & 31) == 0 && nbad != 0 && a.flags != nullptr) atomicAdd(&a.flags[DCT_FLAG_LABEL], nbad);
     __syncthreads();
     unsigned long long* out = reinterpret_cast<unsigned long long*>(a.out) + (int64_t)b * C * 3;
-    if constexpr (PACKED) {
-        for (int j = threadIdx.x; j < 3 * C; j += blockDim.x) {
-            int v = s_hist[j];
-            if (v) atomicAdd(&out[j], (unsigned long long)v);
-        }
-    } else {
-        for (int c = threadIdx.x; c < C; c += blockDim.x) {
-            int vI = s_hist[c * C + c], vG = 0, vP = 0;
-            for (int j = 0; j < C; ++j) vG += s_hist[c * C + j];
-            for (int r = 0; r <= C; ++r) vP += s_hist[r * C + c];
-            if (vI) atomicAdd(&out[c * 3 + 0], (unsigned long long)vI);
-            if (vG) atomicAdd(&out[c * 3 + 1], (unsigned long long)vG);
-            if (vP) atomicAdd(&out[c * 3 + 2], (unsigned long long)vP);
-        }
+    for (int c = threadIdx.x; c < C; c += blockDim.x) {
+        int vI = s_hist[c * C + c], vG = 0, vP = 0;
+        for (int j = 0; j < C; ++j) vG += s_hist[c * C + j];
+        for (int r = 0; r <= C; ++r) vP += s_hist[r * C + c];
+        if (vI) atomicAdd(&out[c * 3 + 0], (unsigned long long)vI);
+        if (vG) atomicAdd(&out[c * 3 + 1], (unsigned long long)vG);
+        if (vP) atomicAdd(&out[c * 3 + 2], (unsigned long long)vP);
     }
 }
 
@@ -253,18 +200,19 @@ static int dice_launch_ct(const MetricArgs& a, int64_t B, cudaStream_t s) {
         t.in[0] = a.x; t.HW = a.HW; t.flags = a.flags; t.labels = a.labels;
         t.counts = reinterpret_cast<unsigned long long*>(a.out); t.count_view_stride = B * CT * 3;
         if (tile_eligible<DiceOp>(t, B)) return tile_launch_ct<DiceOp, CT>(t, B, s);
+        return DCT_ERR_UNSUPPORTED;   // the caller falls back to dice_kernel<0, 1>
+    } else {
+        constexpr int VEC = metric_vec<CT>();
+        if ((a.HW % VEC) != 0 || !aligned(a.x, 4 * VEC) || !aligned(a.labels, VEC >= 2 ? 16 : 8)) return DCT_ERR_UNSUPPORTED;
+        const int C = CT ? CT : a.C;
+        const size_t smem = sizeof(int) * (C + 1) * C;
+        // each thread takes ~4 pixel groups so that the per-CTA merge (<= 3C global atomics) amortises
+        int64_t gpi = a.HW / VEC;
+        int64_t gx = (gpi + 256 * 4 - 1) / (256 * 4);
+        if (gx > 65535) gx = 65535;
+        dice_kernel<CT, VEC><<<dim3((unsigned)gx, (unsigned)B), 256, smem, s>>>(a);
+        return check_launch();
     }
-    constexpr int VEC = metric_vec<CT>();
-    if ((a.HW % VEC) != 0 || !aligned(a.x, 4 * VEC) || !aligned(a.labels, VEC >= 2 ? 16 : 8)) return DCT_ERR_UNSUPPORTED;
-    const int C = CT ? CT : a.C;
-    const bool packed = (CT > 0 && CT <= 4);
-    const size_t smem = sizeof(int) * (packed ? 3 * C : (C + 1) * C);
-    // each thread takes ~4 pixel groups so that the per-CTA merge (<= 3C global atomics) amortises
-    int64_t gpi = a.HW / VEC;
-    int64_t gx = (gpi + 256 * 4 - 1) / (256 * 4);
-    if (gx > 65535) gx = 65535;
-    dice_kernel<CT, VEC><<<dim3((unsigned)gx, (unsigned)B), 256, smem, s>>>(a);
-    return check_launch();
 }
 
 template <int CT>

@@ -23,9 +23,10 @@ struct PixArgs {
     Workspace* ws;
 };
 
+// (NIN*CT <= 16 has no register-tiled instantiation: the tile pipeline takes every call such a kernel could, see pix_launch_ct)
 template <int NIN, int CT>
 constexpr int pix_vec() {
-    return CT == 0 ? 1 : (NIN * CT <= 16 ? 4 : (NIN * CT <= 40 ? 2 : 1));
+    return CT == 0 ? 1 : (NIN * CT <= 40 ? 2 : 1);
 }
 
 // Op interface:
@@ -109,19 +110,23 @@ int pix_launch_ct(const PixArgs& a, int64_t B, cudaStream_t stream) {
         t.HW = a.HW; t.map = a.map; t.sum = a.sum; t.up = a.up; t.eps = a.eps; t.flags = a.flags; t.ws = a.ws;
         if (tile_eligible<Op>(t, B)) return tile_launch_ct<Op, CT>(t, B, stream);
     }
-    constexpr int VEC = pix_vec<Op::NIN, CT>();
-    bool al = (a.HW % VEC) == 0 && (a.map == nullptr || aligned(a.map, 4 * VEC)) &&
-              (a.up.gmap == nullptr || aligned(a.up.gmap, 4 * VEC));
-    for (int n = 0; n < Op::NIN; ++n) al = al && aligned(a.in[n], 4 * VEC);
-    for (int n = 0; n < Op::NOUT; ++n) al = al && (a.out[n] == nullptr || aligned(a.out[n], 4 * VEC));
-    if (!al) return DCT_ERR_UNSUPPORTED;
-    const int threads = 256;
-    dim3 grid = image_grid(B, a.HW / VEC, threads);
-    if (Op::HAS_MAP && !fits_partials(grid)) return DCT_ERR_UNSUPPORTED;
-    PixArgs ab = a;
-    ab.B = B;
-    pix_kernel<Op, CT, VEC><<<grid, threads, 0, stream>>>(ab);
-    return check_launch();
+    if constexpr (CT > 0 && Op::NIN * CT <= 16) {
+        return DCT_ERR_UNSUPPORTED;   // refused by the tile pipeline: the caller falls back to pix_kernel<Op, 0, 1>
+    } else {
+        constexpr int VEC = pix_vec<Op::NIN, CT>();
+        bool al = (a.HW % VEC) == 0 && (a.map == nullptr || aligned(a.map, 4 * VEC)) &&
+                  (a.up.gmap == nullptr || aligned(a.up.gmap, 4 * VEC));
+        for (int n = 0; n < Op::NIN; ++n) al = al && aligned(a.in[n], 4 * VEC);
+        for (int n = 0; n < Op::NOUT; ++n) al = al && (a.out[n] == nullptr || aligned(a.out[n], 4 * VEC));
+        if (!al) return DCT_ERR_UNSUPPORTED;
+        const int threads = 256;
+        dim3 grid = image_grid(B, a.HW / VEC, threads);
+        if (Op::HAS_MAP && !fits_partials(grid)) return DCT_ERR_UNSUPPORTED;
+        PixArgs ab = a;
+        ab.B = B;
+        pix_kernel<Op, CT, VEC><<<grid, threads, 0, stream>>>(ab);
+        return check_launch();
+    }
 }
 
 template <class Op>

@@ -32,8 +32,6 @@
 #pragma once
 #include <cuda_bf16.h>
 
-#include <cstdlib>
-
 #include "dct_common.cuh"
 #include "dct_tma.cuh"
 #include "dct_tmap.cuh"
@@ -82,37 +80,17 @@ __device__ __forceinline__ void tile_st_row(unsigned char* row, int p0, const FV
     }
 }
 
-// stages with at least this many fp32 rows per pixel use an op's shared-memory-resident body, if it has one.  Off in
-// the product: with the launch shapes below the register-resident body is as fast or faster at every measured shape
-// (profiles/r08/kbench_wide_{reg,stream}.log); tools/kbench_tile.cu builds with -DDCT_STREAM_MIN_ROWS=41 for the A/B,
-// and tests/test_gpu_parity.py covers the same inputs whichever body is compiled in.
-#ifndef DCT_STREAM_MIN_ROWS
-#define DCT_STREAM_MIN_ROWS 1000
-#endif
-// Fused Dice counters (NDICE > 0).  1 (product): every consumer thread keeps its packed 8-bit counters in registers ACROSS
-// tiles.  The producer marks the tiles after which they must be handed over (the CTA's next tile belongs to another image
-// or does not exist, or a field could overflow); only on a marked tile do the consumer warps reduce their counters into
-// their slice of the stage's label row, and the producer warp adds the 8 warps' numbers to the global int64 counters --
-// a handful of times per CTA, nothing Dice-related in the other tiles but the per-pixel arg-max.
-// 0: the first scheme (EVERY tile: 1 + 2*NDICE warp reductions into the label row, folded into registers by the producer),
-// kept for the A/B (tools/kbench_tile.cu -DDCT_DICE_LOCAL=0).  Measured (profiles/r19, r20): per-tile fold 41.9 us at c2;
-// consumer warps adding to global memory themselves 41.6 us at c2 but +1 us at c1 / +2.7 us at c3-sized inputs (8x the
-// atomics on a few dozen addresses at the kernel's end); marked tiles: see profiles/r20/kbench_dice_ab.log.
-#ifndef DCT_DICE_LOCAL
-#define DCT_DICE_LOCAL 1
-#endif
+// Fused Dice counters (NDICE > 0): every consumer thread keeps its packed 8-bit counters in registers ACROSS tiles.  The
+// producer marks the tiles after which they must be handed over (the CTA's next tile belongs to another image or does not
+// exist, or a field could overflow); only on a marked tile do the consumer warps reduce their counters into their slice of
+// the stage's label row, and the producer warp adds the 8 warps' numbers to the global int64 counters -- a handful of
+// times per CTA, nothing Dice-related in the other tiles but the per-pixel arg-max.  Measured (profiles/r19, r20): a fold
+// through the producer on EVERY tile 41.9 us at c2; consumer warps adding to global memory themselves 41.6 us at c2 but
+// +1 us at c1 / +2.7 us at c3-sized inputs (8x the atomics on a few dozen addresses at the kernel's end); marked tiles:
+// see profiles/r20/kbench_dice_ab.log.
 // (An experiment that handed the last level(s) of the tail pool out as 2 or 4 sub-tiles per tile -- to shrink the CTAs' end
 // spread below one tile's service time -- was measured and removed: the extra indirection in the tile loop cost far more
 // than the tail it saved: c2 step 106.2 -> 124.2 (2 sub-tiles) / 136.4 us (4), c4 1.385 -> 1.738 ms; profiles/r26/ab_split.log.)
-// 1 (product): stages of C > 4 shapes whose tile is one box are moved by tensor-map TMA; 0: row copies everywhere (A/B builds)
-#ifndef DCT_TMAP
-#define DCT_TMAP 1
-#endif
-// 1 (product): 5..16-row stages (ACDC: K*C = 8..16, the KL family) run as 256-pixel tiles through tensor maps, 4 consumer warps,
-// 3 CTAs/SM; 0: the round-1 shape (512-pixel tiles, 8 warps, 2 CTAs/SM, row copies) for A/B builds
-#ifndef DCT_SMALL_TMAP
-#define DCT_SMALL_TMAP 1
-#endif
 constexpr int kTileMaxTensors = 8;
 constexpr int kTileMaxRows = 80;   // NIN*C rows per stage
 
@@ -140,9 +118,9 @@ struct TileArgs {
     int num_tiles;
     unsigned int tpi_mul;          // tile / tiles_per_image without a division (tile_set_geometry): q = (t + ((n - t) >> tpi_sh1)) >> tpi_sh2,
     int tpi_sh1, tpi_sh2;          //   t = umulhi(tpi_mul, n) -- exact for every 32-bit n
-    int refill;                    // 1: a drained stage is refilled as soon as ITS OWN store group has been read (DCT_TILE_REFILL); 0: one tile later
-    int pool_div;                  // developer knob: the tail pool is 1/pool_div of every CTA's range (0 = default 5)
-    int prefetch;                  // tiles of this CTA's range whose rows are prefetched into L2 before the dependency wait (DCT_TILE_PREFETCH)
+    int refill;                    // 1: a drained stage is refilled as soon as ITS OWN store group has been read; 0: one tile later
+    int pool_div;                  // developer switch (tools/kbench_*.cu): the tail pool is 1/pool_div of every CTA's range (0 = default 5)
+    int prefetch;                  // tiles of this CTA's range whose rows are prefetched into L2 before the dependency wait
     int force_static;              // developer switch (tools/kbench_tile.cu): 1 = no tail pool (purely static contiguous ranges) even with a workspace
     unsigned long long* trace;     // developer tracing: kTraceSlots words per CTA (start, first tile landed, -, end) in ns; null in the product
 };
@@ -168,11 +146,6 @@ template <class Op, class = void>
 struct op_conf : std::false_type {};
 template <class Op>
 struct op_conf<Op, std::enable_if_t<Op::CONF>> : std::true_type {};
-// does the op provide a shared-memory-resident ("streaming") body for stages too wide for registers?
-template <class Op, class = void>
-struct op_stream : std::false_type {};
-template <class Op>
-struct op_stream<Op, std::enable_if_t<Op::STREAM_CAPABLE>> : std::true_type {};
 template <class Op>
 constexpr bool op_label_row() { return Op::NDICE > 0 || op_labels<Op>::value || op_conf<Op>::value; }
 
@@ -248,7 +221,7 @@ inline void tile_set_geometry(TileArgs& a, int64_t B, int tile_pixels) {
 //       bulk load / store, and recycles a stage when its `done` mbarrier (NCW arrivals) has completed and, for ops
 //       with outputs, when the bulk store group that drains it has finished reading shared memory.  Fused Dice: lane 0
 //       marks the last tile of every run of one image (s_info.w); on those tiles all 32 lanes add the counters the
-//       consumer warps hand over through the label row to the global int64 counters (see DCT_DICE_LOCAL above).
+//       consumer warps hand over through the label row to the global int64 counters (see "Fused Dice counters" above).
 //   consumers: wait on the stage's `full` mbarrier (transaction bytes), read the stage's info word (tile -1 = no more work),
 //       compute in registers, write results back in place, fence to the async proxy, arrive on `done`.
 //       No CTA-wide barrier in the tile loop: a fast warp runs ahead by up to STAGES-1 tiles.
@@ -262,12 +235,8 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
     constexpr int CTHREADS = NCW * 32;
     using Cfg = TileCfg<Op, CT, PPT, CTHREADS, STAGES, ET, TMAP>;
     constexpr int TP = Cfg::TP, ROWS = Cfg::ROWS, ES = Cfg::ES, NIN = Op::NIN, NOUT = Op::NOUT, C = CT;
-    constexpr bool DICE = Op::NDICE > 0;
-    constexpr bool DICE_LOCAL = DICE && (DCT_DICE_LOCAL != 0);   // counters live in the consumers' registers across tiles
-    constexpr bool DICE_FOLD = DICE && !DICE_LOCAL;               // per-tile fold through the label row by the producer warp
+    constexpr bool DICE = Op::NDICE > 0;         // fused Dice counts (see "Fused Dice counters" above)
     constexpr bool LAB = op_labels<Op>::value;   // the op consumes the labels itself
-    // > 40 fp32 rows per pixel do not fit the register file as a pixel pair: ops that can, work on the stage in place
-    constexpr bool STREAM = op_stream<Op>::value && ROWS >= DCT_STREAM_MIN_ROWS && PPT <= 2 && std::is_same<ET, float>::value && !TMAP;
     constexpr bool CONF = op_conf<Op>::value;    // confusion counts of tensor 0 vs the labels (CTA-shared histogram)
     constexpr bool LROW = DICE || LAB || CONF;   // the stage carries a label row
     constexpr int LW = (PPT % 2 == 0) ? 2 : 1;   // pixels per math lane group: pairs use packed FP32x2
@@ -281,7 +250,7 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
     uint64_t* done = full + STAGES;
     // per stage, written by the producer lane before the stage's `full` barrier is armed: x = tile index held by the stage
     // (-1 = end of work), y = its image, z = its pixel count (a ragged last tile of an image is shorter than TP),
-    // w = DICE_LOCAL: 1 = hand the Dice counters over after this tile
+    // w = Dice: 1 = hand the Dice counters over after this tile
     __shared__ int4 s_info[STAGES];
     __shared__ unsigned int s_conf[CONF ? CT * CT : 1];   // this CTA's confusion counts (flushed once, at the end)
     const int tid = threadIdx.x, lane = tid & 31;
@@ -396,7 +365,7 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
             ++draws;
             return t;
         };
-        int run_b = -1, run_len = 0;               // DICE_LOCAL: image and length of the current run of tiles (lane 0)
+        int run_b = -1, run_len = 0;               // Dice: image and length of the current run of tiles (lane 0)
         constexpr int kDiceMaxTiles = 255 / PPT;   // a packed 8-bit field grows by at most PPT per tile
         int issued = 0;        // loads issued so far; the k-th goes to stage k % STAGES
         bool more = true;
@@ -413,7 +382,7 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
             pending = draw();
             const int b = tile_image(a, tile);
             int mark = 0;
-            if constexpr (DICE_LOCAL) {
+            if constexpr (DICE) {
                 // last tile of a run of one image (or of this CTA's work), or the run is as long as an 8-bit field allows
                 run_len = (b == run_b) ? run_len + 1 : 1;
                 run_b = b;
@@ -450,14 +419,10 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
             }
             ++issued;
         };
-        // Dice: producer lane r (and r + 32) owns counter r = (view, class, kind).  DICE_LOCAL: it adds what the consumer
-        // warps hand over on a marked tile straight to the global int64 counters; DICE_FOLD: it keeps the counter of the
-        // image being processed in a register, fed on every tile, and adds it to the global counter when the image changes
-        // (integer atomics either way: order-independent)
+        // Dice: producer lane r (and r + 32) owns counter r = (view, class, kind): it adds what the consumer warps hand over
+        // on a marked tile straight to the global int64 counters (integer atomics: order-independent)
         constexpr int kDiceCounters = DICE ? Op::NDICE * C * 3 : 0;
         constexpr int kDiceRounds = (kDiceCounters + 31) / 32;
-        unsigned int dacc[kDiceRounds > 0 ? kDiceRounds : 1] = {};
-        int cur_b = -1;
         bool counts_ready = !(DICE && do_dice && a.counts_overwrite) || blockIdx.x == 0;   // CTA 0 cleared them itself
         auto await_counts = [&]() {   // all lanes; once per CTA, right before its first add to the global counters
             if (!counts_ready) {
@@ -466,20 +431,6 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
                     asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(z) : "l"(&a.ws->counts_zeroed) : "memory");
                 } while (z == 0u);
                 counts_ready = true;
-            }
-        };
-        auto flush_dice = [&](int bb) {
-            if constexpr (DICE_FOLD) {
-                await_counts();
-#pragma unroll
-                for (int rr = 0; rr < kDiceRounds; ++rr) {
-                    const int r = rr * 32 + lane;
-                    if (r < kDiceCounters && dacc[rr] != 0u) {
-                        const int n = r / (C * 3), rc = r - n * C * 3;
-                        atomicAdd(a.counts + (int64_t)n * a.count_view_stride + (int64_t)bb * C * 3 + rc, (unsigned long long)dacc[rr]);
-                    }
-                    dacc[rr] = 0u;
-                }
             }
         };
         if (lane == 0) {
@@ -500,16 +451,13 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
             tma::mbar_wait(&done[stage], (uint32_t)(i / STAGES) & 1u);  // every consumer warp is through with load i
             const int4 info = s_info[stage];
             const int tile = info.x, b = info.y;
-            // Dice counts of this tile: every consumer warp left its warp-reduced packed counters (8-bit fields,
-            // word 0 = |gt==c|, words 1+2n / 2+2n = I / P of view n) in its own slice of the stage's label row; the
-            // 32 producer lanes sum one (view, class, kind) counter each over the warps (before the stage is refilled)
-            // and, AFTER this iteration's copies have been issued, add it to their per-image registers (any global
-            // atomics of an image change then never sit in front of the release of the refill's barrier arrive).
+            // Dice counts handed over on a marked tile: every consumer warp left 2 * (1 + 2*NDICE) words of 16-bit fields
+            // (classes 0,2 / 1,3 of |gt==c|, then I / P of every view) in its slice of the stage's label row; lane r sums
+            // counter r over the warps (before the stage is refilled) and, AFTER this iteration's copies have been issued,
+            // adds it to the global counter (the atomics then never sit in front of the release of the refill's barrier arrive).
             unsigned int dsum[kDiceRounds > 0 ? kDiceRounds : 1];
             bool hand_over = false;
-            if constexpr (DICE_LOCAL) {
-                // marked tile: every consumer warp left 2 * (1 + 2*NDICE) words of 16-bit fields (classes 0,2 / 1,3 of
-                // |gt==c|, then I / P of every view) in its slice of the label row; lane r sums counter r over the warps
+            if constexpr (DICE) {
                 hand_over = do_dice && info.w != 0;   // written by lane 0 at issue time (a __syncwarp() ago)
                 if (hand_over) {
                     const unsigned int* pkw = reinterpret_cast<const unsigned int*>(stages + (size_t)stage * Cfg::kStageBytes + Cfg::kLabelOffB);
@@ -522,23 +470,6 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
                             const int widx = kind == 1 ? 0 : (kind == 0 ? 1 + 2 * n : 2 + 2 * n);
 #pragma unroll
                             for (int w = 0; w < NCW; ++w) sum += (pkw[w * 64 * PPT + 2 * widx + (c & 1)] >> (16 * (c >> 1))) & 0xffffu;
-                        }
-                        dsum[rr] = sum;
-                    }
-                }
-            }
-            if constexpr (DICE_FOLD) {
-                if (do_dice) {
-                    const unsigned int* pkw = reinterpret_cast<const unsigned int*>(stages + (size_t)stage * Cfg::kStageBytes + Cfg::kLabelOffB);
-#pragma unroll
-                    for (int rr = 0; rr < kDiceRounds; ++rr) {
-                        const int r = rr * 32 + lane;
-                        unsigned int sum = 0u;
-                        if (r < kDiceCounters) {
-                            const int n = r / (C * 3), rc = r - n * C * 3, c = rc / 3, kind = rc - c * 3;
-                            const int widx = kind == 1 ? 0 : (kind == 0 ? 1 + 2 * n : 2 + 2 * n);
-#pragma unroll
-                            for (int w = 0; w < NCW; ++w) sum += (pkw[w * 64 * PPT + widx] >> (8 * c)) & 0xffu;
                         }
                         dsum[rr] = sum;
                     }
@@ -579,7 +510,7 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
                     try_issue();
                 }
             }
-            if constexpr (DICE_LOCAL) {
+            if constexpr (DICE) {
                 if (hand_over) {   // uniform across the warp; after this iteration's copies have been issued
                     await_counts();
 #pragma unroll
@@ -592,20 +523,7 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
                     }
                 }
             }
-            if constexpr (DICE_FOLD) {
-                if (do_dice) {
-                    if (b != cur_b) {  // uniform across the warp
-                        if (cur_b >= 0) flush_dice(cur_b);
-                        cur_b = b;
-                    }
-#pragma unroll
-                    for (int rr = 0; rr < kDiceRounds; ++rr) dacc[rr] += dsum[rr];
-                }
-            }
             __syncwarp();
-        }
-        if constexpr (DICE_FOLD) {
-            if (do_dice && cur_b >= 0) flush_dice(cur_b);
         }
         if constexpr (NOUT > 0) {
             if (lane == 0) tma::bulk_wait_all<0>();
@@ -622,7 +540,7 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
         if constexpr (Op::USES_UP) gs = upstream_scalar(a.up);
         int nbad_label = 0;
         // Dice: packed 8-bit per-class counters of this thread, [view][I,P], and |gt == c| (the same for every view).
-        // DICE_LOCAL: they live across tiles until the producer marks a tile (s_info.w); DICE_FOLD: they are one tile's.
+        // They live across tiles until the producer marks a tile (s_info.w).
         unsigned int pk[DICE ? Op::NDICE : 1][2] = {};
         unsigned int pkG = 0u;
 #pragma unroll 1
@@ -634,30 +552,14 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
             if (a.trace != nullptr && i == 0 && tid == 0) a.trace[kTraceSlots * blockIdx.x + 1] = globaltimer_ns();
             if (tile < 0) break;
             const int b = info.y;
-            const bool hand_over = DICE_LOCAL && do_dice && info.w != 0;   // uniform across the CTA's consumers
+            const bool hand_over = do_dice && info.w != 0;   // uniform across the CTA's consumers
             const int64_t off = (int64_t)(tile - b * tpi) * TP;
             const int len = info.z;
             unsigned char* st = stages + (size_t)stage * Cfg::kStageBytes;
             const int p0 = tid * PPT;
             const bool active = p0 < len;
             const unsigned int amask = CONF ? __ballot_sync(0xffffffffu, active) : 0u;  // lanes that enter the block below
-            if constexpr (DICE_FOLD) {
-                pkG = 0u;
-#pragma unroll
-                for (int n = 0; n < Op::NDICE; ++n) pk[n][0] = pk[n][1] = 0u;
-            }
-            if constexpr (STREAM) {
-                if (active) {
-                    const T mv = Op::template stream<C, T>(st, Cfg::kRowBytes, p0, gs);
-                    acc_fx += to_fixed(vhsum(mv), nonfinite);
-                    if (a.map != nullptr) {
-                        FVec<PPT> mapv;
-#pragma unroll
-                        for (int v = 0; v < PPT; ++v) mapv.v[v] = vget(mv, v);
-                        st_stream<PPT>(a.map + (int64_t)b * HW + off + p0, mapv);
-                    }
-                }
-            } else if (active) {
+            if (active) {
                 FVec<PPT> gm;
 #pragma unroll
                 for (int v = 0; v < PPT; ++v) gm.v[v] = 1.0f;
@@ -818,7 +720,7 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
             }
             if constexpr (NOUT > 0) tma::fence_proxy_async_smem();
             __syncwarp();
-            if constexpr (DICE_LOCAL) {
+            if constexpr (DICE) {
                 if (hand_over) {
                     // widen every packed word into two words of 16-bit fields (classes 0,2 and 1,3; 32 lanes * 255 < 2^16),
                     // reduce them across the warp (REDUX) and leave them in the warp's slice of the label row (its labels
@@ -838,24 +740,6 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
                     pkG = 0u;
 #pragma unroll
                     for (int n = 0; n < Op::NDICE; ++n) pk[n][0] = pk[n][1] = 0u;
-                    __syncwarp();
-                }
-            }
-            if constexpr (DICE_FOLD) {
-                if (do_dice) {
-                    // every packed field is <= 32 lanes * PPT < 256, so the packed words are reduced across the warp as
-                    // they are (REDUX); the warp's labels have all been read, so its slice of the label row is free
-                    const unsigned int wG = __reduce_add_sync(0xffffffffu, pkG);
-                    unsigned int mine = wG;
-#pragma unroll
-                    for (int n = 0; n < Op::NDICE; ++n) {
-                        const unsigned int ri = __reduce_add_sync(0xffffffffu, pk[n][0]);
-                        const unsigned int rp = __reduce_add_sync(0xffffffffu, pk[n][1]);
-                        if (lane == 1 + 2 * n) mine = ri;
-                        if (lane == 2 + 2 * n) mine = rp;
-                    }
-                    if (lane < 1 + 2 * Op::NDICE)
-                        reinterpret_cast<unsigned int*>(st + Cfg::kLabelOffB)[(tid >> 5) * 64 * PPT + lane] = mine;
                     __syncwarp();
                 }
             }
@@ -911,8 +795,11 @@ int tile_launch_ct(TileArgs a, int64_t B, cudaStream_t stream) {
     // consumer warps are latency-bound (ncu: 21% issue-slot use with one warp per scheduler), so the shape must put
     // >= 6 consumer warps on an SM while keeping >= 3 stages for ops with outputs (2 stages stall on the store drain);
     // two small CTAs per SM beat one large CTA (two independent producers).
-    //   rows <= 4        4 pixels/thread, 8 consumer warps, 2 CTAs/SM (Dice counting, spleen K = C = 2)
-    //   rows <= 16       2 pixels/thread (ACDC: K*C = 8..16, the KL family), 8 warps, 2 CTAs/SM, 4..7 stages
+    //   rows <= 4        4 pixels/thread, 8 consumer warps, 2 CTAs/SM, row copies (Dice counting, spleen K = C = 2)
+    //   5 <= rows <= 16  ACDC: K*C = 8..16, the KL family: tiles of 256 pixels (2 pixels/thread, 4 consumer warps), 3 CTAs/SM,
+    //                    one tensor-map box per tensor instead of C row copies: 3 independent producers per SM, 7 copies per
+    //                    tile instead of 25 at c2 (round 1: 512-pixel tiles, 8 warps, 2 CTAs/SM, row copies;
+    //                    profiles/r35/kbench_small.log: c2 JSD+Dice 40.9 -> 39.4 us, KL 25.4 -> 24.8, c1 9.4 -> 8.7)
     //   rows <= 24       one C = 19 tensor (cross-entropy): 4 warps, 2 CTAs/SM, 5 stages        (99% of the copy peak)
     //   rows <= 40       Cityscapes C = 19 with 2 tensors: 3 warps, 2 CTAs/SM, 3 stages           (JSD 4449 -> 5930 GB/s)
     //                    read-only ops: 8 warps, 1 CTA/SM, 2 stages
@@ -920,19 +807,16 @@ int tile_launch_ct(TileArgs a, int64_t B, cudaStream_t stream) {
     //                    (profiles/r08/kbench_wide_reg.log: 5244 GB/s against 4641 for the pixel-pair shape)
     //   rows <= 80       K = 4, C = 19: one pixel/thread, 7 warps, 1 CTA/SM, 3 stages of 68 KB (the most that fits)
     //                    (profiles/r09/kbench_wide_more.log: 4245 GB/s; 6 warps 3750, 2 x 3 warps 3744, 5 warps x 4 stages 3205)
-    //   DCT_STREAM_MIN_ROWS (off by default): ops with a shared-memory-resident body work on the stage in place; measured
-    //                    equal or slower than the register-resident body at every shape (profiles/r08/kbench_wide_stream.log)
-    //   5 <= rows <= 16  (round 2, DCT_SMALL_TMAP) tiles of 256 pixels, 4 consumer warps, 3 CTAs/SM, one tensor-map box per tensor
-    //                    instead of C row copies: 3 independent producers per SM, 7 copies per tile instead of 25 at c2
-    //                    (profiles/r35/kbench_small.log: c2 JSD+Dice 40.9 -> 39.4 us, KL 25.4 -> 24.8, c1 9.4 -> 8.7)
-    constexpr bool SMALL = (DCT_TMAP != 0) && (DCT_SMALL_TMAP != 0) && ROWS > 4 && ROWS <= 16;
+    // (A shared-memory-resident JSD body for the > 40-row stages measured equal or slower than the register-resident one at
+    // every shape and was removed: profiles/r08/kbench_wide_stream.log.)
+    constexpr bool SMALL = ROWS > 4 && ROWS <= 16;
     constexpr int PPT = ROWS <= 4 ? 4 : (ROWS <= 40 ? 2 : 1);
-    constexpr int NCW = SMALL ? 4 : (ROWS <= 16 ? 8 : (ROWS <= 24 ? 4 : (ROWS <= 40 ? (Op::NOUT == 0 ? 8 : 3) : (ROWS <= 60 ? 5 : 7))));
+    constexpr int NCW = ROWS <= 4 ? 8 : (ROWS <= 24 ? 4 : (ROWS <= 40 ? (Op::NOUT == 0 ? 8 : 3) : (ROWS <= 60 ? 5 : 7)));
     constexpr int MINB = SMALL ? 3 : (ROWS <= 24 ? 2 : (ROWS <= 40 ? (Op::NOUT == 0 ? 1 : 2) : (ROWS <= 60 ? 2 : 1)));
     constexpr int TPX = NCW * 32 * PPT;
     // stages whose tile is one box (<= 256 pixels): tensor-map TMA, one copy per tensor instead of one per row -- the wide
-    // C = 19 stages (round 1) and the small ACDC-sized ones
-    constexpr bool TMAP = (DCT_TMAP != 0) && (CT > 4 || SMALL) && TPX <= 256;
+    // C = 19 stages and the small ACDC-sized ones
+    constexpr bool TMAP = (CT > 4 || SMALL) && TPX <= 256;
     // bf16 tensors: same shapes (the register budget follows the number of rows, not their width); the 2-byte rows
     // simply buy more stages
     constexpr int STAGES = tile_stages<tile_stage_bytes<Op, CT, TPX, ET, TMAP>(), MINB>();
@@ -956,21 +840,15 @@ int tile_launch_ct(TileArgs a, int64_t B, cudaStream_t stream) {
         if (devid >= 0 && devid < 64) configured[devid] = true;
     }
     tile_set_geometry(a, B, Cfg::TP);
-    {   // schedule knobs (developer A/B through the environment; the defaults are the measured product choice)
-        static const int env_pool = [] { const char* e = std::getenv("DCT_TILE_POOL_DIV"); return e ? std::atoi(e) : 0; }();
-        static const int env_pre = [] { const char* e = std::getenv("DCT_TILE_PREFETCH"); return (e && *e) ? std::atoi(e) : -1; }();
-        // 2 tiles per CTA (measured, profiles/r30/ab_prefetch.log: c2 step 102.3 -> 101.9 us, c3 52.6 -> 51.8, c1 11.3 -> 10.5).
-        // Deeper (3..4) makes the KL launches faster when timed alone (c2 kl_logit 19.0 -> 18.5 us) but not the chained step
-        // (91.6 -> 91.6 / 91.9 us) and costs the JSD launch at c3 (12.9 -> 13.3 us): profiles/r39/ab_env.log, r42/ab_refill.log
-        a.prefetch = env_pre >= 0 ? env_pre : 2;
-        static const int env_refill = [] { const char* e = std::getenv("DCT_TILE_REFILL"); return (e && *e) ? std::atoi(e) : -1; }();
-        // Measured (profiles/r34/ab_refill.log): immediate refill pays where the store group is a fraction of the stage and the
-        // stages are few -- the C = 19 KL kernels (2-3 tensors in, 1 out, 3 stages): c4 kl_adv 324 -> 305 us, kl_logit 301 -> 296;
-        // it costs where the store drains the whole stage (JSD: c4 407 -> 418 us, c2 37.5 -> 37.9: the producer lane sits in
-        // the read wait); on the short c2 / c3 KL launches it is neutral within 0.3 us either way (profiles/r42/ab_refill.log)
-        a.refill = env_refill >= 0 ? env_refill : ((TMAP && Op::NOUT < Op::NIN) ? 1 : 0);
-        if (env_pool > 0 && a.pool_div == 0) a.pool_div = env_pool;
-    }
+    // L2 prefetch of 2 tiles per CTA (measured, profiles/r30/ab_prefetch.log: c2 step 102.3 -> 101.9 us, c3 52.6 -> 51.8, c1 11.3
+    // -> 10.5).  Deeper (3..4) makes the KL launches faster when timed alone (c2 kl_logit 19.0 -> 18.5 us) but not the chained
+    // step (91.6 -> 91.6 / 91.9 us) and costs the JSD launch at c3 (12.9 -> 13.3 us): profiles/r39/ab_env.log, r42/ab_refill.log
+    a.prefetch = 2;
+    // Measured (profiles/r34/ab_refill.log): immediate refill pays where the store group is a fraction of the stage and the
+    // stages are few -- the C = 19 KL kernels (2-3 tensors in, 1 out, 3 stages): c4 kl_adv 324 -> 305 us, kl_logit 301 -> 296;
+    // it costs where the store drains the whole stage (JSD: c4 407 -> 418 us, c2 37.5 -> 37.9: the producer lane sits in
+    // the read wait); on the short c2 / c3 KL launches it is neutral within 0.3 us either way (profiles/r42/ab_refill.log)
+    a.refill = (TMAP && Op::NOUT < Op::NIN) ? 1 : 0;
     int grid = kSMs * MINB;
     if (grid > a.num_tiles) grid = a.num_tiles;
     if (a.trace == nullptr) a.trace = trace_next(grid);

@@ -63,7 +63,7 @@ inline EncodeTiledFn encode_tiled_fn() {
 }
 
 // Tensor map of one contiguous [B, C, HW] tensor of `es`-byte elements (4: float32, 2: bfloat16) with box [box_w, C, 1].
-// false: the driver entry point is missing or refused the shape (the caller takes the row-copy path).
+// false: the driver entry point is missing or refused the shape (tile_launch_ct then launches nothing: DCT_ERR_UNSUPPORTED).
 // Descriptors are pure functions of (pointer, element size, shape, box): a training loop presents the same few tensors'
 // addresses step after step (caching allocator), so the last encodings are kept per host thread and a launch outside a
 // CUDA graph pays a 128-byte copy instead of a driver call per tensor.

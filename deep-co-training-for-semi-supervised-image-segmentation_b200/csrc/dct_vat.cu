@@ -13,8 +13,6 @@
 // workspace, then rescale; the second read is served by the 126 MB L2).
 #include <cooperative_groups.h>
 
-#include <cstdlib>
-
 #include "dct_common.cuh"
 
 namespace cg = cooperative_groups;
@@ -36,7 +34,7 @@ struct L2Args {
     float* adv;        // nullable
     Workspace* ws;
     unsigned long long* trace;   // developer tracing (dct_common.cuh, trace_next); null in the product
-    int prefetch;                // 1: the sample's lines are pulled into L2 before the dependency wait (DCT_L2_PREFETCH)
+    int prefetch;                // 1: the sample's lines are pulled into L2 before the dependency wait
 };
 
 __device__ __forceinline__ float block_sum_f(float v, float* s_warp) {
@@ -304,12 +302,6 @@ static bool l2_ll_try(const L2Args& a, int64_t B, int cps, cudaStream_t s, cudaE
     return true;
 }
 
-// 0 = product choice; 1 = cluster kernels only; 2 = prefer the cluster-free kernel wherever it is eligible (developer A/B)
-static int l2_variant() {
-    static const int v = [] { const char* e = std::getenv("DCT_L2_VARIANT"); return e ? std::atoi(e) : 0; }();
-    return v;
-}
-
 // ---- large / odd samples: two grid-wide launches through the workspace ------------------------------------------------
 // Workspace layout of this path: sample b owns gx + 1 doubles: [0, gx) one partial per CTA of its row of the grid, [gx] the
 // sample's sum of squares (as the float the scale launch works with).  The CTA that draws the last ticket of the first
@@ -460,16 +452,15 @@ extern "C" int dct_l2_normalize_f32(const float* d, float* out, int64_t B, int64
     if ((img == nullptr) != (adv == nullptr)) return DCT_ERR_BAD_ARG;
     if (!aligned(d, 4) || !aligned(out, 4) || !aligned(img, 4) || !aligned(adv, 4)) return DCT_ERR_MISALIGNED;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    static const int env_pre = [] { const char* e = std::getenv("DCT_L2_PREFETCH"); return e ? std::atoi(e) : 1; }();   // on: c2 l2 launches 5.93 -> 5.47 / 9.95 -> 8.64 us (profiles/r30)
-    L2Args a{d, out, M, passes, scale, img, adv, static_cast<Workspace*>(workspace), nullptr, env_pre};
+    // prefetch on: c2 l2 launches 5.93 -> 5.47 / 9.95 -> 8.64 us (profiles/r30)
+    L2Args a{d, out, M, passes, scale, img, adv, static_cast<Workspace*>(workspace), nullptr, 1};
     const bool vec_ok = (M % 4) == 0 && aligned(d, 16) && aligned(out, 16) && aligned(img, 16) && aligned(adv, 16);
     // Which one-launch kernel (measured in the c2 / c3 steps, profiles/r24, r25): samples up to 512 KB -> one cluster of 8
     // CTAs (its exchange stays in distributed shared memory; the cluster-free kernel's tagged words go through an L2 that is
     // busy writing back the previous launch's gradients: 10.6 vs 13.5 us inside the c2 step); 512 KB - 1 MB -> the
     // cluster-free kernel (twice the CTAs of a 16-CTA cluster per sample: c3 step 61.0 vs 64.7 us), then the cluster of 16.
     const int64_t nv8 = (M + (int64_t)kL2Cluster * kL2Threads * 4 - 1) / ((int64_t)kL2Cluster * kL2Threads * 4);
-    const bool ll_first = l2_variant() == 2 || (l2_variant() == 0 && nv8 > kL2MaxVecPerThread);
-    if (vec_ok && workspace != nullptr && B <= kL2LLSamples && ll_first) {
+    if (vec_ok && workspace != nullptr && B <= kL2LLSamples && nv8 > kL2MaxVecPerThread) {
         // cluster-free one-launch kernel: cps CTAs of 256 threads per sample, <= 8 float4 per thread, and as many more CTAs
         // (fewer float4 each) as still fit one co-resident wave
         const int64_t nvec = M / 4;

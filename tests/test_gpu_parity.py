@@ -509,7 +509,7 @@ def test_full_size_properties(K, C, B, H, W, dct, dev):
 
 
 # ---------------------------------------------------------------------------------------------
-# Dice counters kept in registers across tiles (csrc/dct_tile.cuh, DCT_DICE_LOCAL): images so large that one CTA works
+# Dice counters kept in registers across tiles (csrc/dct_tile.cuh, "Fused Dice counters"): images so large that one CTA works
 # through hundreds of tiles of the SAME image, so the packed 8-bit fields must be flushed before they overflow
 # (every 255 / pixels-per-thread tiles), plus a ragged last tile and a batch of 1 (fewer flushes than warps)
 # ---------------------------------------------------------------------------------------------
@@ -545,8 +545,8 @@ def test_dice_counters_long_runs_of_one_image(C, B, H, W, dct, dev):
 
 
 # ---------------------------------------------------------------------------------------------
-# K*C > 40 (K = 3, 4 at C = 19): the shared-memory-resident JSD body (jsd_stream_pair) -- ragged tails, saturated
-# logits whose exponentials underflow to zero, identical views, confident and agreeing inputs
+# K*C > 40 (K = 3, 4 at C = 19): the one-pixel-per-thread tile shapes, whose K*C values fill most of the register file --
+# ragged tails, saturated logits whose exponentials underflow to zero, identical views, confident and agreeing inputs
 # ---------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("K", [3, 4])
 @pytest.mark.parametrize("variant", ["plain", "confident", "agreeing", "saturated", "identical"])

@@ -3,9 +3,6 @@
 #   tools/gpu_call.sh <tag> [sections...]     sections: tests tests:<file> smoke bench bench:<workload> refarm ncu_list[:<workload>]
 #                                             ncu_full:<workload>:<demangled-name regex> sh:<script> py:<script>
 #                                             quick[:<workloads,>]            per-launch times of the steps (no extras), twice each
-#                                             ab:<ENVVAR>:<v1,v2,..>[:<workloads,>]  the same under every value of a developer knob
-#                                                                              (DCT_TILE_REFILL, DCT_TILE_POOL_DIV, DCT_TILE_PREFETCH,
-#                                                                              DCT_L2_VARIANT, DCT_L2_PREFETCH; "unset" = product rule)
 #                                             kb:<group>                      tools/kbench_c2 (0: c2 launches + per-CTA dump, 1: c3 / c1 shapes)
 #                                             multi                           both bench arms under torch.distributed.run on all visible GPUs
 #                                             extras                          configs[4] sweep, sanitizer memcheck, step timeline
@@ -31,10 +28,6 @@ for sec in "$@"; do
     ncu_list:*) w=${sec#ncu_list:}; timeout 600 ncu --metrics gpu__time_duration.sum --clock-control none -c 300 --csv --log-file $out/ncu_launches_bench_$w.csv python bench.py --workload $w --steps 8 --warmup 4 --no-extras --no-cpu-baseline --e2e-steps 3 > $out/ncu_list_bench_$w.log 2>&1; grep -c dct $out/ncu_launches_bench_$w.csv ;;
     ncu_full:*) spec=${sec#ncu_full:}; w=${spec%%:*}; k=${spec#*:}; timeout 900 ncu --set full --clock-control none --import-source on --kernel-name-base demangled -k regex:$k -s 6 -c 2 -o $out/ncu_full_${w}_$(echo $k | tr -cd 'A-Za-z0-9_') -f python bench.py --workload $w --steps 8 --warmup 4 --no-extras --no-cpu-baseline --e2e-steps 3 > $out/ncu_full_${w}.log 2>&1; ls -la $out/*.ncu-rep ;;
     quick|quick:*) wls=${sec#quick}; wls=${wls#:}; for wl in $(echo ${wls:-c2,c3,c1,c4} | tr ',' ' '); do for rep in 1 2; do quick_bench $wl | step_line "$wl"; done; done | tee $out/bench_quick.log ;;
-    ab:*)     spec=${sec#ab:}; var=${spec%%:*}; rest=${spec#*:}; vals=${rest%%:*}; wls=c2,c3,c4; [ "$rest" != "$vals" ] && wls=${rest#*:}
-              for wl in $(echo $wls | tr ',' ' '); do for rep in 1 2; do for v in $(echo $vals | tr ',' ' '); do
-                if [ $v = unset ]; then quick_bench $wl; else env $var=$v bash -c "$(declare -f quick_bench); quick_bench $wl"; fi | step_line "$wl $var=$v"
-              done; done; done | tee $out/ab_$var.log ;;
     kb:*)     g=${sec#kb:}; [ $g = 0 ] && ( KB_DUMP=1 timeout 100 tools/kbench_c2 200 0 0 2>&1 ) > $out/kbench_c2_dump.log
               ( timeout 200 tools/kbench_c2 200 -1 $g 2>&1 ) > $out/kbench_c2_g$g.log; grep -v "^ " $out/kbench_c2_g$g.log ;;
     multi)    N=$(nvidia-smi -L | wc -l)

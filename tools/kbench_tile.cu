@@ -281,27 +281,6 @@ int main(int argc, char** argv) {
         run_auto<CF, 19, 4, 4, 2>("cefwd C19", B, HWc, reps, 84, true);
         run_auto<CF, 19, 2, 8, 1>("cefwd C19", B, HWc, reps, 84, true);
     }
-    if (which == 6) {  // K*C > 40: register-resident vs shared-memory-resident body (build twice: -DDCT_STREAM_MIN_ROWS=41 / 1000)
-        const int64_t HWc = 512 * 1024;
-        using J4 = JsdOp<4, true, kFwdBwd, false>;
-        run_auto<J4, 19, 2, 3, 1>("jsd K4 C19", B, HWc, reps, 608, false);
-        run_auto<J4, 19, 2, 4, 1>("jsd K4 C19", B, HWc, reps, 608, false);
-        run_auto<J4, 19, 2, 2, 2>("jsd K4 C19", B, HWc, reps, 608, false);
-        run_auto<J4, 19, 2, 2, 1>("jsd K4 C19", B, HWc, reps, 608, false);
-        run_auto<J4, 19, 1, 6, 1>("jsd K4 C19", B, HWc, reps, 608, false);
-        run_auto<J4, 19, 1, 8, 1>("jsd K4 C19", B, HWc, reps, 608, false);
-        run_auto<J4, 19, 1, 4, 2>("jsd K4 C19", B, HWc, reps, 608, false);
-        run_auto<J4, 19, 1, 4, 1>("jsd K4 C19", B, HWc, reps, 608, false);
-        using J3 = JsdOp<3, true, kFwdBwd, false>;
-        run_auto<J3, 19, 2, 4, 1>("jsd K3 C19", B, HWc, reps, 456, false);
-        run_auto<J3, 19, 2, 5, 1>("jsd K3 C19", B, HWc, reps, 456, false);
-        run_auto<J3, 19, 2, 3, 1>("jsd K3 C19", B, HWc, reps, 456, false);
-        run_auto<J3, 19, 2, 2, 2>("jsd K3 C19", B, HWc, reps, 456, false);
-        run_auto<J3, 19, 1, 8, 1>("jsd K3 C19", B, HWc, reps, 456, false);
-        run_auto<J3, 19, 1, 6, 1>("jsd K3 C19", B, HWc, reps, 456, false);
-        run_auto<J3, 19, 1, 4, 2>("jsd K3 C19", B, HWc, reps, 456, false);
-        run_auto<J3, 19, 1, 5, 2>("jsd K3 C19", B, HWc, reps, 456, false);
-    }
     if (which == 7) {  // K = 4, C = 19: remaining shapes around the r08 winner (one pixel/thread, 6 warps, 3 stages)
         const int64_t HWc = 512 * 1024;
         using J4 = JsdOp<4, true, kFwdBwd, false>;
