@@ -33,7 +33,10 @@ struct Workspace {
     unsigned int counts_zeroed;  // DCT_COUNTS_OVERWRITE: set (release) by CTA 0 once the launch's counters are cleared
     unsigned long long fx_lo;    // order-independent loss sum in 2^-40 fixed point: sum of the low 32 bits ...
     long long fx_hi;             // ... and of the (signed) high bits of every partial
-    unsigned int pad[8];
+    unsigned long long fx2_lo;   // the same for the second sum of a tile op with two map values (Op::SUM2, dct_tile.cuh)
+    long long fx2_hi;
+    unsigned int nonfinite2;
+    unsigned int pad[3];
     double partials[kMaxPartials];
     // per-sample exchange of the one-launch perturbation normalisation (dct_vat.cu, l2_ll_kernel): a launch counter that
     // gives every launch fresh tags, its ticket, and kL2LLSamples x 2 passes x kL2LLSlots self-validating 8-byte words
@@ -287,12 +290,14 @@ __device__ __forceinline__ long long warp_sum(long long v) {
 
 // Called by every thread of the CTA at the end of a tile-pipeline kernel.  `out` may be null.
 // Also re-arms the workspace header (ticket, tile counter, accumulators) when the last CTA is through.
-template <bool PUB = false>
+// SUM2: a second, independent sum (acc_fx2 / nonfinite2 -> ws->fx2_* -> *out2, nullable) with the same scheme.
+template <bool PUB = false, bool SUM2 = false>
 __device__ __forceinline__ void tile_grid_finish(long long acc_fx, bool nonfinite, Workspace* ws, double* out, int num_ctas,
-                                                 const PeerPub* pub = nullptr, int pub_early = 0) {
+                                                 const PeerPub* pub = nullptr, int pub_early = 0, long long acc_fx2 = 0,
+                                                 bool nonfinite2 = false, double* out2 = nullptr) {
     if (ws == nullptr) return;
-    __shared__ long long s_lo[20], s_hi[20];  // <= 17 warps per CTA
-    __shared__ int s_nf;
+    __shared__ long long s_lo[SUM2 ? 40 : 20], s_hi[SUM2 ? 40 : 20];  // <= 17 warps per CTA (second sum at +20)
+    __shared__ int s_nf, s_nf2;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = (blockDim.x + 31) >> 5;
     if (out != nullptr) {
         if (threadIdx.x == 0) s_nf = 0;
@@ -303,8 +308,28 @@ __device__ __forceinline__ void tile_grid_finish(long long acc_fx, bool nonfinit
         __syncthreads();
         if (lane == 0) { s_lo[wid] = lo; s_hi[wid] = hi; if (wnf) s_nf = 1; }
     }
+    if constexpr (SUM2) {
+        if (out2 != nullptr) {
+            if (threadIdx.x == 0) s_nf2 = 0;
+            long long lo = (long long)((unsigned long long)acc_fx2 & 0xffffffffull), hi = acc_fx2 >> 32;
+            lo = warp_sum(lo);
+            hi = warp_sum(hi);
+            const bool wnf = __any_sync(0xffffffffu, nonfinite2);
+            __syncthreads();
+            if (lane == 0) { s_lo[20 + wid] = lo; s_hi[20 + wid] = hi; if (wnf) s_nf2 = 1; }
+        }
+    }
     __syncthreads();
     if (threadIdx.x == 0) {
+        if constexpr (SUM2) {
+            if (out2 != nullptr) {
+                long long lo = 0, hi = 0;
+                for (int w = 0; w < nw; ++w) { lo += s_lo[20 + w]; hi += s_hi[20 + w]; }
+                atomicAdd(&ws->fx2_lo, (unsigned long long)lo);
+                atomicAdd(reinterpret_cast<unsigned long long*>(&ws->fx2_hi), (unsigned long long)hi);
+                if (s_nf2) atomicAdd(&ws->nonfinite2, 1u);
+            }
+        }
         if (out != nullptr) {
             long long lo = 0, hi = 0;
             for (int w = 0; w < nw; ++w) { lo += s_lo[w]; hi += s_hi[w]; }
@@ -326,6 +351,17 @@ __device__ __forceinline__ void tile_grid_finish(long long acc_fx, bool nonfinit
         }
         if (ticket == (unsigned int)num_ctas - 1u) {  // last CTA: publish the sum and re-arm the header
             __threadfence();
+            if constexpr (SUM2) {   // (ahead of `out`: a late publication below may carry this sum as well)
+                if (out2 != nullptr) {
+                    const unsigned long long lo = __ldcg(&ws->fx2_lo);
+                    const long long hi = __ldcg(&ws->fx2_hi);
+                    const double total = ((double)hi * 4294967296.0 + (double)lo) * (1.0 / 1099511627776.0);
+                    *out2 = __ldcg(&ws->nonfinite2) ? __longlong_as_double(0x7ff8000000000000ll) : total;
+                    ws->fx2_lo = 0ull;
+                    ws->fx2_hi = 0ll;
+                    ws->nonfinite2 = 0u;
+                }
+            }
             if (out != nullptr) {
                 const unsigned long long lo = __ldcg(&ws->fx_lo);
                 const long long hi = __ldcg(&ws->fx_hi);

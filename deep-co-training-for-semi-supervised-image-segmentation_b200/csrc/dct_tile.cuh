@@ -26,6 +26,8 @@
 //   LABELS (optional) the op itself consumes the int64 label of every pixel (supervised cross-entropy): it then
 //                    provides apply_lab<CM>(x, C, g, cls[LW], w[LW], bad) instead, with cls = label in [0,C) or -1
 //                    (ignored / out of range) and w = class weight of the label (0 when cls < 0 or ignored)
+//   SUM2 (optional)  a second per-pixel scalar with its own deterministic grid sum (TileArgs::sum2): the op then provides
+//                    apply<CM>(x, C, g, eps, bad, v2) instead, which also leaves the second value in v2
 //   CONF (optional)  the kernel also counts the confusion matrix conf[gt][argmax x] of input tensor 0 against the labels
 //                    (IoU.add / ConfusionMatrix.add, generalframework/metrics/iou.py:43-69, confusionmatrix.py:32-85):
 //                    raw arg-max with torch.max semantics, labels outside [0,C) dropped (ignore-255 included)
@@ -123,6 +125,7 @@ struct TileArgs {
     int prefetch;                  // tiles of this CTA's range whose rows are prefetched into L2 before the dependency wait
     int force_static;              // developer switch (tools/kbench_tile.cu): 1 = no tail pool (purely static contiguous ranges) even with a workspace
     unsigned long long* trace;     // developer tracing: kTraceSlots words per CTA (start, first tile landed, -, end) in ns; null in the product
+    double* sum2;                  // SUM2 ops: grid sum of the second per-pixel value (nullable)
 };
 
 // Tensor maps of a launch whose stages are filled / drained by tensor-map TMA (dct_tmap.cuh): second kernel parameter,
@@ -146,6 +149,10 @@ template <class Op, class = void>
 struct op_conf : std::false_type {};
 template <class Op>
 struct op_conf<Op, std::enable_if_t<Op::CONF>> : std::true_type {};
+template <class Op, class = void>
+struct op_sum2 : std::false_type {};
+template <class Op>
+struct op_sum2<Op, std::enable_if_t<Op::SUM2>> : std::true_type {};
 template <class Op>
 constexpr bool op_label_row() { return Op::NDICE > 0 || op_labels<Op>::value || op_conf<Op>::value; }
 
@@ -239,6 +246,7 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
     constexpr bool LAB = op_labels<Op>::value;   // the op consumes the labels itself
     constexpr bool CONF = op_conf<Op>::value;    // confusion counts of tensor 0 vs the labels (CTA-shared histogram)
     constexpr bool LROW = DICE || LAB || CONF;   // the stage carries a label row
+    constexpr bool SUM2 = op_sum2<Op>::value;    // a second per-pixel value and grid sum
     constexpr int LW = (PPT % 2 == 0) ? 2 : 1;   // pixels per math lane group: pairs use packed FP32x2
     constexpr int NG = PPT / LW;
     using T = typename std::conditional<LW == 2, f2, float>::type;
@@ -333,6 +341,8 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
 
     long long acc_fx = 0;     // this thread's share of the map sum, 2^-40 fixed point
     bool nonfinite = false;
+    long long acc_fx2 = 0;    // SUM2: the same for the second value
+    bool nonfinite2 = false;
     bool bad = false;
 
     if (is_producer) {
@@ -588,7 +598,7 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
 #pragma unroll
                     for (int c = 0; c < C; ++c) xin[n][c] = tile_ld_row<PPT, ET>(st + Cfg::row_off(n, c), p0);
                 FVec<PPT> mapv;
-                float part = 0.0f;
+                float part = 0.0f, part2 = 0.0f;
 #pragma unroll
                 for (int gi = 0; gi < NG; ++gi) {
                     T x[NIN][C];
@@ -693,6 +703,10 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
                             cw[j] = use ? (a.class_w != nullptr ? __ldg(a.class_w + lb.x) : 1.0f) : 0.0f;
                         }
                         mv = Op::template apply_lab<C, T>(x, C, gv, cls, cw, bad);
+                    } else if constexpr (SUM2) {
+                        T mv2;
+                        mv = Op::template apply<C, T>(x, C, gv, a.eps, bad, mv2);
+                        part2 += vhsum(mv2);
                     } else {
                         mv = Op::template apply<C, T>(x, C, gv, a.eps, bad);
                     }
@@ -711,6 +725,7 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
                     acc_fx += to_fixed(part, nonfinite);
                     if (a.map != nullptr) st_stream<PPT>(a.map + (int64_t)b * HW + off + p0, mapv);
                 }
+                if constexpr (SUM2) acc_fx2 += to_fixed(part2, nonfinite2);
 #pragma unroll
                 for (int n = 0; n < NOUT; ++n)
                     if (a.out[n] != nullptr) {
@@ -769,7 +784,11 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
             if (bad) atomicAdd(&a.flags[DCT_FLAG_SIMPLEX], 1);
         }
     }
-    tile_grid_finish<PUB>(acc_fx, nonfinite, a.ws, Op::HAS_MAP ? a.sum : nullptr, gridDim.x, &a.pub, a.pub_early);
+    if constexpr (SUM2)
+        tile_grid_finish<PUB, true>(acc_fx, nonfinite, a.ws, Op::HAS_MAP ? a.sum : nullptr, gridDim.x, &a.pub, a.pub_early,
+                                    acc_fx2, nonfinite2, a.sum2);
+    else
+        tile_grid_finish<PUB>(acc_fx, nonfinite, a.ws, Op::HAS_MAP ? a.sum : nullptr, gridDim.x, &a.pub, a.pub_early);
     if (a.trace != nullptr && tid == 0) a.trace[kTraceSlots * blockIdx.x + 3] = globaltimer_ns();
 }
 

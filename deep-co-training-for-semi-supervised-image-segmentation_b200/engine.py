@@ -12,6 +12,9 @@ Where the step sits in the reference iteration (generalframework/trainer/cotrain
   AEGenerator.py:93-119 (VAT): normalise(d) -> xi*normalise(d) -> net -> kl_div_with_logit.mean().backward()
                                -> eps*normalise(d.grad) -> clamp(img + r)       [l2 x3, kl_logit]
   :391-392  KL_Divergence_2D(reduce=True)(softmax(adv_logits), real.detach())   [kl_from_logits]
+Both the JSD and kl_div_with_logit read the first view's logits (pred = views[0]).  The JSD's outputs are only consumed
+at totalLoss.backward() and by the meters, so the JSD can wait for the VAT forward yhat = net(img + xi*d): where the shape
+allows (see ConsistencyStep.fused_vat) one launch does both, and the step is l2_direction, jsd (+ VAT KL), l2_radv, kl_adv.
 The network forward/backward passes between those points stay in PyTorch/cuDNN; here their
 outputs are whatever tensors the caller binds (synthetic ones in bench.py).
 """
@@ -100,12 +103,15 @@ class ConsistencyStep:
         self.exchange_mode = exchange_mode
         self._pub_stream = None
         self._h = _lib.lib()
+        # the VAT KL rides the JSD launch (dct_jsd_vat_kl_fwdbwd_f32) where that launch's stage holds the K views and yhat in
+        # 5..16 rows of 256-pixel tensor-map tiles; other shapes (C = 19) keep the two launches
+        self.fused_vat = with_vat and K >= 2 and C <= 4 and (K + 1) * C <= 16 and self.HW % 4 == 0
         # kernels launched per run(): the JSD kernel (Dice fused for C <= 4, else K counting launches), the two KL kernels,
         # the two normalisations (one launch each up to 16 x 256 x 64 floats per sample, else a sum-of-squares launch + a
         # scale launch each), the publication kernel of a chained / deferred exchange
         big = (self.M > 16 * 256 * 64) or (self.M % 4 != 0)   # (a cluster of 16 CTAs serves samples up to 1 MB)
         self.launches_per_step = 1 + (0 if (not with_dice or (C <= 4 and K * C <= 16)) else K) + \
-            ((2 + (2 + 2 if big else 2)) if with_vat else 0) + \
+            ((2 + (2 + 2 if big else 2) - (1 if self.fused_vat else 0)) if with_vat else 0) + \
             (1 if (exchange is not None and exchange_mode != "early" and (not with_vat or exchange_mode != "fused")) else 0)
 
     # bytes that MUST move per step (algorithmic, fp32): see DESIGN.md "Algorithmic bytes"
@@ -141,22 +147,28 @@ class ConsistencyStep:
 
     # the step's launches by name, in stream order (bench.py times each one on its own as well)
     PARTS = ("jsd", "l2_direction", "kl_logit", "l2_radv", "kl_adv")
+    FUSED_VAT_PARTS = ("l2_direction", "jsd", "l2_radv", "kl_adv")   # "jsd" also runs the VAT KL (fused_vat)
 
     def parts(self):
-        return self.PARTS if self.with_vat else self.PARTS[:1]
+        if not self.with_vat:
+            return self.PARTS[:1]
+        return self.FUSED_VAT_PARTS if self.fused_vat else self.PARTS
 
     def part_bytes(self):
         """Algorithmic bytes of every launch of :meth:`parts` (what MUST cross HBM; DESIGN.md 3)."""
         K, C, n = self.K, self.C, self.B * self.HW
         cin = self.M // self.HW
         fused = self.with_dice and C <= 4 and K * C <= 16   # Dice counted inside the JSD kernel: + labels only
-        b = {"jsd": n * (2 * K * C * 4) + (n * 8 if fused else 0) +
+        kv = K + 1 if self.fused_vat else K                 # fused VAT KL: yhat read, grad_yhat written as well
+        b = {"jsd": n * (2 * kv * C * 4) + (n * 8 if fused else 0) +
                     ((n * K * (C * 4 + 8)) if (self.with_dice and not fused) else 0)}
         if self.with_vat:
             b.update({"l2_direction": n * cin * 4 * 2,      # d read, xi * normalise(normalise(d)) written (one launch)
                       "kl_logit": n * 3 * C * 4,            # two logits tensors read, one gradient written
                       "l2_radv": n * cin * 4 * 4,           # d.grad + img read, r_adv + img_adv written
                       "kl_adv": n * 3 * C * 4})
+            if self.fused_vat:
+                del b["kl_logit"]
         return b
 
     def run_part(self, bufs: StepBuffers, part: str, zero_counts: bool = True, publish_prev: Optional[StepBuffers] = None) -> None:
@@ -166,7 +178,21 @@ class ConsistencyStep:
         ws, s = st.workspace.data_ptr(), _runtime.stream_ptr(dev)
         fl = _runtime.flags_ptr(st)
         sums = bufs.sums.data_ptr()
-        if part == "jsd" and self.exchange is not None and publish_prev is not None:
+        if part == "jsd" and self.fused_vat:
+            # JSD fwd+bwd + Dice and kl_div_with_logit(pred.detach(), y_hat) + backward to y_hat in one launch; it also
+            # publishes the previous step's sums when asked (as dct_jsd_fwdbwd_pub_f32 below)
+            pub = None
+            if self.exchange is not None and publish_prev is not None:
+                pub = ctypes.byref(self.exchange.descriptor(publish_prev.sums))
+            _lib.check(h.dct_jsd_vat_kl_fwdbwd_f32(_lib.ptr_array(bufs.logits), K, C, B, HW, self.jsd_weight / self.n, sums,
+                                                   _lib.ptr_array(bufs.grad_logits),
+                                                   bufs.labels.data_ptr() if self.with_dice else None,
+                                                   bufs.dice_counts.data_ptr() if self.with_dice else None,
+                                                   _lib.COUNTS_OVERWRITE if zero_counts else _lib.COUNTS_ACCUMULATE,
+                                                   bufs.yhat_logits.data_ptr(), 1.0 / self.n, sums + 8,
+                                                   bufs.grad_yhat.data_ptr(), fl, ws, pub, s),
+                       "dct_jsd_vat_kl_fwdbwd_f32")
+        elif part == "jsd" and self.exchange is not None and publish_prev is not None:
             # the step's first kernel also publishes the PREVIOUS step's sums (final since that step's last kernel completed)
             _lib.check(h.dct_jsd_fwdbwd_pub_f32(_lib.ptr_array(bufs.logits), K, C, B, HW, _lib.IN_LOGITS,
                                                 self.jsd_weight / self.n, None, sums, _lib.ptr_array(bufs.grad_logits),

@@ -172,6 +172,20 @@ DCT_API int dct_jsd_fwdbwd_f32(const float* const* views, int K, int C, int64_t 
                        const int64_t* labels, int64_t* counts, int counts_mode,
                        int32_t* flags, void* workspace, void* stream);
 
+/* The consistency step's JSD launch with the VAT KL folded in.  In the trainer the JSD of the K views
+ * (cotraining_totalloss.py:223-226) and VATGenerator's kl_div_with_logit(pred.detach(), yhat) (AEGenerator.py:93-119,
+ * pred = views[0]) both read the first view's logits, and nothing between the two points reads what the JSD writes, so
+ * a trainer can call this once the VAT forward yhat = net(img + xi*d) exists.  Defined as
+ *   dct_jsd_fwdbwd_f32(views, K, C, B, HW, DCT_IN_LOGITS, jsd_gconst, NULL, jsd_sum, grad_views, labels, counts,
+ *                      counts_mode, flags, workspace)   [dct_jsd_fwdbwd_pub_f32 with pub_desc when pub_desc != NULL]
+ *   dct_kl_logit_f32(views[0], yhat, C, B, HW, NULL, kl_sum, 1, NULL, NULL, kl_gconst, grad_yhat, NULL, workspace)
+ * and returns the same results.  Shapes with (K + 1) * C <= 16 and C <= 4, 16-byte aligned rows and HW % 4 == 0 run as ONE
+ * launch that reads views[0] once; every other shape runs the two calls above. */
+DCT_API int dct_jsd_vat_kl_fwdbwd_f32(const float* const* views, int K, int C, int64_t B, int64_t HW, float jsd_gconst,
+                                      double* jsd_sum, float* const* grad_views, const int64_t* labels, int64_t* counts,
+                                      int counts_mode, const float* yhat, float kl_gconst, double* kl_sum, float* grad_yhat,
+                                      int32_t* flags, void* workspace, const dct_peer_pub* pub_desc, void* stream);
+
 /* grad[i] *= *gscalar for i < n, skipped entirely (no memory traffic) when *gscalar == 1.0f.
  * Used by the fused loss' backward: the upstream of `total = sup + fused_loss` is exactly 1. */
 DCT_API int dct_scale_if_not_one_f32(float* grad, int64_t n, const float* gscalar, void* stream);
