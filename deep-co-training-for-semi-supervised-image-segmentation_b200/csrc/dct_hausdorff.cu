@@ -29,6 +29,11 @@
 //   sd_pick_kernel<P>    narrows prefix and rank from the histogram of pass P.
 //   sd_finish_kernel     hd, hd95, asd, assd.
 // Launches: 14 for '2d', 15 for a volume.
+//
+// dct_surface_dice_i64 (normalized surface Dice at tolerance tol[c]) runs the same passes with the last one in its TOL
+// mode, which only counts per line the queries and the queries with sqrt((double)d^2) <= tol[c], then:
+//   nsd_finish_kernel    per (row, class): 64-bit sums of both sides' line counts; nsd, overlap_pg, overlap_gp, counts.
+// Launches: 4 for '2d', 5 for a volume.
 #include <math_constants.h>
 
 #include <algorithm>
@@ -62,6 +67,7 @@ inline size_t hd_align256(size_t v) { return (v + 255) & ~(size_t)255; }
 struct HdLayout {
     size_t hdr, rec, g, f, total;              // dct_hausdorff_i64
     size_t qd, lsum, lcnt, hist, st, surf_total;   // dct_surface_distances_i64: the same, then these
+    size_t tq, tw, dice_total;                 // dct_surface_dice_i64: the Hausdorff scratch, then these
 };
 constexpr size_t kSdStateBytes = 64;   // sizeof(SdState)
 inline HdLayout hd_layout(int C, int64_t B, int64_t H, int64_t W, int volume) {
@@ -79,6 +85,9 @@ inline HdLayout hd_layout(int C, int64_t B, int64_t H, int64_t W, int volume) {
     L.hist = hd_align256(L.lcnt + fold_lines * 4);         // uint64 [rows][C][256]
     L.st = hd_align256(L.hist + rows * C * 256 * 8);       // SdState [rows][C]
     L.surf_total = hd_align256(L.st + rows * C * kSdStateBytes);
+    L.tq = L.total;                                        // uint32 [fold_lines] queries
+    L.tw = hd_align256(L.tq + fold_lines * 4);             // uint32 [fold_lines] queries within the tolerance
+    L.dice_total = hd_align256(L.tw + fold_lines * 4);
     return L;
 }
 
@@ -163,8 +172,17 @@ struct EnvArgs {
     double w_in, w;          // squared spacing of the previous axis (FROM_G) and of this one
     float* qd;               // SURF: [2][N] squared distance of each query pixel to the border set of that side
     double* lsum;            // SURF: per line of the last pass, sum of sqrt(d^2) over its queries
-    unsigned* lcnt;          // SURF: per line of the last pass, number of its queries
+    unsigned* lcnt;          // SURF, TOL: per line of the last pass, number of its queries
 };
+
+// TOL (last pass of dct_surface_dice_i64): the tolerances travel by value in the kernel arguments (no copy, graph-safe);
+// only this mode's instantiations take the larger argument block
+struct EnvTolArgs : EnvArgs {
+    unsigned* lwin;                  // per line of the last pass, number of its queries within tol[c]
+    double tol[DCT_MAX_CLASSES];     // per class, in spacing units
+};
+template <bool TOL>
+using EnvParams = std::conditional_t<TOL, EnvTolArgs, EnvArgs>;
 
 template <bool FROM_G>
 __device__ __forceinline__ double env_load(const EnvArgs& a, int64_t plane, int64_t off) {
@@ -180,10 +198,12 @@ __device__ __forceinline__ double env_load(const EnvArgs& a, int64_t plane, int6
 // line.  Stack entry k = (position v_k, first integer position z_k at which parabola v_k is the lowest); a new parabola q
 // (to the right of every stacked one) is at or below v_k from ceil(sep) on, so v_k is popped when ceil(sep) <= z_k and q is
 // only pushed when ceil(sep) < n.  SURF (last pass of dct_surface_distances_i64): also keep every query's d^2 and the
-// line's sum of distances and query count.
-template <bool FROM_G, bool FOLD, bool SURF = false>
-__global__ void __launch_bounds__(64) hd_envelope_kernel(const EnvArgs a) {
-    static_assert(FOLD || !SURF, "only the last pass has queries");
+// line's sum of distances and query count.  TOL (last pass of dct_surface_dice_i64): instead of the maximum, only the
+// line's query count and the number of its queries with sqrt((double)d^2) <= tol[c].
+template <bool FROM_G, bool FOLD, bool SURF = false, bool TOL = false>
+__global__ void __launch_bounds__(64) hd_envelope_kernel(const EnvParams<TOL> a) {
+    static_assert(FOLD || !(SURF || TOL), "only the last pass has queries");
+    static_assert(!(SURF && TOL), "one query mode per pass");
     extern __shared__ unsigned stk_all[];
     const int64_t line = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (line >= 2 * a.g.C * a.lines_per_plane) return;
@@ -216,7 +236,9 @@ __global__ void __launch_bounds__(64) hd_envelope_kernel(const EnvArgs a) {
     float m = 0.0f;
     bool any = false;
     double dsum = 0.0;
-    unsigned cnt = 0;
+    unsigned cnt = 0, win = 0;
+    double tol = 0.0;
+    if constexpr (TOL) tol = a.tol[c];
     int k = 0;
     for (int x = 0; x < n; ++x) {
         const int64_t off = base + x * stride;
@@ -236,14 +258,19 @@ __global__ void __launch_bounds__(64) hd_envelope_kernel(const EnvArgs a) {
             dsum += sqrt((double)d);
             ++cnt;
         }
+        if constexpr (TOL) {
+            ++cnt;
+            if (sqrt((double)d) <= tol) ++win;   // d = +inf (no border on this side) is never within
+        }
     }
-    if constexpr (FOLD) {
+    if constexpr (FOLD && !TOL) {
         if (any) {
             const int64_t row = l / a.lines_per_row;
             atomicMax(&a.rowmax[(row * a.g.C + c) * 2 + side], __float_as_uint(m));
         }
     }
     if constexpr (SURF) { a.lsum[line] = dsum; a.lcnt[line] = cnt; }
+    if constexpr (TOL) { a.lcnt[line] = cnt; a.lwin[line] = win; }
 }
 
 __device__ __forceinline__ float hd_value(const unsigned* __restrict__ rowmax, const unsigned* __restrict__ present,
@@ -460,19 +487,82 @@ __global__ void sd_finish_kernel(const unsigned* __restrict__ rowmax, const unsi
     }
 }
 
-template <bool FROM_G, bool FOLD, bool SURF = false>
-cudaError_t launch_envelope(const EnvArgs& a, cudaStream_t s) {
+// ---- normalized surface Dice (dct_surface_dice_i64): counts of the TOL last pass -------------------------------------
+
+// one CTA per (row, class): 64-bit sums of both sides' per-line query and within-tolerance counts (integers: the order
+// does not matter), then nsd = (W_pg + W_gp) / (|S_pg| + |S_gp|), overlap_pg = W_pg / |S_pg|, overlap_gp = W_gp / |S_gp|
+// as double ratios rounded once to float (NaN for a zero denominator).  Side 1's queries are the prediction's border
+// pixels (S_pg), side 0's the label's (S_gp).  out [3][nrc]; counts (nullable) [nrc][4] = W_pg, |S_pg|, W_gp, |S_gp|.
+constexpr int kNsdThreads = 256;
+__global__ void __launch_bounds__(kNsdThreads) nsd_finish_kernel(const unsigned* __restrict__ lq,
+                                                                 const unsigned* __restrict__ lw, int C,
+                                                                 int64_t lines_per_plane, int64_t lines_per_row,
+                                                                 int64_t nrc, float* __restrict__ out,
+                                                                 long long* __restrict__ counts) {
+    __shared__ unsigned long long part[kNsdThreads / 32][4];
+    const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    for (int64_t rc = blockIdx.x; rc < nrc; rc += gridDim.x) {
+        const int64_t row = rc / C;
+        const int c = (int)(rc - row * C);
+        unsigned long long v[4] = {0ull, 0ull, 0ull, 0ull};   // W_pg, |S_pg|, W_gp, |S_gp|
+#pragma unroll
+        for (int side = 0; side < 2; ++side) {
+            const int64_t base = (int64_t)(side * C + c) * lines_per_plane + row * lines_per_row;
+            const int slot = side ? 0 : 2;
+            for (int64_t j = t; j < lines_per_row; j += kNsdThreads) {
+                v[slot] += lw[base + j];
+                v[slot + 1] += lq[base + j];
+            }
+        }
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+            for (int o = 16; o > 0; o >>= 1) v[i] += __shfl_xor_sync(0xffffffffu, v[i], o);
+            if (lane == 0) part[warp][i] = v[i];
+        }
+        __syncthreads();
+        if (t == 0) {
+            unsigned long long s[4] = {0ull, 0ull, 0ull, 0ull};
+            for (int w = 0; w < kNsdThreads / 32; ++w)
+                for (int i = 0; i < 4; ++i) s[i] += part[w][i];
+            const unsigned long long n = s[1] + s[3];
+            out[rc] = n ? (float)((double)(s[0] + s[2]) / (double)n) : CUDART_NAN_F;
+            out[nrc + rc] = s[1] ? (float)((double)s[0] / (double)s[1]) : CUDART_NAN_F;
+            out[2 * nrc + rc] = s[3] ? (float)((double)s[2] / (double)s[3]) : CUDART_NAN_F;
+            if (counts != nullptr)
+                for (int i = 0; i < 4; ++i) counts[rc * 4 + i] = (long long)s[i];
+        }
+        __syncthreads();   // part[] is reused by the next (row, class)
+    }
+}
+
+template <bool FROM_G, bool FOLD, bool SURF = false, bool TOL = false>
+cudaError_t launch_envelope(const EnvParams<TOL>& a, cudaStream_t s) {
     const int64_t lines = 2 * a.g.C * a.lines_per_plane;
     int R = kEnvSmemBudget / (4 * a.n);
     R = R > 64 ? 64 : (R < 1 ? 1 : R);
     const size_t smem = (size_t)R * a.n * 4;
     if (smem > (size_t)kEnvSmemBudget) {
-        cudaError_t e = cudaFuncSetAttribute(hd_envelope_kernel<FROM_G, FOLD, SURF>,
+        cudaError_t e = cudaFuncSetAttribute(hd_envelope_kernel<FROM_G, FOLD, SURF, TOL>,
                                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
     }
-    hd_envelope_kernel<FROM_G, FOLD, SURF><<<(unsigned)((lines + R - 1) / R), R, smem, s>>>(a);
+    hd_envelope_kernel<FROM_G, FOLD, SURF, TOL><<<(unsigned)((lines + R - 1) / R), R, smem, s>>>(a);
     return cudaGetLastError();
+}
+
+// the last envelope pass of one entry point: plain (Hausdorff), SURF, or TOL with the per-class tolerances
+template <bool FROM_G, bool SURF, bool TOL>
+cudaError_t launch_last_pass(const EnvArgs& a, const double* tol, const HdLayout& L, char* base, cudaStream_t s) {
+    if constexpr (TOL) {
+        EnvTolArgs t{};
+        static_cast<EnvArgs&>(t) = a;
+        t.lcnt = reinterpret_cast<unsigned*>(base + L.tq);
+        t.lwin = reinterpret_cast<unsigned*>(base + L.tw);
+        for (int c = 0; c < a.g.C; ++c) t.tol[c] = tol[c];
+        return launch_envelope<FROM_G, true, false, true>(t, s);
+    } else {
+        return launch_envelope<FROM_G, true, SURF>(a, s);
+    }
 }
 
 // argument checks of both entry points; fills the spacing (sz, sy, sx)
@@ -495,10 +585,12 @@ inline int hd_check_args(const int64_t* pred, const int64_t* labels, int C, int6
 }
 
 // classify, column and envelope passes (3 launches for '2d', 4 for a volume): leave the per-(row, class, side) maxima
-// and presence words in the scratch header and, with SURF, every query's d^2 and the last pass's per-line slots
-template <bool SURF>
+// and presence words in the scratch header and, with SURF, every query's d^2 and the last pass's per-line slots; with
+// TOL (tolerances `tol`, C host values) only the last pass's per-line query and within-tolerance counts
+template <bool SURF, bool TOL = false>
 cudaError_t hd_distance_passes(const int64_t* pred, const int64_t* labels, const HdGeom& g, const double sp[3],
-                               const HdLayout& L, char* base, int32_t* flags, cudaStream_t s) {
+                               const HdLayout& L, char* base, int32_t* flags, cudaStream_t s,
+                               const double* tol = nullptr) {
     const int64_t B = g.B, H = g.H, W = g.W, nrc = (g.volume ? 1 : B) * g.C;
     unsigned* rowmax = reinterpret_cast<unsigned*>(base + L.hdr);
     unsigned* present = rowmax + 2 * nrc;
@@ -524,7 +616,7 @@ cudaError_t hd_distance_passes(const int64_t* pred, const int64_t* labels, const
     }
     if (!g.volume) {
         a.lines_per_row = H;   // line l = b * H + y lies in image b
-        return launch_envelope<true, true, SURF>(a, s);
+        return launch_last_pass<true, SURF, TOL>(a, tol, L, base, s);
     }
     a.fout = f;
     e = launch_envelope<true, false>(a, s);
@@ -533,7 +625,7 @@ cudaError_t hd_distance_passes(const int64_t* pred, const int64_t* labels, const
     z.lines_per_plane = H * W; z.line_step = 1; z.stride = H * W; z.n = (int)B;
     z.lines_per_row = H * W;   // one row: the volume
     z.w_in = 0.0; z.w = sp[0] * sp[0];
-    if (e == cudaSuccess) e = launch_envelope<false, true, SURF>(z, s);
+    if (e == cudaSuccess) e = launch_last_pass<false, SURF, TOL>(z, tol, L, base, s);
     return e;
 }
 
@@ -643,6 +735,38 @@ extern "C" int dct_surface_distances_i64(const int64_t* pred, const int64_t* lab
     if (e == cudaSuccess) {
         sd_finish_kernel<<<(unsigned)std::min<int64_t>((nrc + 127) / 128, 1024), 128, 0, s>>>(rowmax, rowmax + 2 * nrc,
                                                                                               st, nrc, out);
+        e = cudaGetLastError();
+    }
+    if (e != cudaSuccess) { g_last_cuda_error = e; return DCT_ERR_CUDA; }
+    return DCT_OK;
+}
+
+extern "C" size_t dct_surface_dice_scratch_bytes(int C, int64_t B, int64_t H, int64_t W, int volume) {
+    if (C < 1 || B < 1 || H < 1 || W < 1 || !hd_supported(C, B, H, W, volume)) return 0;
+    return hd_layout(C, B, H, W, volume).dice_total;
+}
+
+extern "C" int dct_surface_dice_i64(const int64_t* pred, const int64_t* labels, int C, int64_t B, int64_t H, int64_t W,
+                                    int volume, const double* spacing, const double* tolerance, float* out,
+                                    int64_t* counts, int32_t* flags, void* scratch, void* stream) {
+    double sp[3];
+    const int rc = hd_check_args(pred, labels, C, B, H, W, volume, spacing, out, flags, scratch, sp);
+    if (rc != DCT_OK) return rc;
+    if (tolerance == nullptr) return DCT_ERR_BAD_ARG;
+    for (int c = 0; c < C; ++c)
+        if (!(tolerance[c] >= 0.0) || !std::isfinite(tolerance[c])) return DCT_ERR_BAD_ARG;   // also rejects NaN
+    if (!aligned(counts, 8)) return DCT_ERR_MISALIGNED;
+    const HdGeom g{C, B, H, W, B * H * W, volume ? 1 : 0};
+    const HdLayout L = hd_layout(C, B, H, W, volume);
+    char* base = static_cast<char*>(scratch);
+    const int64_t nrc = (volume ? 1 : B) * C;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    cudaError_t e = hd_distance_passes<false, true>(pred, labels, g, sp, L, base, flags, s, tolerance);
+    if (e == cudaSuccess) {
+        const int64_t lines_per_plane = volume ? H * W : B * H, lines_per_row = volume ? H * W : H;
+        nsd_finish_kernel<<<(unsigned)std::min<int64_t>(nrc, (int64_t)kSMs * 8), kNsdThreads, 0, s>>>(
+            reinterpret_cast<const unsigned*>(base + L.tq), reinterpret_cast<const unsigned*>(base + L.tw), C,
+            lines_per_plane, lines_per_row, nrc, out, reinterpret_cast<long long*>(counts));
         e = cudaGetLastError();
     }
     if (e != cudaSuccess) { g_last_cuda_error = e; return DCT_ERR_CUDA; }

@@ -9,7 +9,7 @@ Mirrors ``generalframework/metrics`` of the reference:
 plus ``hausdorff`` / ``HausdorffMeter``: the Hausdorff distance Summary.py:25 takes from the external ``deepclustering``
 package, with the definition of ``medpy.metric.binary.hd`` (exact distance transforms on the device), and
 ``surface_distances`` / ``SurfaceDistanceMeter``: HD95, ASD and ASSD (``medpy.metric.binary`` hd95 / asd / assd) from the
-same distance transforms.
+same distance transforms, and ``surface_dice`` / ``SurfaceDiceMeter``: the normalized surface Dice at a tolerance.
 
 ``add`` never leaves the device (no one-hot tensors, no ``torch.unique(a.cpu())``, no numpy
 ``bincount``); ``value()`` / ``summary()`` keep the reference's return structures.  Counts are exact
@@ -284,6 +284,65 @@ def surface_distances(pred, gt, C=None, method='2d', voxelspacing=None) -> dict:
     return dict(zip(_SURFACE_KEYS, out.unbind(0)))
 
 
+_DICE_KEYS = ('nsd', 'overlap_pg', 'overlap_gp')
+
+
+def _tolerances(tolerance, C):
+    """``C`` host doubles from a scalar (every class) or a sequence / array / tensor of ``C`` values, each finite and >= 0."""
+    if torch.is_tensor(tolerance):
+        tolerance = tolerance.tolist()
+    t = np.asarray(tolerance, dtype=np.float64)
+    t = np.full(C, float(t)) if t.ndim == 0 else t.ravel()
+    assert t.size == C, f"surface_dice: {t.size} tolerances for C={C} classes"
+    if not (np.all(np.isfinite(t)) and np.all(t >= 0)):
+        raise ValueError(f"surface_dice: tolerances must be finite and >= 0, got {t.tolist()}")
+    return (ctypes.c_double * C)(*t.tolist())
+
+
+def surface_dice(pred, gt, tolerance, C=None, method='2d', voxelspacing=None) -> dict:
+    """Normalized surface Dice (surface Dice at a tolerance) per class from one device call: ``{'nsd', 'overlap_pg',
+    'overlap_gp'}``, each float32 ``[rows, C]``, and ``'counts'``, int64 ``[rows, C, 4]``, on the input's device.
+    Arguments, borders, grids and spacing are those of ``hausdorff``.
+
+    With ``S_pg`` the distances from each border pixel of ``{pred == c}`` to the border of ``{gt == c}``, ``S_gp`` the other
+    direction, and a distance to an empty border counted as +inf: ``W_pg`` = the number of ``S_pg`` within
+    ``tolerance[c]`` (``<=``), ``W_gp`` likewise; ``nsd`` = ``(W_pg + W_gp) / (|S_pg| + |S_gp|)``; ``overlap_pg`` =
+    ``W_pg / |S_pg|`` and ``overlap_gp`` = ``W_gp / |S_gp|``, the two directional surface overlaps.  ``counts[..., :]`` =
+    ``(W_pg, |S_pg|, W_gp, |S_gp|)``: sum them over a dataset to pool the NSD exactly.  This is the border-pixel form:
+    every border pixel counts once, as MONAI's ``compute_surface_dice`` with ``use_subvoxels=False`` is described (not
+    checked against MONAI); the surfel-area form of DeepMind's ``surface-distance`` package is not computed.
+
+    ``nsd`` is NaN only when both borders are empty, and 0 when exactly one is: a missed or hallucinated structure scores
+    0.  This differs on purpose from ``hausdorff`` / ``surface_distances``, which are NaN when either side is empty.  Each
+    overlap is NaN when its own border is empty.
+
+    ``tolerance``: one finite value >= 0 per class, in the units of ``voxelspacing``, or a scalar for every class.  A
+    distance is compared as ``sqrt(d2) <= tolerance[c]`` in double on the float squared distance of the distance passes:
+    at unit spacing the counts are exactly those of scipy's EDT, tolerances equal to attained distances (1, sqrt(2), 2, ...)
+    included; at anisotropic spacing only distances within about 1e-7 relative of a tolerance can count differently.
+    """
+    p, g, C, volume, sp = _distance_args(pred, gt, C, method, voxelspacing, "surface_dice")
+    tols = _tolerances(tolerance, C)
+    B, H, W = p.shape
+    h = _lib.lib()
+    nbytes = h.dct_surface_dice_scratch_bytes(C, B, H, W, int(volume))
+    if nbytes == 0:
+        _lib.check(_lib.ERR_UNSUPPORTED, f"dct_surface_dice_scratch_bytes (C={C}, shape {(B, H, W)})")
+    scratch = torch.empty(nbytes, dtype=torch.uint8, device=p.device)
+    rows = 1 if volume else B
+    out = torch.empty((3, rows, C), dtype=torch.float32, device=p.device)
+    counts = torch.empty((rows, C, 4), dtype=torch.int64, device=p.device)
+    st = _runtime.state(p.device)
+    _lib.check(h.dct_surface_dice_i64(p.data_ptr(), g.data_ptr(), C, B, H, W, int(volume), sp,
+                                      tols, out.data_ptr(), counts.data_ptr(),
+                                      _runtime.flags_ptr(st), scratch.data_ptr(), _runtime.stream_ptr(p.device)),
+               "dct_surface_dice_i64")
+    _runtime.after_call(st)
+    r = dict(zip(_DICE_KEYS, out.unbind(0)))
+    r['counts'] = counts
+    return r
+
+
 def _nan_mean_std(x: torch.Tensor, dim: int):
     """Mean and unbiased standard deviation along ``dim`` over the non-NaN entries (NaN where fewer than 1 / 2 remain)."""
     valid = ~torch.isnan(x)
@@ -389,6 +448,48 @@ class SurfaceDistanceMeter(Metric):
             (mean, var), _ = self.value(k)
             out.update({f'm{name}': mean.item(), f'm{name}Vars': var.item()})
         return out
+
+
+class SurfaceDiceMeter(Metric):
+    """Normalized surface Dice per class next to ``DiceMeter`` (same ``method`` / ``report_axises`` / ``C``; definition of
+    ``surface_dice`` at ``tolerance``, a scalar or one value per class).  ``add`` makes one device call and appends one
+    row per image (``'2d'``) or per batch (``'3d'``); the statistics are ``HausdorffMeter``'s and skip the NaN of classes
+    absent from both the prediction and the label."""
+
+    def __init__(self, tolerance, method='2d', report_axises='all', C=4) -> None:
+        super().__init__()
+        assert method in ('2d', '3d')
+        assert report_axises == 'all' or isinstance(report_axises, list)
+        self.tolerance = tolerance
+        self.method = method
+        self.report_axis = report_axises
+        self.C = C
+        self.nsdLog = []
+
+    def reset(self):
+        self.nsdLog = []
+
+    def add(self, pred, gt, voxelspacing=None):
+        r = surface_dice(pred, gt, self.tolerance, C=self.C, method=self.method, voxelspacing=voxelspacing)
+        self.nsdLog.append(r['nsd'])
+
+    @property
+    def log(self):
+        if len(self.nsdLog) == 0:
+            return torch.full((1, self.C), float('nan'))
+        return torch.cat(self.nsdLog)
+
+    def value(self, **kwargs):
+        """``((mean, std), (means[C], stds[C]))`` of the NSD log, as ``HausdorffMeter.value``."""
+        return _nan_statistics(self.log, self.report_axis)
+
+    def detailed_summary(self) -> dict:
+        _, (means, _) = self.value()
+        return {f'NSD{i}': means[i].item() for i in range(len(means))}
+
+    def summary(self) -> dict:
+        (mean, var), _ = self.value()
+        return {'mNSD': mean.item(), 'mNSDVars': var.item()}
 
 
 class ConfusionMatrix(Metric):

@@ -419,6 +419,32 @@ DCT_API int dct_surface_distances_i64(const int64_t* pred, const int64_t* labels
                                       int volume, const double* spacing, float* out, int32_t* flags, void* scratch,
                                       void* stream);
 
+/* Normalized surface Dice (surface Dice at tolerance tol[c]) of the same borders, grids and spacing, border-pixel form:
+ * every border pixel counts once.  Per (row, class c), with S_pg and S_gp as for dct_surface_distances_i64 and a distance
+ * to an empty border set being +inf (never within the tolerance):
+ *   W_pg = #{s in S_pg : s <= tol[c]}, W_gp likewise, each s compared as sqrt((double)d^2) <= tol[c] on the float d^2 the
+ *          distance passes produce (at unit spacing d^2 is exact, so the counts are those of scipy's EDT);
+ *   nsd        = (W_pg + W_gp) / (|S_pg| + |S_gp|): NaN only when both borders are empty, 0 when exactly one is (a missed or
+ *                hallucinated structure scores 0; unlike hd, which is NaN when either is empty);
+ *   overlap_pg = W_pg / |S_pg|, overlap_gp = W_gp / |S_gp|: each NaN when its denominator is 0;
+ * each a double ratio of the 64-bit counts, rounded once to float.  Same limits, flags, argument checks and error codes
+ * as dct_hausdorff_i64.  The last distance pass only counts, per line, its queries and those within the tolerance; one
+ * more launch sums them per (row, class).  4 launches for a slice batch, 5 for a volume; no host synchronisation, no
+ * allocation, no copies (the tolerances travel in the kernel arguments). */
+
+/* bytes of `scratch` dct_surface_dice_i64 needs: dct_hausdorff_scratch_bytes() + 8 per line of the last pass (2*C*B*H
+ * lines for a slice batch, 2*C*H*W for a volume), each region rounded up to 256 bytes; 0 for a shape it rejects.  Host
+ * only. */
+DCT_API size_t dct_surface_dice_scratch_bytes(int C, int64_t B, int64_t H, int64_t W, int volume);
+/* pred, labels, spacing, flags, scratch as for dct_hausdorff_i64 (scratch >= dct_surface_dice_scratch_bytes());
+ * tolerance: HOST array of C finite values >= 0 in the units of spacing (NULL, negative, NaN or infinite: DCT_ERR_BAD_ARG,
+ * nothing launched); out float32 [3][volume ? 1 : B][C] = nsd, overlap_pg, overlap_gp, overwritten; counts (nullable,
+ * 8-byte aligned) int64 [volume ? 1 : B][C][4] = W_pg, |S_pg|, W_gp, |S_gp|, overwritten -- sum them over a dataset to
+ * pool the NSD exactly. */
+DCT_API int dct_surface_dice_i64(const int64_t* pred, const int64_t* labels, int C, int64_t B, int64_t H, int64_t W,
+                                 int volume, const double* spacing, const double* tolerance, float* out, int64_t* counts,
+                                 int32_t* flags, void* scratch, void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * Connected components of a class map (evaluation path: the post-processing in front of the Dice and surface distances;
  * getLargestCC of the UA-MT / DTC / MC-Net test scripts, nnU-Net's "remove all but the largest component").
