@@ -14,13 +14,15 @@
 //                        nearest feature of the column (uint16, 0xFFFF = none); coalesced across columns.
 //   hd_envelope_kernel   exact squared EDT along one more axis: lower envelope of the parabolas f(q) + w (x - q)^2
 //                        (Felzenszwalb-Huttenlocher) restricted to integer positions, one thread per line with its stack in
-//                        shared memory.  Along W it either writes the float map (volume) or is the last pass; along B
+//                        shared memory.  Along W it either writes the d^2 map (volume) or is the last pass; along B
 //                        (volume) it is the last pass.  The last pass folds max over the other side's border pixels of d^2
-//                        into the (row, class, side) maximum with an integer atomicMax on the float bits (non-negative
-//                        floats order like their bit patterns): order-independent, so bit-reproducible.
-//   hd_finish_kernel     HD = __fsqrt_rn(max of the two sides), NaN where a side's set is empty.
-// Launches: 4 for '2d', 5 for a volume.  Envelope arithmetic is double; at unit spacing every d^2 is an integer, exact in
-// the float maxima up to 2^24, so the result is the correctly rounded square root of the exact squared distance.
+//                        into the (row, class, side) maximum with an integer atomicMax on the d^2 key (d2_key):
+//                        order-independent, so bit-reproducible.
+//   hd_finish_kernel     HD = square root of the max of the two sides, NaN where a side's set is empty.
+// Launches: 4 for '2d', 5 for a volume.  Envelope arithmetic is double.  Every d^2 that leaves a pass is a 32-bit key that
+// orders like the value: at unit spacing the exact integer (3 * 32767^2 < 2^32), otherwise the bits of the float d^2.  So
+// at unit spacing the result is the correctly rounded square root of the exact squared distance for every accepted shape
+// (a float d^2 would be rounded from 4096 pixels of distance on).
 //
 // dct_surface_distances_i64 (HD95, ASD, ASSD; medpy.metric.binary hd95 / asd / assd) runs the same passes with the last
 // one in its SURF mode, which also keeps every query's d^2 and per-line sums, then:
@@ -48,16 +50,31 @@ constexpr int kHdMaxAxis = 32768;                 // stack entries hold (positio
 constexpr uint16_t kNone = 0xFFFF;                // hd_column_kernel: no feature in the column
 constexpr unsigned char kOutOfRange = 0x7F;       // record byte of a value outside [0,C): matches no (class | 0x80)
 constexpr int kEnvSmemBudget = 48 * 1024;         // per CTA; a line of n positions takes 4n bytes of stack
+constexpr unsigned kInfKey = 0xFFFFFFFFu;         // d2_key of +inf at unit spacing
 
 struct HdGeom {
     int C;
     int64_t B, H, W, N;   // N = B*H*W
     int volume;
+    int exact;            // unit spacing: d^2 keys are the exact integers
 };
 
-// shapes the kernels take: axes within the 16-bit stack entries, every grid within 2^31 - 1 threads
+// d^2 as a 32-bit key that orders like the value (maxima by integer atomicMax, percentiles by a radix select on the key):
+// at unit spacing (exact) the integer d^2 itself, which fits since every axis is at most 32768 long, with kInfKey for
+// +inf; otherwise the bits of the float d^2 (non-negative floats order like their bits)
+__device__ __forceinline__ unsigned d2_key(double d2, bool exact) {
+    if (exact) return isinf(d2) ? kInfKey : (unsigned)d2;
+    return __float_as_uint((float)d2);
+}
+__device__ __forceinline__ double d2_value(unsigned key, bool exact) {
+    if (exact) return key == kInfKey ? CUDART_INF : (double)key;
+    return (double)__uint_as_float(key);
+}
+
+// shapes the kernels take: axes within the 16-bit stack entries, every grid within 2^31 - 1 threads (B is bounded
+// first so that the line count cannot overflow int64)
 inline bool hd_supported(int C, int64_t B, int64_t H, int64_t W, int volume) {
-    if (C > DCT_MAX_CLASSES || H > kHdMaxAxis || W > kHdMaxAxis || (volume && B > kHdMaxAxis)) return false;
+    if (C > DCT_MAX_CLASSES || H > kHdMaxAxis || W > kHdMaxAxis || B > (volume ? kHdMaxAxis : INT_MAX)) return false;
     const int64_t lines = 2 * (int64_t)C * B * std::max(H, W);   // column and row passes
     return lines <= INT_MAX && (!volume || 2 * (int64_t)C * H * W <= INT_MAX);
 }
@@ -77,9 +94,9 @@ inline HdLayout hd_layout(int C, int64_t B, int64_t H, int64_t W, int volume) {
     L.hdr = 0;                                          // uint32 rowmax[rows][C][2], present[rows][C][2]
     L.rec = hd_align256(L.hdr + rows * C * 2 * 2 * 4);     // uint16 [N]: pred byte | gt byte << 8
     L.g = hd_align256(L.rec + N * 2);                      // uint16 [2][C][N]
-    L.f = hd_align256(L.g + 2 * (size_t)C * N * 2);        // float  [2][C][N] (volume only)
+    L.f = hd_align256(L.g + 2 * (size_t)C * N * 2);        // uint32 [2][C][N] d^2 keys (volume only)
     L.total = volume ? hd_align256(L.f + 2 * (size_t)C * N * 4) : L.f;
-    L.qd = L.total;                                        // float  [2][N]
+    L.qd = L.total;                                        // uint32 [2][N] d^2 keys
     L.lsum = hd_align256(L.qd + 2 * N * 4);                // double [fold_lines]
     L.lcnt = hd_align256(L.lsum + fold_lines * 8);         // uint32 [fold_lines]
     L.hist = hd_align256(L.lcnt + fold_lines * 4);         // uint64 [rows][C][256]
@@ -162,15 +179,15 @@ __global__ void __launch_bounds__(128) hd_column_kernel(const uint16_t* __restri
 
 struct EnvArgs {
     const uint16_t* gdist;   // FROM_G: input distances in rows (weight w_in)
-    const float* fin;        // !FROM_G: input squared distances
-    float* fout;             // !FOLD: output squared distances
+    const unsigned* fin;     // !FROM_G: input d^2 keys
+    unsigned* fout;          // !FOLD: output d^2 keys
     const uint16_t* rec;     // FOLD: border records of the queries
-    unsigned* rowmax;        // FOLD: [rows][C][2] float bits
+    unsigned* rowmax;        // FOLD: [rows][C][2] d^2 keys
     HdGeom g;
     int64_t lines_per_plane, line_step, stride, lines_per_row;
     int n;
     double w_in, w;          // squared spacing of the previous axis (FROM_G) and of this one
-    float* qd;               // SURF: [2][N] squared distance of each query pixel to the border set of that side
+    unsigned* qd;            // SURF: [2][N] d^2 key of each query pixel to the border set of that side
     double* lsum;            // SURF: per line of the last pass, sum of sqrt(d^2) over its queries
     unsigned* lcnt;          // SURF, TOL: per line of the last pass, number of its queries
 };
@@ -190,7 +207,7 @@ __device__ __forceinline__ double env_load(const EnvArgs& a, int64_t plane, int6
         const uint16_t d = a.gdist[plane + off];
         return d == kNone ? CUDART_INF : a.w_in * (double)d * (double)d;
     } else {
-        return (double)a.fin[plane + off];
+        return d2_value(a.fin[plane + off], a.g.exact);
     }
 }
 
@@ -233,7 +250,8 @@ __global__ void __launch_bounds__(64) hd_envelope_kernel(const EnvParams<TOL> a)
         if (push) stk[++top * R] = (unsigned)q | ((unsigned)zq << 16);
     }
     const unsigned want = (unsigned)c | 0x80u;
-    float m = 0.0f;
+    const bool exact = a.g.exact;
+    unsigned m = 0u;
     bool any = false;
     double dsum = 0.0;
     unsigned cnt = 0, win = 0;
@@ -245,51 +263,55 @@ __global__ void __launch_bounds__(64) hd_envelope_kernel(const EnvParams<TOL> a)
         if constexpr (FOLD) {
             if (side_byte(a.rec[off], 1 - side) != want) continue;   // queries: the other side's border pixels of c
         }
-        float d = CUDART_INF_F;
+        double d2 = CUDART_INF;
         if (top >= 0) {
             while (k < top && (int)(stk[(k + 1) * R] >> 16) <= x) ++k;
             const int v = (int)(stk[k * R] & 0xFFFFu);
-            d = (float)(env_load<FROM_G>(a, plane, base + v * stride) + w * (double)(x - v) * (double)(x - v));
+            d2 = env_load<FROM_G>(a, plane, base + v * stride) + w * (double)(x - v) * (double)(x - v);
         }
-        if constexpr (FOLD) { m = fmaxf(m, d); any = true; }
-        else a.fout[plane + off] = d;
+        const unsigned key = d2_key(d2, exact);
+        if constexpr (FOLD) { m = max(m, key); any = true; }
+        else a.fout[plane + off] = key;
+        if constexpr (SURF || TOL) d2 = d2_value(key, exact);   // the d^2 the maxima and keys hold
         if constexpr (SURF) {
-            a.qd[side * a.g.N + off] = d;   // a pixel is a query of one class per side: no other line writes here
-            dsum += sqrt((double)d);
+            a.qd[side * a.g.N + off] = key;   // a pixel is a query of one class per side: no other line writes here
+            dsum += sqrt(d2);
             ++cnt;
         }
         if constexpr (TOL) {
             ++cnt;
-            if (sqrt((double)d) <= tol) ++win;   // d = +inf (no border on this side) is never within
+            if (sqrt(d2) <= tol) ++win;   // d2 = +inf (no border on this side) is never within
         }
     }
     if constexpr (FOLD && !TOL) {
         if (any) {
             const int64_t row = l / a.lines_per_row;
-            atomicMax(&a.rowmax[(row * a.g.C + c) * 2 + side], __float_as_uint(m));
+            atomicMax(&a.rowmax[(row * a.g.C + c) * 2 + side], m);
         }
     }
     if constexpr (SURF) { a.lsum[line] = dsum; a.lcnt[line] = cnt; }
     if constexpr (TOL) { a.lcnt[line] = cnt; a.lwin[line] = win; }
 }
 
+// the square root of the larger side's maximum, correctly rounded: at unit spacing of the exact integer d^2 (the double
+// square root rounded to float is the correctly rounded float square root, as 53 >= 2 * 24 + 2)
 __device__ __forceinline__ float hd_value(const unsigned* __restrict__ rowmax, const unsigned* __restrict__ present,
-                                          int64_t j) {
+                                          int64_t j, bool exact) {
     const bool both = present[2 * j] != 0u && present[2 * j + 1] != 0u;
-    const unsigned bits = max(rowmax[2 * j], rowmax[2 * j + 1]);
-    return both ? __fsqrt_rn(__uint_as_float(bits)) : CUDART_NAN_F;
+    const unsigned key = max(rowmax[2 * j], rowmax[2 * j + 1]);
+    if (!both) return CUDART_NAN_F;
+    return exact ? (float)sqrt((double)key) : __fsqrt_rn(__uint_as_float(key));
 }
 
 __global__ void hd_finish_kernel(const unsigned* __restrict__ rowmax, const unsigned* __restrict__ present, int64_t n,
-                                 float* __restrict__ hd) {
+                                 int exact, float* __restrict__ hd) {
     for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < n; j += (int64_t)gridDim.x * blockDim.x)
-        hd[j] = hd_value(rowmax, present, j);
+        hd[j] = hd_value(rowmax, present, j, exact);
 }
 
 // ---- surface distances (dct_surface_distances_i64): HD95, ASD, ASSD from the last pass's per-query d^2 -------------
 //
-// Per (row, class) the keys are the float bits of the d^2 of both sides' queries (non-negative floats order like their
-// bits).  HD95 is numpy's 'linear' percentile of the distances: with n keys, v = (n - 1) * 0.95, lo = floor(v), the
+// Per (row, class) the keys are the d2_key of the d^2 of both sides' queries.  HD95 is numpy's 'linear' percentile of the distances: with n keys, v = (n - 1) * 0.95, lo = floor(v), the
 // keys at ranks lo and lo + 1 are found by a radix select (4 passes of 8 bits, integer histograms) and, when the run of
 // keys equal to the one at rank lo ends there, one pass for the least key above it.
 struct SdState {
@@ -360,7 +382,7 @@ struct SdTasks {
 // the selected prefix, counted in shared memory per task and added to `hist`.  PASS 4: least key above the selected one
 // for the (row, class) that need it.  Every block runs the same number of iterations per task (whole warps vote).
 template <int PASS>
-__global__ void __launch_bounds__(256) sd_select_kernel(const uint16_t* __restrict__ rec, const float* __restrict__ qd,
+__global__ void __launch_bounds__(256) sd_select_kernel(const uint16_t* __restrict__ rec, const unsigned* __restrict__ qd,
                                                         const HdGeom g, const SdTasks tk, unsigned long long* hist,
                                                         SdState* st) {
     constexpr bool MIN = PASS == 4;
@@ -391,7 +413,7 @@ __global__ void __launch_bounds__(256) sd_select_kernel(const uint16_t* __restri
                 const int c = (int)(byte & 0x7Fu);
                 unsigned tag = 0xFFFFFFFFu, key = 0u;
                 if ((byte & 0x80u) && act[c]) {
-                    key = __float_as_uint(qd[s * g.N + p]);
+                    key = qd[s * g.N + p];
                     if constexpr (PASS == 0) {
                         tag = (unsigned)c * 256u + (key >> 24);
                     } else if constexpr (!MIN) {
@@ -464,7 +486,7 @@ __global__ void __launch_bounds__(256) sd_pick_kernel(unsigned long long* hist, 
 
 // out [4][n]: hd (as hd_finish_kernel), hd95, asd = mean of side 1's queries (pred border -> label border), assd
 __global__ void sd_finish_kernel(const unsigned* __restrict__ rowmax, const unsigned* __restrict__ present,
-                                 const SdState* __restrict__ st, int64_t n, float* __restrict__ out) {
+                                 const SdState* __restrict__ st, int64_t n, int exact, float* __restrict__ out) {
     for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < n; j += (int64_t)gridDim.x * blockDim.x) {
         const bool both = present[2 * j] != 0u && present[2 * j + 1] != 0u;
         float hd95 = CUDART_NAN_F, asd = CUDART_NAN_F, assd = CUDART_NAN_F;
@@ -472,15 +494,15 @@ __global__ void sd_finish_kernel(const unsigned* __restrict__ rowmax, const unsi
             const SdState& s = st[j];
             long long lo;
             const double t = sd_rank95(s.cnt[0] + s.cnt[1], &lo);
-            const double a = sqrt((double)__uint_as_float(s.prefix));
-            const double b = s.need_hi ? sqrt((double)__uint_as_float(s.hikey)) : a;
+            const double a = sqrt(d2_value(s.prefix, exact));
+            const double b = s.need_hi ? sqrt(d2_value(s.hikey, exact)) : a;
             const double d = b - a;
             hd95 = (float)(t >= 0.5 ? b - d * (1.0 - t) : a + d * t);   // numpy's _lerp
             const double m1 = s.sum[1] / (double)s.cnt[1], m0 = s.sum[0] / (double)s.cnt[0];
             asd = (float)m1;
             assd = (float)((m1 + m0) / 2.0);
         }
-        out[j] = hd_value(rowmax, present, j);
+        out[j] = hd_value(rowmax, present, j, exact);
         out[n + j] = hd95;
         out[2 * n + j] = asd;
         out[3 * n + j] = assd;
@@ -584,6 +606,10 @@ inline int hd_check_args(const int64_t* pred, const int64_t* labels, int C, int6
     return DCT_OK;
 }
 
+inline HdGeom hd_geom(int C, int64_t B, int64_t H, int64_t W, int volume, const double sp[3]) {
+    return HdGeom{C, B, H, W, B * H * W, volume ? 1 : 0, sp[0] == 1.0 && sp[1] == 1.0 && sp[2] == 1.0};
+}
+
 // classify, column and envelope passes (3 launches for '2d', 4 for a volume): leave the per-(row, class, side) maxima
 // and presence words in the scratch header and, with SURF, every query's d^2 and the last pass's per-line slots; with
 // TOL (tolerances `tol`, C host values) only the last pass's per-line query and within-tolerance counts
@@ -596,7 +622,7 @@ cudaError_t hd_distance_passes(const int64_t* pred, const int64_t* labels, const
     unsigned* present = rowmax + 2 * nrc;
     uint16_t* rec = reinterpret_cast<uint16_t*>(base + L.rec);
     uint16_t* gdist = reinterpret_cast<uint16_t*>(base + L.g);
-    float* f = reinterpret_cast<float*>(base + L.f);
+    unsigned* f = reinterpret_cast<unsigned*>(base + L.f);
 
     const int64_t cls_blocks = std::min<int64_t>((g.N + 255) / 256, (int64_t)kSMs * 16);
     hd_classify_kernel<<<(unsigned)cls_blocks, 256, 0, s>>>(pred, labels, g, rec, rowmax, (int)(4 * nrc), flags);
@@ -610,7 +636,7 @@ cudaError_t hd_distance_passes(const int64_t* pred, const int64_t* labels, const
     a.lines_per_plane = B * H; a.line_step = W; a.stride = 1; a.n = (int)W;
     a.w_in = sp[1] * sp[1]; a.w = sp[2] * sp[2];
     if (SURF) {
-        a.qd = reinterpret_cast<float*>(base + L.qd);
+        a.qd = reinterpret_cast<unsigned*>(base + L.qd);
         a.lsum = reinterpret_cast<double*>(base + L.lsum);
         a.lcnt = reinterpret_cast<unsigned*>(base + L.lcnt);
     }
@@ -643,7 +669,7 @@ inline SdTasks sd_tasks(const HdGeom& g) {
 }
 
 template <int PASS>
-cudaError_t launch_select(const uint16_t* rec, const float* qd, const HdGeom& g, const SdTasks& tk,
+cudaError_t launch_select(const uint16_t* rec, const unsigned* qd, const HdGeom& g, const SdTasks& tk,
                           unsigned long long* hist, SdState* st, cudaStream_t s) {
     const size_t smem = ((PASS == 4 ? (size_t)g.C : (size_t)g.C * 256) + 2 * (size_t)g.C) * 4;
     if (smem > 48 * 1024) {
@@ -676,7 +702,7 @@ extern "C" int dct_hausdorff_i64(const int64_t* pred, const int64_t* labels, int
     double sp[3];
     const int rc = hd_check_args(pred, labels, C, B, H, W, volume, spacing, hd, flags, scratch, sp);
     if (rc != DCT_OK) return rc;
-    const HdGeom g{C, B, H, W, B * H * W, volume ? 1 : 0};
+    const HdGeom g = hd_geom(C, B, H, W, volume, sp);
     const HdLayout L = hd_layout(C, B, H, W, volume);
     char* base = static_cast<char*>(scratch);
     const unsigned* rowmax = reinterpret_cast<const unsigned*>(base + L.hdr);
@@ -685,7 +711,7 @@ extern "C" int dct_hausdorff_i64(const int64_t* pred, const int64_t* labels, int
     cudaError_t e = hd_distance_passes<false>(pred, labels, g, sp, L, base, flags, s);
     if (e == cudaSuccess) {
         hd_finish_kernel<<<(unsigned)std::min<int64_t>((nrc + 127) / 128, 1024), 128, 0, s>>>(rowmax, rowmax + 2 * nrc,
-                                                                                               nrc, hd);
+                                                                                               nrc, g.exact, hd);
         e = cudaGetLastError();
     }
     if (e != cudaSuccess) { g_last_cuda_error = e; return DCT_ERR_CUDA; }
@@ -703,12 +729,12 @@ extern "C" int dct_surface_distances_i64(const int64_t* pred, const int64_t* lab
     double sp[3];
     const int rc = hd_check_args(pred, labels, C, B, H, W, volume, spacing, out, flags, scratch, sp);
     if (rc != DCT_OK) return rc;
-    const HdGeom g{C, B, H, W, B * H * W, volume ? 1 : 0};
+    const HdGeom g = hd_geom(C, B, H, W, volume, sp);
     const HdLayout L = hd_layout(C, B, H, W, volume);
     char* base = static_cast<char*>(scratch);
     const unsigned* rowmax = reinterpret_cast<const unsigned*>(base + L.hdr);
     const uint16_t* rec = reinterpret_cast<const uint16_t*>(base + L.rec);
-    const float* qd = reinterpret_cast<const float*>(base + L.qd);
+    const unsigned* qd = reinterpret_cast<const unsigned*>(base + L.qd);
     unsigned long long* hist = reinterpret_cast<unsigned long long*>(base + L.hist);
     SdState* st = reinterpret_cast<SdState*>(base + L.st);
     const int64_t nrc = (volume ? 1 : B) * C;
@@ -734,7 +760,7 @@ extern "C" int dct_surface_distances_i64(const int64_t* pred, const int64_t* lab
     if (e == cudaSuccess) e = launch_select<4>(rec, qd, g, tk, hist, st, s);
     if (e == cudaSuccess) {
         sd_finish_kernel<<<(unsigned)std::min<int64_t>((nrc + 127) / 128, 1024), 128, 0, s>>>(rowmax, rowmax + 2 * nrc,
-                                                                                              st, nrc, out);
+                                                                                              st, nrc, g.exact, out);
         e = cudaGetLastError();
     }
     if (e != cudaSuccess) { g_last_cuda_error = e; return DCT_ERR_CUDA; }
@@ -756,7 +782,7 @@ extern "C" int dct_surface_dice_i64(const int64_t* pred, const int64_t* labels, 
     for (int c = 0; c < C; ++c)
         if (!(tolerance[c] >= 0.0) || !std::isfinite(tolerance[c])) return DCT_ERR_BAD_ARG;   // also rejects NaN
     if (!aligned(counts, 8)) return DCT_ERR_MISALIGNED;
-    const HdGeom g{C, B, H, W, B * H * W, volume ? 1 : 0};
+    const HdGeom g = hd_geom(C, B, H, W, volume, sp);
     const HdLayout L = hd_layout(C, B, H, W, volume);
     char* base = static_cast<char*>(scratch);
     const int64_t nrc = (volume ? 1 : B) * C;

@@ -382,8 +382,9 @@ DCT_API int dct_vote_f32(const float* const* views, int K, int C, int64_t B, int
  *   hd        = max(max over border(A) of d(., border(G)), max over border(G) of d(., border(A))); NaN if A or G is empty.
  * Values outside [0,C) belong to no class (a non-c neighbour for every c) and are counted in flags[DCT_FLAG_PRED]
  * (pred) / flags[DCT_FLAG_LABEL] (labels).  Exact separable Euclidean distance transforms of the 2C border sets:
- * 4 launches for a slice batch, 5 for a volume; no host synchronisation.  At unit spacing hd is the correctly rounded
- * square root of the exact squared distance (while that stays below 2^24).
+ * 4 launches for a slice batch, 5 for a volume; no host synchronisation.  At unit spacing (spacing NULL or all ones) the
+ * squared distances are carried as exact integers, so hd is the correctly rounded square root of the exact squared
+ * distance for every accepted shape; otherwise they are rounded to float (within 1e-6 relative).
  * Limits (DCT_ERR_UNSUPPORTED): C <= DCT_MAX_CLASSES; H, W (and B when volume != 0) <= 32768 (each line's envelope stack
  * keeps 16-bit positions); 2*C*B*max(H,W) (and 2*C*H*W for a volume) <= 2^31 - 1.
  * ------------------------------------------------------------------------------------------ */
@@ -422,8 +423,8 @@ DCT_API int dct_surface_distances_i64(const int64_t* pred, const int64_t* labels
 /* Normalized surface Dice (surface Dice at tolerance tol[c]) of the same borders, grids and spacing, border-pixel form:
  * every border pixel counts once.  Per (row, class c), with S_pg and S_gp as for dct_surface_distances_i64 and a distance
  * to an empty border set being +inf (never within the tolerance):
- *   W_pg = #{s in S_pg : s <= tol[c]}, W_gp likewise, each s compared as sqrt((double)d^2) <= tol[c] on the float d^2 the
- *          distance passes produce (at unit spacing d^2 is exact, so the counts are those of scipy's EDT);
+ *   W_pg = #{s in S_pg : s <= tol[c]}, W_gp likewise, each s compared as sqrt((double)d^2) <= tol[c] on the d^2 the
+ *          distance passes produce (at unit spacing the exact integer, so the counts are those of scipy's EDT);
  *   nsd        = (W_pg + W_gp) / (|S_pg| + |S_gp|): NaN only when both borders are empty, 0 when exactly one is (a missed or
  *                hallucinated structure scores 0; unlike hd, which is NaN when either is empty);
  *   overlap_pg = W_pg / |S_pg|, overlap_gp = W_gp / |S_gp|: each NaN when its denominator is 0;

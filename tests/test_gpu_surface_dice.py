@@ -1,8 +1,8 @@
 """GPU parity of the normalized surface Dice (dct_surface_dice_i64 through ``dct_b200.surface_dice`` /
 ``SurfaceDiceMeter``) against the scipy restatement (oracle/oracle_surface_dice.py).
 
-At unit spacing every d^2 is an integer, so ``sqrt((double)d2) <= tol`` compares the same doubles scipy's EDT gives: the
-counts equal the oracle's exactly, tolerances equal to attained distances included, and nsd and the overlaps are the
+At unit spacing the kernels carry every d^2 as the exact integer, so ``sqrt((double)d2) <= tol`` compares the same doubles
+scipy's EDT gives: the counts equal the oracle's exactly, tolerances equal to attained distances included, and nsd and the overlaps are the
 oracle's double ratios rounded to float32.  At anisotropic spacing d^2 is rounded to float, so a count may differ only by
 the number of distances within 1e-6 relative of the tolerance; away from every attained distance the counts are exact."""
 import ctypes

@@ -1,8 +1,8 @@
 """GPU parity of the surface distances (dct_surface_distances_i64 through ``dct_b200.surface_distances`` /
 ``SurfaceDistanceMeter``) against the scipy restatement of medpy hd95 / asd / assd (oracle/oracle_surface.py).
 
-``hd`` equals ``hausdorff()`` bit for bit.  At unit spacing every d^2 is an integer below 2^24, so both sides interpolate
-the same doubles and ``hd95`` equals the oracle rounded to float32 bit for bit; ``asd`` / ``assd`` sum in another order
+``hd`` equals ``hausdorff()`` bit for bit.  At unit spacing the kernels carry every d^2 as the exact integer, so both sides
+interpolate the same doubles and ``hd95`` equals the oracle rounded to float32 bit for bit; ``asd`` / ``assd`` sum in another order
 (within 1e-6 relative).  At anisotropic spacing everything is within 1e-6 relative.  NaN where a class is absent from one
 side."""
 import ctypes
