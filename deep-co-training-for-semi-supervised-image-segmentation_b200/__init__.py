@@ -5,9 +5,10 @@ reference's own loss / meter / generator interfaces.
 Import as ``dct_b200`` (the repo-root alias module) or via importlib under the directory name.
 """
 from . import _lib, _runtime  # noqa: F401
-from . import loss, metrics, generators, utils, distributed, ensemble, components  # noqa: F401
+from . import loss, metrics, generators, utils, distributed, ensemble, components, distance  # noqa: F401
 from ._lib import DctError, build, library_path  # noqa: F401
 from .components import connected_components, largest_component  # noqa: F401
+from .distance import distance_transform_edt, signed_distance_map  # noqa: F401
 from ._runtime import get_check_mode, raise_if_flagged, set_check_mode  # noqa: F401
 from .ensemble import Ensembleway, Kappa2Annotator, KappaMetrics, KappaMetrics2, hard_vote, soft_vote, vote_class  # noqa: F401
 from .generators import FSGMGenerator, VATGenerator, fgsm_perturb, l2_normalize  # noqa: F401

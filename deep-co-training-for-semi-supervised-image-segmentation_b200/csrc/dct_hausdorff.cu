@@ -36,6 +36,13 @@
 // mode, which only counts per line the queries and the queries with sqrt((double)d^2) <= tol[c], then:
 //   nsd_finish_kernel    per (row, class): 64-bit sums of both sides' line counts; nsd, overlap_pg, overlap_gp, counts.
 // Launches: 4 for '2d', 5 for a volume.
+//
+// dct_distance_map_i64 (signed / inside Euclidean distance maps of one class map, scipy's EDT semantics: cells off the
+// grid are not features) runs the same transform on the sets {map != c} and, for signed maps, {map == c}:
+//   dm_classify_kernel   one class byte per pixel; zeroes the presence words.
+//   dm_column_kernel     hd_column_kernel with those feature sets.
+//   hd_envelope_kernel   as above; the last pass in its MAP mode writes each query's distance into the float map.
+// Launches: 3 for '2d', 4 for a volume.
 #include <math_constants.h>
 
 #include <algorithm>
@@ -177,6 +184,78 @@ __global__ void __launch_bounds__(128) hd_column_kernel(const uint16_t* __restri
     }
 }
 
+// ---- distance maps (dct_distance_map_i64): classify and column passes of one class map --------------------------------
+//
+// g.C counts the computed classes first_class .. first_class + g.C - 1; `sides` feature sets per class: side 0's
+// features are out_c = {byte != c} (the inside distances), side 1's, in signed mode only, in_c = {byte == c}.
+
+// scratch: uint32 present[rows][Cc][2], uint8 class byte [N], uint16 column distances [sides][Cc][N], and for a volume
+// uint32 d^2 keys [sides][Cc][N] after the row pass
+struct DmLayout {
+    size_t cls, g, f, total;
+};
+inline DmLayout dm_layout(int Cc, int64_t B, int64_t H, int64_t W, int volume, int sides) {
+    const size_t N = (size_t)B * H * W, rows = volume ? 1 : (size_t)B, sets = (size_t)sides * Cc;
+    DmLayout L;
+    L.cls = hd_align256(rows * Cc * 2 * 4);
+    L.g = hd_align256(L.cls + N);
+    L.f = hd_align256(L.g + sets * N * 2);
+    L.total = volume ? hd_align256(L.f + sets * N * 4) : L.f;
+    return L;
+}
+
+// one class byte per pixel (kOutOfRange for a value outside [0,C), counted in flags[DCT_FLAG_PRED]); zeroes the
+// presence words
+__global__ void __launch_bounds__(256) dm_classify_kernel(const int64_t* __restrict__ map, int64_t N, int C,
+                                                          unsigned char* __restrict__ cls, unsigned* present, int npres,
+                                                          int32_t* flags) {
+    const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, nthr = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = tid; i < npres; i += nthr) present[i] = 0u;
+    int bad = 0;
+    for (int64_t p = tid; p < N; p += nthr) {
+        const long long v = map[p];
+        const bool in = v >= 0 && v < C;
+        bad += !in;
+        cls[p] = in ? (unsigned char)v : kOutOfRange;
+    }
+    if (flags != nullptr) {
+        bad = __reduce_add_sync(0xffffffffu, bad);
+        if ((threadIdx.x & 31) == 0 && bad) atomicAdd(&flags[DCT_FLAG_PRED], bad);
+    }
+}
+
+// hd_column_kernel with the map's feature sets: one thread per (side, class, image, column)
+__global__ void __launch_bounds__(128) dm_column_kernel(const unsigned char* __restrict__ cls, const HdGeom g, int sides,
+                                                        int first_class, uint16_t* __restrict__ gdist,
+                                                        unsigned* present) {
+    const int64_t line = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int64_t per_sc = g.B * g.W;
+    if (line >= sides * g.C * per_sc) return;
+    const int sc = (int)(line / per_sc), side = sc / g.C, c = sc - side * g.C;
+    const int64_t r = line - sc * per_sc, b = r / g.W, x = r - b * g.W;
+    const int64_t base = b * g.H * g.W + x;
+    const unsigned char want = (unsigned char)(first_class + c);
+    const bool feat_in = side == 1;   // side 1: features in_c; side 0: out_c
+    const unsigned char* in = cls + base;
+    uint16_t* out = gdist + (int64_t)sc * g.N + base;
+    int last = -1;
+    for (int y = 0; y < g.H; ++y) {
+        if ((in[(int64_t)y * g.W] == want) == feat_in) last = y;
+        out[(int64_t)y * g.W] = last < 0 ? kNone : (uint16_t)(y - last);
+    }
+    if (last < 0) return;   // no feature in this column
+    present[((g.volume ? 0 : b) * g.C + c) * 2 + side] = 1u;
+    int next = -1;
+    for (int y = (int)g.H - 1; y >= 0; --y) {
+        const int64_t o = (int64_t)y * g.W;
+        if ((in[o] == want) == feat_in) next = y;
+        if (next >= 0) {
+            const uint16_t d = (uint16_t)(next - y);
+            if (d < out[o]) out[o] = d;
+        }
+    }
+}
+
 struct EnvArgs {
     const uint16_t* gdist;   // FROM_G: input distances in rows (weight w_in)
     const unsigned* fin;     // !FROM_G: input d^2 keys
@@ -198,8 +277,24 @@ struct EnvTolArgs : EnvArgs {
     unsigned* lwin;                  // per line of the last pass, number of its queries within tol[c]
     double tol[DCT_MAX_CLASSES];     // per class, in spacing units
 };
-template <bool TOL>
-using EnvParams = std::conditional_t<TOL, EnvTolArgs, EnvArgs>;
+// MAP (dct_distance_map_i64): g.C counts the computed classes first_class .. first_class + g.C - 1, and only `sides`
+// feature sets per class exist (1: the inside distances alone); the last pass writes the map itself
+struct EnvMapArgs : EnvArgs {
+    const unsigned char* cls;   // class byte per pixel (kOutOfRange outside [0,C))
+    const unsigned* present;    // [rows][g.C][2]: the column pass found a feature of that side
+    float* out;                 // [B][g.C][H][W]
+    int64_t HW, ostride;        // out index of pixel base + x * stride: base + (row * (g.C - 1) + c) * HW + x * ostride
+    int sides, first_class;
+};
+template <bool TOL, bool MAP = false>
+using EnvParams = std::conditional_t<TOL, EnvTolArgs, std::conditional_t<MAP, EnvMapArgs, EnvArgs>>;
+
+// lines of one envelope pass: one per (side, class, line of a plane)
+template <bool MAP>
+__host__ __device__ __forceinline__ int64_t env_lines(const EnvParams<false, MAP>& a) {
+    if constexpr (MAP) return (int64_t)a.sides * a.g.C * a.lines_per_plane;
+    else return 2 * a.g.C * a.lines_per_plane;
+}
 
 template <bool FROM_G>
 __device__ __forceinline__ double env_load(const EnvArgs& a, int64_t plane, int64_t off) {
@@ -211,19 +306,60 @@ __device__ __forceinline__ double env_load(const EnvArgs& a, int64_t plane, int6
     }
 }
 
+// MAP, last pass: the values of one line of class c's plane of the map, from the line's envelope (stack entries
+// stk[k * R], k <= top).  Side 0's features are out_c and its queries in_c: it writes -d (signed) or d (unsigned), and in
+// unsigned mode also the 0 of every other position.  Side 1's features are in_c and its queries out_c: it writes +d.
+// So every element of the plane is written by exactly one thread.  A signed plane is 0 where either feature set is
+// empty on the grid; an unsigned query with no out_c on the grid gets +inf, the d of the empty envelope.
+template <bool FROM_G>
+__device__ __forceinline__ void env_write_map(const EnvMapArgs& a, const unsigned* stk, int R, int top, int64_t plane,
+                                              int64_t base, int side, int c, int64_t l) {
+    const int64_t row = l / a.lines_per_row;
+    const bool is_signed = a.sides == 2;
+    const unsigned* pr = a.present + (row * a.g.C + c) * 2;
+    const bool empty = is_signed && (pr[0] == 0u || pr[1] == 0u);
+    const unsigned cls = (unsigned)(a.first_class + c);
+    float* out = a.out + base + (row * (a.g.C - 1) + c) * a.HW;
+    const int n = a.n;
+    const int64_t stride = a.stride, ostride = a.ostride;
+    const double w = a.w;
+    int k = 0;
+    for (int x = 0; x < n; ++x) {
+        const bool inside = a.cls[base + x * stride] == cls;
+        float v = 0.0f;
+        if (inside == (side == 0)) {   // a query of this side
+            if (!empty) {
+                while (k < top && (int)(stk[(k + 1) * R] >> 16) <= x) ++k;
+                double d2 = CUDART_INF;
+                if (top >= 0) {
+                    const int q = (int)(stk[k * R] & 0xFFFFu);
+                    d2 = env_load<FROM_G>(a, plane, base + q * stride) + w * (double)(x - q) * (double)(x - q);
+                }
+                v = (float)sqrt(d2);
+                if (is_signed && side == 0) v = -v;
+            }
+        } else if (is_signed) {
+            continue;   // the other side's line writes this position
+        }
+        out[x * ostride] = v;
+    }
+}
+
 // Lower envelope of {f(q) + w (x - q)^2} over the finite f(q) of one line, evaluated at the integer positions x of the
 // line.  Stack entry k = (position v_k, first integer position z_k at which parabola v_k is the lowest); a new parabola q
 // (to the right of every stacked one) is at or below v_k from ceil(sep) on, so v_k is popped when ceil(sep) <= z_k and q is
 // only pushed when ceil(sep) < n.  SURF (last pass of dct_surface_distances_i64): also keep every query's d^2 and the
 // line's sum of distances and query count.  TOL (last pass of dct_surface_dice_i64): instead of the maximum, only the
-// line's query count and the number of its queries with sqrt((double)d^2) <= tol[c].
-template <bool FROM_G, bool FOLD, bool SURF = false, bool TOL = false>
-__global__ void __launch_bounds__(64) hd_envelope_kernel(const EnvParams<TOL> a) {
+// line's query count and the number of its queries with sqrt((double)d^2) <= tol[c].  MAP (dct_distance_map_i64): the
+// line count follows a.sides and, in the last pass, env_write_map writes the line's values of the map.
+template <bool FROM_G, bool FOLD, bool SURF = false, bool TOL = false, bool MAP = false>
+__global__ void __launch_bounds__(64) hd_envelope_kernel(const EnvParams<TOL, MAP> a) {
     static_assert(FOLD || !(SURF || TOL), "only the last pass has queries");
     static_assert(!(SURF && TOL), "one query mode per pass");
+    static_assert(!(MAP && (SURF || TOL)), "the map is its own query mode");
     extern __shared__ unsigned stk_all[];
     const int64_t line = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (line >= 2 * a.g.C * a.lines_per_plane) return;
+    if (line >= env_lines<MAP>(a)) return;
     const int sc = (int)(line / a.lines_per_plane), side = sc / a.g.C, c = sc - side * a.g.C;
     const int64_t l = line - sc * a.lines_per_plane;
     const int64_t plane = (int64_t)sc * a.g.N, base = l * a.line_step, stride = a.stride;
@@ -248,6 +384,10 @@ __global__ void __launch_bounds__(64) hd_envelope_kernel(const EnvParams<TOL> a)
             break;
         }
         if (push) stk[++top * R] = (unsigned)q | ((unsigned)zq << 16);
+    }
+    if constexpr (MAP && FOLD) {
+        env_write_map<FROM_G>(a, stk, R, top, plane, base, side, c, l);
+        return;
     }
     const unsigned want = (unsigned)c | 0x80u;
     const bool exact = a.g.exact;
@@ -557,18 +697,18 @@ __global__ void __launch_bounds__(kNsdThreads) nsd_finish_kernel(const unsigned*
     }
 }
 
-template <bool FROM_G, bool FOLD, bool SURF = false, bool TOL = false>
-cudaError_t launch_envelope(const EnvParams<TOL>& a, cudaStream_t s) {
-    const int64_t lines = 2 * a.g.C * a.lines_per_plane;
+template <bool FROM_G, bool FOLD, bool SURF = false, bool TOL = false, bool MAP = false>
+cudaError_t launch_envelope(const EnvParams<TOL, MAP>& a, cudaStream_t s) {
+    const int64_t lines = env_lines<MAP>(a);
     int R = kEnvSmemBudget / (4 * a.n);
     R = R > 64 ? 64 : (R < 1 ? 1 : R);
     const size_t smem = (size_t)R * a.n * 4;
     if (smem > (size_t)kEnvSmemBudget) {
-        cudaError_t e = cudaFuncSetAttribute(hd_envelope_kernel<FROM_G, FOLD, SURF, TOL>,
+        cudaError_t e = cudaFuncSetAttribute(hd_envelope_kernel<FROM_G, FOLD, SURF, TOL, MAP>,
                                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
     }
-    hd_envelope_kernel<FROM_G, FOLD, SURF, TOL><<<(unsigned)((lines + R - 1) / R), R, smem, s>>>(a);
+    hd_envelope_kernel<FROM_G, FOLD, SURF, TOL, MAP><<<(unsigned)((lines + R - 1) / R), R, smem, s>>>(a);
     return cudaGetLastError();
 }
 
@@ -794,6 +934,63 @@ extern "C" int dct_surface_dice_i64(const int64_t* pred, const int64_t* labels, 
             reinterpret_cast<const unsigned*>(base + L.tq), reinterpret_cast<const unsigned*>(base + L.tw), C,
             lines_per_plane, lines_per_row, nrc, out, reinterpret_cast<long long*>(counts));
         e = cudaGetLastError();
+    }
+    if (e != cudaSuccess) { g_last_cuda_error = e; return DCT_ERR_CUDA; }
+    return DCT_OK;
+}
+
+extern "C" size_t dct_distance_map_scratch_bytes(int C, int first_class, int64_t B, int64_t H, int64_t W, int volume,
+                                                 int signed_map) {
+    if (C < 1 || C > DCT_MAX_CLASSES || first_class < 0 || first_class >= C || (signed_map != 0 && signed_map != 1))
+        return 0;
+    if (B < 1 || H < 1 || W < 1 || !hd_supported(C - first_class, B, H, W, volume)) return 0;
+    return dm_layout(C - first_class, B, H, W, volume, signed_map ? 2 : 1).total;
+}
+
+extern "C" int dct_distance_map_i64(const int64_t* map, int C, int first_class, int64_t B, int64_t H, int64_t W,
+                                    int volume, const double* spacing, int signed_map, float* out, int32_t* flags,
+                                    void* scratch, void* stream) {
+    if (C < 1 || first_class < 0 || first_class >= C || (signed_map != 0 && signed_map != 1)) return DCT_ERR_BAD_ARG;
+    if (C > DCT_MAX_CLASSES) return DCT_ERR_UNSUPPORTED;
+    const int Cc = C - first_class, sides = signed_map ? 2 : 1;
+    double sp[3];
+    const int rc = hd_check_args(map, map, Cc, B, H, W, volume, spacing, out, flags, scratch, sp);
+    if (rc != DCT_OK) return rc;
+    const HdGeom g = hd_geom(Cc, B, H, W, volume, sp);
+    const DmLayout L = dm_layout(Cc, B, H, W, volume, sides);
+    char* base = static_cast<char*>(scratch);
+    unsigned* present = reinterpret_cast<unsigned*>(base);
+    unsigned char* cls = reinterpret_cast<unsigned char*>(base + L.cls);
+    uint16_t* gdist = reinterpret_cast<uint16_t*>(base + L.g);
+    unsigned* f = reinterpret_cast<unsigned*>(base + L.f);
+    const int64_t nrc = (volume ? 1 : B) * Cc;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+
+    const int64_t cls_blocks = std::min<int64_t>((g.N + 255) / 256, (int64_t)kSMs * 16);
+    dm_classify_kernel<<<(unsigned)cls_blocks, 256, 0, s>>>(map, g.N, C, cls, present, (int)(2 * nrc), flags);
+    const int64_t col_lines = (int64_t)sides * Cc * B * W;
+    dm_column_kernel<<<(unsigned)((col_lines + 127) / 128), 128, 0, s>>>(cls, g, sides, first_class, gdist, present);
+    cudaError_t e = cudaGetLastError();
+
+    EnvMapArgs a{};
+    a.gdist = gdist; a.g = g;
+    a.lines_per_plane = B * H; a.line_step = W; a.stride = 1; a.n = (int)W;
+    a.w_in = sp[1] * sp[1]; a.w = sp[2] * sp[2];
+    a.cls = cls; a.present = present; a.out = out; a.HW = H * W; a.ostride = 1;
+    a.sides = sides; a.first_class = first_class;
+    if (e == cudaSuccess && !volume) {
+        a.lines_per_row = H;   // line l = b * H + y lies in image b
+        e = launch_envelope<true, true, false, false, true>(a, s);
+    } else if (e == cudaSuccess) {
+        a.fout = f;
+        e = launch_envelope<true, false, false, false, true>(a, s);
+        EnvMapArgs z = a;
+        z.gdist = nullptr; z.fout = nullptr; z.fin = f;
+        z.lines_per_plane = H * W; z.line_step = 1; z.stride = H * W; z.n = (int)B;
+        z.lines_per_row = H * W;   // one row: the volume
+        z.w_in = 0.0; z.w = sp[0] * sp[0];
+        z.ostride = (int64_t)Cc * H * W;
+        if (e == cudaSuccess) e = launch_envelope<false, true, false, false, true>(z, s);
     }
     if (e != cudaSuccess) { g_last_cuda_error = e; return DCT_ERR_CUDA; }
     return DCT_OK;

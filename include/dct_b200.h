@@ -446,6 +446,32 @@ DCT_API int dct_surface_dice_i64(const int64_t* pred, const int64_t* labels, int
                                  int volume, const double* spacing, const double* tolerance, float* out, int64_t* counts,
                                  int32_t* flags, void* scratch, void* stream);
 
+/* Euclidean distance maps of one class map (scipy.ndimage.distance_transform_edt semantics).  Grids and spacing as for
+ * dct_hausdorff_i64; d(x, S) = min over y in S of ||(x - y) * spacing||_2 with S taken on the grid only (cells off the
+ * grid are not features, unlike the border rule above).  For each computed class c = first_class .. C-1, with
+ * in_c = {map == c} and out_c its complement on the grid (values outside [0,C) are in out_c for every c and are counted
+ * in flags[DCT_FLAG_PRED]):
+ *   signed_map = 1:  phi_c(x) = d(x, in_c) for x in out_c, -d(x, out_c) for x in in_c (positive outside, negative
+ *                    inside, no offset); a grid on which in_c or out_c is empty has phi_c = 0 everywhere;
+ *   signed_map = 0:  d_in(x) = d(x, out_c) for x in in_c, 0 elsewhere (for a binary map and c = 1 scipy's
+ *                    distance_transform_edt(map != 0, sampling=spacing)); +inf on a grid that in_c fills, where scipy
+ *                    returns an artifact of its feature transform instead.  Only the inside feature sets are computed.
+ * out float32 [B][C - first_class][H][W], overwritten.  Each value is computed in double and rounded once to float: at
+ * unit spacing d^2 is the exact integer, so every value is the float of scipy's float64 value; otherwise within 1e-6
+ * relative.  Limits (DCT_ERR_UNSUPPORTED): C <= DCT_MAX_CLASSES and those of dct_hausdorff_i64 with C - first_class
+ * classes.  3 launches for a slice batch, 4 for a volume; no host synchronisation, no allocation, no copies. */
+
+/* bytes of `scratch` dct_distance_map_i64 needs: 8 per computed class and row (rows = B for a slice batch, 1 for a
+ * volume) + 1 per pixel + 2*S*(C - first_class) per pixel, + 4*S*(C - first_class) per pixel for a volume, with S = 2
+ * (signed_map = 1) or 1, each region rounded up to 256 bytes; 0 for arguments dct_distance_map_i64 rejects.  Host only. */
+DCT_API size_t dct_distance_map_scratch_bytes(int C, int first_class, int64_t B, int64_t H, int64_t W, int volume,
+                                              int signed_map);
+/* map int64 [B,H,W]; first_class in [0, C) and signed_map in {0, 1}, else DCT_ERR_BAD_ARG; spacing, flags, scratch as
+ * for dct_hausdorff_i64 (scratch >= dct_distance_map_scratch_bytes()). */
+DCT_API int dct_distance_map_i64(const int64_t* map, int C, int first_class, int64_t B, int64_t H, int64_t W, int volume,
+                                 const double* spacing, int signed_map, float* out, int32_t* flags, void* scratch,
+                                 void* stream);
+
 /* ------------------------------------------------------------------------------------------
  * Connected components of a class map (evaluation path: the post-processing in front of the Dice and surface distances;
  * getLargestCC of the UA-MT / DTC / MC-Net test scripts, nnU-Net's "remove all but the largest component").
