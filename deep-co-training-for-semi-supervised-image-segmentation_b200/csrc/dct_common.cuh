@@ -274,14 +274,25 @@ __device__ __forceinline__ void grid_sum_to(double v, Workspace* ws, double* out
 // Every per-thread fp32 partial (the sum of one thread's 1..4 pixel values of one tile) is
 // converted exactly to 2^-40 fixed point (fp32 * 2^40 is exact; the int64 conversion is exact for
 // |partial| < 2^23) and accumulated with integer adds, which are associative: the result does not
-// depend on which CTA processed which tile.  Low and high halves are summed separately so that
-// nothing can overflow (N < 2^31 partials).  NaN / inf partials poison the result (NaN).
+// depend on which CTA processed which tile.  A fixed value can be as large as 2^63, so a plain int64
+// running sum wraps after two of them: every add (FxAcc) and every later stage keeps the sum of the
+// low 32 bits (unsigned) apart from the sum of the signed high bits, and neither can overflow for
+// N < 2^31 partials.  A partial with |partial| >= 2^23, NaN or inf poisons the result (NaN).
 // ---------------------------------------------------------------------------------------------
 constexpr float kFxScale = 1099511627776.0f;  // 2^40
 __device__ __forceinline__ long long to_fixed(float part, bool& nonfinite) {
     nonfinite |= !(fabsf(part) < 8388608.0f);
     return __float2ll_rn(part * kFxScale);
 }
+// One thread's running sum of fixed-point partials: lo < n * 2^32 and |hi| <= n * 2^31 after n adds.
+struct FxAcc {
+    unsigned long long lo = 0ull;
+    long long hi = 0ll;
+    __device__ __forceinline__ void add(long long fx) {
+        lo += (unsigned long long)fx & 0xffffffffull;
+        hi += fx >> 32;
+    }
+};
 __device__ __forceinline__ long long warp_sum(long long v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -291,9 +302,11 @@ __device__ __forceinline__ long long warp_sum(long long v) {
 // Called by every thread of the CTA at the end of a tile-pipeline kernel.  `out` may be null.
 // Also re-arms the workspace header (ticket, tile counter, accumulators) when the last CTA is through.
 // SUM2: a second, independent sum (acc_fx2 / nonfinite2 -> ws->fx2_* -> *out2, nullable) with the same scheme.
+// Each thread first carries its low sum's bits above 32 into the high sum; the (lo, hi) pair then holds the same value
+// with lo < 2^32 (for a sum that a single int64 held, exactly that int64's low and high halves).
 template <bool PUB = false, bool SUM2 = false>
-__device__ __forceinline__ void tile_grid_finish(long long acc_fx, bool nonfinite, Workspace* ws, double* out, int num_ctas,
-                                                 const PeerPub* pub = nullptr, int pub_early = 0, long long acc_fx2 = 0,
+__device__ __forceinline__ void tile_grid_finish(const FxAcc& acc_fx, bool nonfinite, Workspace* ws, double* out, int num_ctas,
+                                                 const PeerPub* pub = nullptr, int pub_early = 0, const FxAcc& acc_fx2 = FxAcc{},
                                                  bool nonfinite2 = false, double* out2 = nullptr) {
     if (ws == nullptr) return;
     __shared__ long long s_lo[SUM2 ? 40 : 20], s_hi[SUM2 ? 40 : 20];  // <= 17 warps per CTA (second sum at +20)
@@ -301,7 +314,7 @@ __device__ __forceinline__ void tile_grid_finish(long long acc_fx, bool nonfinit
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = (blockDim.x + 31) >> 5;
     if (out != nullptr) {
         if (threadIdx.x == 0) s_nf = 0;
-        long long lo = (long long)((unsigned long long)acc_fx & 0xffffffffull), hi = acc_fx >> 32;
+        long long lo = (long long)(acc_fx.lo & 0xffffffffull), hi = acc_fx.hi + (long long)(acc_fx.lo >> 32);
         lo = warp_sum(lo);
         hi = warp_sum(hi);
         const bool wnf = __any_sync(0xffffffffu, nonfinite);
@@ -311,7 +324,7 @@ __device__ __forceinline__ void tile_grid_finish(long long acc_fx, bool nonfinit
     if constexpr (SUM2) {
         if (out2 != nullptr) {
             if (threadIdx.x == 0) s_nf2 = 0;
-            long long lo = (long long)((unsigned long long)acc_fx2 & 0xffffffffull), hi = acc_fx2 >> 32;
+            long long lo = (long long)(acc_fx2.lo & 0xffffffffull), hi = acc_fx2.hi + (long long)(acc_fx2.lo >> 32);
             lo = warp_sum(lo);
             hi = warp_sum(hi);
             const bool wnf = __any_sync(0xffffffffu, nonfinite2);

@@ -339,9 +339,9 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
         }
     }
 
-    long long acc_fx = 0;     // this thread's share of the map sum, 2^-40 fixed point
+    FxAcc acc_fx;             // this thread's share of the map sum, 2^-40 fixed point
     bool nonfinite = false;
-    long long acc_fx2 = 0;    // SUM2: the same for the second value
+    FxAcc acc_fx2;            // SUM2: the same for the second value
     bool nonfinite2 = false;
     bool bad = false;
 
@@ -722,10 +722,10 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
                         }
                 }
                 if constexpr (Op::HAS_MAP) {
-                    acc_fx += to_fixed(part, nonfinite);
+                    acc_fx.add(to_fixed(part, nonfinite));
                     if (a.map != nullptr) st_stream<PPT>(a.map + (int64_t)b * HW + off + p0, mapv);
                 }
-                if constexpr (SUM2) acc_fx2 += to_fixed(part2, nonfinite2);
+                if constexpr (SUM2) acc_fx2.add(to_fixed(part2, nonfinite2));
 #pragma unroll
                 for (int n = 0; n < NOUT; ++n)
                     if (a.out[n] != nullptr) {

@@ -32,6 +32,13 @@
  *    incoming gradient is   gconst * (gscalar ? *gscalar : 1) * (gmap ? gmap[b,i] : 1).
  *  - Return value: DCT_OK (0) or a negative DCT_ERR_* code; nothing was launched
  *    on error except where noted.
+ *  - `sum` (double[1], nullable) of a loss map m with N pixels: deterministic (the same
+ *    inputs give the same bits, whatever the schedule), and within
+ *    2^-22 * sum_i |m_i| + N * 2^-41 of the float64 sum of the map the same call writes.
+ *    It is finite whenever every map value is finite with |v| < 2^21, and non-finite
+ *    (NaN or +-inf) when a map value is non-finite.  On the tile pipeline (the kernels
+ *    that add the map in 2^-40 fixed point) it may be NaN when a value has |v| >= 2^21:
+ *    it is NaN as soon as the sum of one thread's 1, 2 or 4 pixels of a tile reaches 2^23.
  */
 #ifndef DCT_B200_H
 #define DCT_B200_H

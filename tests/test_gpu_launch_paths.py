@@ -539,40 +539,48 @@ SUM_OPS = {"jsd_fwd": "pp", "jsd_fwdbwd": "zz", "ce_fwd": "z-", "ce_fwdbwd": "z-
 
 
 def _sum_call(op, h, C, B, HW, bufs, ws):
-    """Calls `op` with the loss sum into bufs['sum']; returns its status."""
+    """Calls `op` with the loss sum into bufs['sum']; returns its status.  Optional: the map into bufs['map'], the
+    cross-entropy class weights from bufs['w']."""
     a, b, g0, g1, lab = bufs["a"], bufs["b"], bufs["g0"], bufs["g1"], bufs["lab"]
     sm, s = bufs["sum"].data_ptr(), _s()
-    P = lambda t: t.data_ptr()  # noqa: E731
+    P = lambda t: None if t is None else t.data_ptr()  # noqa: E731
+    mp, w = P(bufs.get("map")), P(bufs.get("w"))
     if op == "jsd_fwd":
-        return h.dct_jsd_fwd_f32(ptrs([a, b]), 2, C, B, HW, IN_PROBS, None, sm, None, ws, s)
+        return h.dct_jsd_fwd_f32(ptrs([a, b]), 2, C, B, HW, IN_PROBS, mp, sm, None, ws, s)
     if op == "jsd_fwdbwd":
-        return h.dct_jsd_fwdbwd_f32(ptrs([a, b]), 2, C, B, HW, IN_LOGITS, 1.0, None, sm, ptrs([g0, g1]), None, None, 0,
+        return h.dct_jsd_fwdbwd_f32(ptrs([a, b]), 2, C, B, HW, IN_LOGITS, 1.0, mp, sm, ptrs([g0, g1]), None, None, 0,
                                     None, ws, s)
     if op == "ce_fwd":
-        return h.dct_ce_fwd_f32(P(a), P(lab), C, B, HW, None, 255, None, sm, None, ws, s)
+        return h.dct_ce_fwd_f32(P(a), P(lab), C, B, HW, w, 255, mp, sm, None, ws, s)
     if op == "ce_fwdbwd":
-        return h.dct_ce_fwdbwd_f32(P(a), P(lab), C, B, HW, None, 255, None, 1.0, None, sm, P(g0), None, None, ws, s)
+        return h.dct_ce_fwdbwd_f32(P(a), P(lab), C, B, HW, w, 255, None, 1.0, mp, sm, P(g0), None, None, ws, s)
     if op == "kl_fwd":
-        return h.dct_kl_fwd_f32(P(a), P(b), C, B, HW, EPS, None, sm, None, ws, s)
+        return h.dct_kl_fwd_f32(P(a), P(b), C, B, HW, EPS, mp, sm, None, ws, s)
     if op == "kl_logit":
-        return h.dct_kl_logit_f32(P(a), P(b), C, B, HW, None, sm, 0, None, None, 1.0, None, None, ws, s)
+        return h.dct_kl_logit_f32(P(a), P(b), C, B, HW, mp, sm, 0, None, None, 1.0, None, None, ws, s)
     if op == "kl_from_logits":
-        return h.dct_kl_from_logits_fwdbwd_f32(P(a), P(b), C, B, HW, EPS, 1.0, None, sm, P(g0), None, ws, s)
+        return h.dct_kl_from_logits_fwdbwd_f32(P(a), P(b), C, B, HW, EPS, 1.0, mp, sm, P(g0), None, ws, s)
     if op == "kl_div_fwd":
-        return h.dct_kl_div_fwd_f32(P(a), P(b), C, B, HW, EPS, None, sm, None, ws, s)
+        return h.dct_kl_div_fwd_f32(P(a), P(b), C, B, HW, EPS, mp, sm, None, ws, s)
     if op == "entropy_fwd":
-        return h.dct_entropy_fwd_f32(P(a), C, B, HW, None, sm, None, ws, s)
+        return h.dct_entropy_fwd_f32(P(a), C, B, HW, mp, sm, None, ws, s)
     raise AssertionError(op)
 
 
 def _sum_ref(op, a, b, gt, oracle):
     """float64 sum and pixel count of the op's loss map, from the float64 oracle on the op's own inputs."""
+    m = _map_ref(op, a, b, gt, oracle)
+    return float(m.sum(dtype=np.float64)), m.size
+
+
+def _map_ref(op, a, b, gt, oracle, w=None):
+    """The op's loss map from the float64 oracle on the op's own inputs (`w`: cross-entropy class weights)."""
     if op == "jsd_fwd":
         m = oracle.jsd_fwd([a, b])
     elif op == "jsd_fwdbwd":
         m = oracle.jsd_fwd([oracle.softmax(a), oracle.softmax(b)])
     elif op in ("ce_fwd", "ce_fwdbwd"):
-        m = oracle.cross_entropy(a, gt, reduction="none", want_grad=False)[0]
+        m = oracle.cross_entropy(a, gt, weight=w, reduction="none", want_grad=False)[0]
     elif op == "kl_fwd":
         m = oracle.kl_fwd(a, b, EPS)
     elif op == "kl_logit":
@@ -583,7 +591,7 @@ def _sum_ref(op, a, b, gt, oracle):
         m = oracle.kl_div_fwd(a, b, EPS)
     else:
         m = oracle.entropy(a)
-    return float(m.sum(dtype=np.float64)), m.size
+    return m
 
 
 # (C, HW) of shapes that never tile: HW = 1 takes the runtime-C kernels, HW = 2 at C = 19 the register-tiled VEC = 2
