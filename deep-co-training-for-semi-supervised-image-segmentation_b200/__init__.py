@@ -16,7 +16,8 @@ from .install import install, uninstall  # noqa: F401
 from .loss import (JSD, JSD_2D, CrossEntropyLoss2d, Entropy, Entropy_2D, FusedJSDConsistency, KL_div, KL_Divergence_2D,  # noqa: F401
                    KL_Divergence_2D_Logit, get_loss_fn, jsd_consistency_from_logits, jsd_map_from_logits,
                    kl_consistency_from_logits, kl_div_with_logit, softmax_dim1, supervised_from_logits)
-from .metrics import (ConfusionMatrix, DiceMeter, DiceMeter2, HausdorffMeter, IoU, SurfaceDiceMeter,  # noqa: F401
-                      SurfaceDistanceMeter, dice_counts, dice_from_counts, hausdorff, surface_dice, surface_distances)
+from .metrics import (BoundaryIoUMeter, ConfusionMatrix, DiceMeter, DiceMeter2, HausdorffMeter, IoU,  # noqa: F401
+                      SurfaceDiceMeter, SurfaceDistanceMeter, boundary_iou, dice_counts, dice_from_counts, hausdorff,
+                      surface_dice, surface_distances)
 
 __version__ = "0.1.0"

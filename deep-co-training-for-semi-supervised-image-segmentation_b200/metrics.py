@@ -9,13 +9,15 @@ Mirrors ``generalframework/metrics`` of the reference:
 plus ``hausdorff`` / ``HausdorffMeter``: the Hausdorff distance Summary.py:25 takes from the external ``deepclustering``
 package, with the definition of ``medpy.metric.binary.hd`` (exact distance transforms on the device), and
 ``surface_distances`` / ``SurfaceDistanceMeter``: HD95, ASD and ASSD (``medpy.metric.binary`` hd95 / asd / assd) from the
-same distance transforms, and ``surface_dice`` / ``SurfaceDiceMeter``: the normalized surface Dice at a tolerance.
+same distance transforms, and ``surface_dice`` / ``SurfaceDiceMeter``: the normalized surface Dice at a tolerance, and
+``boundary_iou`` / ``BoundaryIoUMeter``: Boundary IoU (Cheng et al., CVPR 2021) for the Cityscapes evaluation loop.
 
 ``add`` never leaves the device (no one-hot tensors, no ``torch.unique(a.cpu())``, no numpy
 ``bincount``); ``value()`` / ``summary()`` keep the reference's return structures.  Counts are exact
 int64; ``conf`` is exposed as the reference's ``np.int32`` view.
 """
 import ctypes
+import math
 
 import numpy as np
 import torch
@@ -490,6 +492,132 @@ class SurfaceDiceMeter(Metric):
     def summary(self) -> dict:
         (mean, var), _ = self.value()
         return {'mNSD': mean.item(), 'mNSDVars': var.item()}
+
+
+def boundary_dilation(H: int, W: int, dilation_ratio=0.02, dilation=None) -> int:
+    """Band width ``d`` of ``boundary_iou``: ``dilation`` if given, else ``max(1, int(round(dilation_ratio *
+    sqrt(H**2 + W**2))))`` in float64 with Python's ``round`` (half to even), as ``mask_to_boundary`` computes it."""
+    r = float(dilation_ratio)
+    if not (math.isfinite(r) and r > 0):
+        raise ValueError(f"boundary_iou: dilation_ratio must be finite and > 0, got {dilation_ratio}")
+    if dilation is not None:
+        if int(dilation) != dilation or dilation < 1:
+            raise ValueError(f"boundary_iou: dilation must be an integer >= 1, got {dilation}")
+        return int(dilation)
+    return max(1, int(round(r * math.sqrt(H ** 2 + W ** 2))))
+
+
+def _ignore_arg(ignore_index, C):
+    if ignore_index is None:
+        return -1
+    if int(ignore_index) != ignore_index or ignore_index < C:
+        raise ValueError(f"boundary_iou: ignore_index must be None or an integer >= C={C}, got {ignore_index}")
+    return int(ignore_index)
+
+
+def boundary_iou(pred, gt, C=None, dilation_ratio=0.02, dilation=None, ignore_index=None) -> dict:
+    """Boundary IoU (Cheng et al., CVPR 2021) per image and class from one device call: ``{'biou': float32 [B, C],
+    'counts': int64 [B, C, 3]}`` on the input's device.
+
+    Definition of ``mask_to_boundary`` (boundary-iou-api): the band of a class mask ``M`` is ``M`` minus its erosion by
+    a 3 x 3 square ``d`` times, with the grid's outside as background -- the pixels of ``M`` whose (2d+1) x (2d+1)
+    square leaves the grid or ``M``.  ``counts[b, c]`` = ``(I, G, P)`` = ``(|band(P) & band(G) & valid|, |band(G)|,
+    |band(P) & valid|)`` with ``P = pred == c``, ``G = gt == c`` and ``valid = gt != ignore_index``; ``biou`` = ``I / (G + P
+    - I)``, the float32 of the float64 quotient, NaN when the class is absent from both.  Sum ``counts`` over a dataset
+    to pool the Boundary IoU exactly (``BoundaryIoUMeter``).
+
+    ``pred``: float32 scores ``[B,C,H,W]`` -- reduced with the raw arg-max ``IoU.add`` uses (``torch.max`` semantics), so
+    the IoU and the Boundary IoU of one batch describe the same segmentation -- or an integer class map ``[B,H,W]`` /
+    ``[B,1,H,W]`` (then ``C`` is required).  ``gt``: integer ``[B,H,W]`` / ``[B,1,H,W]``.  ``d`` = ``dilation`` if given,
+    else ``max(1, round(dilation_ratio * sqrt(H^2 + W^2)))`` (``boundary_dilation``).  ``ignore_index``: a label value
+    ``>= C`` left out of every count (e.g. 255), or None.  Values outside ``[0, C)`` belong to no class and raise the
+    label / prediction range checks under the current check mode.
+    """
+    if pred.is_floating_point():
+        from .utils import _classmap
+        assert pred.dim() == 4, f"boundary_iou: scores [B,C,H,W] expected, got {tuple(pred.shape)}"
+        if pred.dtype != torch.float32:
+            raise TypeError(f"boundary_iou: float32 scores expected, got {pred.dtype}")
+        assert C is None or C == pred.shape[1], f"C={C} does not match scores {tuple(pred.shape)}"
+        p, C = _classmap(pred.detach(), 0, want_cls=True)[0], pred.shape[1]
+    else:
+        assert C is not None, "boundary_iou: C is required for an integer class map"
+        p = _class_map(pred, C, "boundary_iou")
+    g = _class_map(gt, C, "boundary_iou")
+    assert g.shape == p.shape, f"label shape {tuple(gt.shape)} does not match prediction {tuple(pred.shape)}"
+    B, H, W = p.shape
+    d = boundary_dilation(H, W, dilation_ratio, dilation)
+    ignore = _ignore_arg(ignore_index, C)
+    h = _lib.lib()
+    nbytes = h.dct_boundary_iou_scratch_bytes(C, B, H, W)
+    if nbytes == 0:
+        _lib.check(_lib.ERR_UNSUPPORTED, f"dct_boundary_iou_scratch_bytes (C={C}, shape {(B, H, W)})")
+    scratch = torch.empty(nbytes, dtype=torch.uint8, device=p.device)
+    biou = torch.empty((B, C), dtype=torch.float32, device=p.device)
+    counts = torch.empty((B, C, 3), dtype=torch.int64, device=p.device)
+    st = _runtime.state(p.device)
+    _lib.check(h.dct_boundary_iou_i64(p.data_ptr(), g.data_ptr(), C, B, H, W, d, ignore, biou.data_ptr(),
+                                      counts.data_ptr(), _runtime.flags_ptr(st), scratch.data_ptr(),
+                                      _runtime.stream_ptr(p.device)), "dct_boundary_iou_i64")
+    _runtime.after_call(st)
+    return {'biou': biou, 'counts': counts}
+
+
+class BoundaryIoUMeter(Metric):
+    """Boundary IoU per class pooled over a dataset, next to ``IoU`` (definition of ``boundary_iou``).  ``add`` sums each
+    batch's counts into one int64 ``[C, 3]`` device tensor without synchronising the host; ``value()`` reads it once.
+    Under data parallelism, pool the ranks with ``distributed.all_reduce_counts(meter.device_counts(dev))`` before
+    ``value()``."""
+
+    def __init__(self, C, dilation_ratio=0.02, dilation=None, ignore_index=None, report_axises='all') -> None:
+        super().__init__()
+        assert report_axises == 'all' or isinstance(report_axises, list)
+        if int(C) != C or not 1 <= C <= _lib.MAX_CLASSES:
+            raise ValueError(f"BoundaryIoUMeter: C must be an integer in [1, {_lib.MAX_CLASSES}], got {C}")
+        boundary_dilation(1, 1, dilation_ratio, dilation)   # argument checks at construction
+        _ignore_arg(ignore_index, C)
+        self.C = C
+        self.dilation_ratio = dilation_ratio
+        self.dilation = dilation
+        self.ignore_index = ignore_index
+        self.report_axis = report_axises
+        self._counts = None
+
+    def reset(self):
+        if self._counts is not None:
+            self._counts.zero_()
+
+    def device_counts(self, device) -> torch.Tensor:
+        """The int64 ``[C, 3]`` accumulator ``(I, G, P)`` on ``device`` (moved there if it lives elsewhere)."""
+        device = torch.device(device)
+        if self._counts is None:
+            self._counts = torch.zeros((self.C, 3), dtype=torch.int64, device=device)
+        elif self._counts.device != device:
+            self._counts = self._counts.to(device)
+        return self._counts
+
+    def add(self, pred, gt):
+        r = boundary_iou(pred, gt, C=self.C, dilation_ratio=self.dilation_ratio, dilation=self.dilation,
+                         ignore_index=self.ignore_index)
+        self.device_counts(r['counts'].device).add_(r['counts'].sum(0))
+
+    def value(self, **kwargs):
+        """``(mean, per_class)``: the pooled Boundary IoU per class, float64 ``[C]`` (NaN for a class absent from every
+        prediction and label so far), and its mean over the report axes with NaN skipped."""
+        counts = (self._counts.cpu() if self._counts is not None
+                  else torch.zeros((self.C, 3), dtype=torch.int64)).to(torch.float64)
+        inter, union = counts[:, 0], counts[:, 1] + counts[:, 2] - counts[:, 0]
+        per_class = torch.where(union > 0, inter / union.clamp(min=1), torch.full_like(inter, float('nan')))
+        axes = per_class if self.report_axis == 'all' else per_class[self.report_axis]
+        return torch.nanmean(axes), per_class
+
+    def detailed_summary(self) -> dict:
+        _, per_class = self.value()
+        return {f'BIoU{i}': per_class[i].item() for i in range(self.C)}
+
+    def summary(self) -> dict:
+        mean, _ = self.value()
+        return {'mBIoU': mean.item()}
 
 
 class ConfusionMatrix(Metric):

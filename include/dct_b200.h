@@ -508,6 +508,35 @@ DCT_API size_t dct_components_scratch_bytes(int C, int64_t B, int64_t H, int64_t
 DCT_API int dct_components_i64(const int64_t* map, int C, int64_t B, int64_t H, int64_t W, int volume, int connectivity, int32_t* labels, int64_t* stats, int64_t* largest_map, int32_t* flags, void* scratch, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Boundary IoU (Cheng et al., CVPR 2021; boundary-iou-api mask_to_boundary) of a class map against a label map, per
+ * H x W image: the boundary-quality measure of the Cityscapes evaluation loop (cotraining_city.py:320, trainer_city.py:141
+ * report region IoU only).  For image b and class c, with M one of P = {pred == c}, G = {labels == c}:
+ *   band(M) = M - erode(pad(M, 1, value 0), ones(3, 3), iterations = d)[1:H+1, 1:W+1]: x is in band(M) when x is in M
+ *             and some cell of the (2d+1) x (2d+1) square centred on x is off the grid or outside M (every pixel of M
+ *             when 2d+1 > H or W);
+ *   valid   = labels != ignore_index (every pixel when ignore_index < 0); an ignored pixel belongs to no class;
+ *   counts[b][c] = (I, G, P) = (|band(P) & band(G) & valid|, |band(G)|, |band(P) & valid|);
+ *   biou[b][c]   = float(double(I) / (G + P - I)), NaN when the union is empty.
+ * Summing the counts over a dataset pools the Boundary IoU exactly.  Values outside [0,C) belong to no class and are
+ * counted in flags[DCT_FLAG_PRED] (pred) / flags[DCT_FLAG_LABEL] (labels other than ignore_index).  The square test is
+ * separated into run-length tests along H and along W (the work per pixel does not depend on d); the counts are 64-bit
+ * integer sums, bit-reproducible.  3 launches; no host synchronisation, no allocation, no copies.
+ * Limits (DCT_ERR_UNSUPPORTED): C <= DCT_MAX_CLASSES, B*H*W <= 2^31 - 1 (int32 pixel indices).
+ * ------------------------------------------------------------------------------------------ */
+
+/* bytes of `scratch` dct_boundary_iou_i64 needs: 2 per pixel (one record byte per map) + 24 per (image, class), each
+ * rounded up to 256 bytes; 0 for a shape it rejects.  Host only. */
+DCT_API size_t dct_boundary_iou_scratch_bytes(int C, int64_t B, int64_t H, int64_t W);
+/* pred, labels int64 [B,H,W]; dilation d >= 1 (else DCT_ERR_BAD_ARG; any d >= 1 is accepted); ignore_index < 0 for none,
+ * a value in [0,C) is DCT_ERR_BAD_ARG; biou float32 [B][C] and counts (nullable) int64 [B][C][3], overwritten; flags as
+ * above (nullable); scratch: >= dct_boundary_iou_scratch_bytes() bytes, 256-byte aligned, no initial state required,
+ * private to the call until the stream reaches its end.  Null pointers are DCT_ERR_BAD_ARG and misaligned ones
+ * DCT_ERR_MISALIGNED, as for dct_surface_dice_i64, with nothing launched. */
+DCT_API int dct_boundary_iou_i64(const int64_t* pred, const int64_t* labels, int C, int64_t B, int64_t H, int64_t W,
+                                 int64_t dilation, int64_t ignore_index, float* biou, int64_t* counts,
+                                 int32_t* flags, void* scratch, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * bfloat16 twins of the one-pass-over-logits entry points (networks under torch.autocast emit bf16 logits;
  * north_star: "within 1e-2 relative in bf16").  Tensors [B,C,HW] are bfloat16 (2-byte elements, same NCHW
  * layout), gradients are written as bfloat16 (round-to-nearest-even); ALL arithmetic is fp32 in registers and the
