@@ -44,6 +44,7 @@ _SIGNATURES = {
     "dct_jsd_fwdbwd_pub_f32": [_p, _i, _i, _i64, _i64, _i, _f, _p, _p, _p, _p, _p, _i, _p, _p, _p, _p],
     "dct_jsd_vat_kl_fwdbwd_f32": [_p, _i, _i, _i64, _i64, _f, _p, _p, _p, _p, _i, _p, _f, _p, _p, _p, _p, _p, _p],
     "dct_scale_if_not_one_f32": [_p, _i64, _p, _p],
+    "dct_scale_if_not_one_bf16": [_p, _i64, _p, _p],
     "dct_kl_fwd_f32": [_p, _p, _i, _i64, _i64, _f, _p, _p, _p, _p, _p],
     "dct_kl_bwd_f32": [_p, _p, _i, _i64, _i64, _f, _p, _p, _f, _p, _p, _p],
     "dct_kl_logit_f32": [_p, _p, _i, _i64, _i64, _p, _p, _i, _p, _p, _f, _p, _p, _p, _p],

@@ -32,12 +32,15 @@ static int jsd_dispatch(const JsdCall& c) {
     if (c.views == nullptr || c.K < 1 || c.C < 1 || c.B < 1 || c.HW < 1) return DCT_ERR_BAD_ARG;
     if (c.K > DCT_MAX_VIEWS || c.C > DCT_MAX_CLASSES || c.B > 65535) return DCT_ERR_UNSUPPORTED;
     if (c.in_kind != DCT_IN_PROBS && c.in_kind != DCT_IN_LOGITS) return DCT_ERR_BAD_ARG;
+    // element alignment: a bf16 tensor at an odd element offset is well formed (the tile pipeline then declines it with
+    // DCT_ERR_UNSUPPORTED and the caller converts to float32)
+    const size_t ealign = c.elem == 1 ? 2 : 4;
     for (int k = 0; k < c.K; ++k) {
         if (c.views[k] == nullptr) return DCT_ERR_BAD_ARG;
-        if (!aligned(c.views[k], 4)) return DCT_ERR_MISALIGNED;
+        if (!aligned(c.views[k], ealign)) return DCT_ERR_MISALIGNED;
         if (c.mode != kFwd) {
             if (c.grads == nullptr || c.grads[k] == nullptr) return DCT_ERR_BAD_ARG;
-            if (!aligned(c.grads[k], 4)) return DCT_ERR_MISALIGNED;
+            if (!aligned(c.grads[k], ealign)) return DCT_ERR_MISALIGNED;
         }
     }
     if (c.mode != kBwd && c.sum != nullptr && c.ws == nullptr) return DCT_ERR_BAD_ARG;

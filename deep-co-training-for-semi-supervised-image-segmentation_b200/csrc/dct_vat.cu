@@ -12,6 +12,7 @@
 // 8 CTAs x 256 threads x 64 floats fall back to a two-launch path (sum of squares into the
 // workspace, then rescale; the second read is served by the 126 MB L2).
 #include <cooperative_groups.h>
+#include <cuda_bf16.h>
 
 #include "dct_common.cuh"
 
@@ -435,6 +436,29 @@ __global__ void __launch_bounds__(256) scale_if_not_one_kernel(float* grad, int6
     }
 }
 
+// bf16 twin: grad[i] = RNE_bf16(float(grad[i]) * g) -- one fp32 multiply of the stored value and one rounding, so a
+// gradient the tile pipeline wrote as RNE_bf16(v) ends as RNE_bf16(RNE_bf16(v) * g).  VEC = 8: one 16-byte word per step.
+template <int VEC>
+__global__ void __launch_bounds__(256) scale_if_not_one_bf16_kernel(__nv_bfloat16* grad, int64_t n, const float* gscalar) {
+    const float g = __ldg(gscalar);
+    if (g == 1.0f) return;  // uniform: the whole grid leaves without touching `grad`
+    for (int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * VEC; i < n; i += (int64_t)gridDim.x * blockDim.x * VEC) {
+        if constexpr (VEC == 8) {
+            uint4 u = __ldcs(reinterpret_cast<const uint4*>(grad + i));
+            uint32_t* w = &u.x;
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                float2 f = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&w[j]));
+                const __nv_bfloat162 r = __floats2bfloat162_rn(f.x * g, f.y * g);
+                w[j] = *reinterpret_cast<const uint32_t*>(&r);
+            }
+            __stcs(reinterpret_cast<uint4*>(grad + i), u);
+        } else {
+            grad[i] = __float2bfloat16_rn(__bfloat162float(grad[i]) * g);
+        }
+    }
+}
+
 static inline unsigned ew_blocks(int64_t n, int vec) {
     int64_t b = (n / vec + 255) / 256;
     if (b < 1) b = 1;
@@ -563,5 +587,15 @@ extern "C" int dct_scale_if_not_one_f32(float* grad, int64_t n, const float* gsc
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     if ((n % 4) == 0 && aligned(grad, 16)) scale_if_not_one_kernel<4><<<ew_blocks(n, 4), 256, 0, s>>>(grad, n, gscalar);
     else scale_if_not_one_kernel<1><<<ew_blocks(n, 1), 256, 0, s>>>(grad, n, gscalar);
+    return check_launch();
+}
+
+extern "C" int dct_scale_if_not_one_bf16(void* grad, int64_t n, const float* gscalar, void* stream) {
+    if (grad == nullptr || gscalar == nullptr || n < 1) return DCT_ERR_BAD_ARG;
+    if (!aligned(grad, 2) || !aligned(gscalar, 4)) return DCT_ERR_MISALIGNED;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    __nv_bfloat16* g = static_cast<__nv_bfloat16*>(grad);
+    if ((n % 8) == 0 && aligned(grad, 16)) scale_if_not_one_bf16_kernel<8><<<ew_blocks(n, 8), 256, 0, s>>>(g, n, gscalar);
+    else scale_if_not_one_bf16_kernel<1><<<ew_blocks(n, 1), 256, 0, s>>>(g, n, gscalar);
     return check_launch();
 }

@@ -154,15 +154,17 @@ def jsd_map_from_logits(logits: Sequence[torch.Tensor]) -> torch.Tensor:
 
 def _finish_grads(grads, g, dtypes):
     """Upstream scaling of gradients that were produced in the forward pass (a zero-traffic launch for the usual
-    upstream of exactly 1) and the cast back to each input's dtype (no-op unless an input was promoted)."""
+    upstream of exactly 1) and the cast back to each input's dtype (no-op unless an input was promoted).  bf16
+    gradients are scaled by the fp32 upstream with one fp32 multiply and one rounding, not by a bf16-rounded upstream."""
     h = _lib.lib()
     out = []
     for gr, dt in zip(grads, dtypes):
         if gr.dtype == torch.float32:
             _lib.check(h.dct_scale_if_not_one_f32(gr.data_ptr(), gr.numel(), g.data_ptr(),
                                                   _runtime.stream_ptr(gr.device)), "dct_scale_if_not_one_f32")
-        else:  # bf16 gradients: the upstream of `total = sup + fused` is exactly 1; anything else is a torch multiply
-            gr = gr * g.to(gr.dtype)
+        else:
+            _lib.check(h.dct_scale_if_not_one_bf16(gr.data_ptr(), gr.numel(), g.data_ptr(),
+                                                   _runtime.stream_ptr(gr.device)), "dct_scale_if_not_one_bf16")
         out.append(gr if gr.dtype == dt else gr.to(dt))
     return out
 
@@ -429,6 +431,10 @@ class _KLLogitFn(torch.autograd.Function):
             gmap, gscalar, gconst = None, g, 1.0 / ctx.n
         else:
             gmap, gscalar, gconst = g, None, 1.0
+            if ql.dtype == torch.bfloat16 and g.data_ptr() % 16 != 0:
+                # the bf16 tile pipeline reads the upstream map in 16-byte rows; autograd may hand over a slice at any
+                # 4-byte offset (e.g. of a torch.cat of the map with a tensor whose size is not a multiple of 4)
+                gmap = g.clone()
         st = _runtime.state(dev)
         fn = _lib.lib().dct_kl_logit_bf16 if ql.dtype == torch.bfloat16 else _lib.lib().dct_kl_logit_f32
         _lib.check(fn(ql.data_ptr(), pl.data_ptr(), c, b, hw, None, None, 1, _ptr(gmap), _ptr(gscalar), gconst,

@@ -196,6 +196,10 @@ DCT_API int dct_jsd_vat_kl_fwdbwd_f32(const float* const* views, int K, int C, i
 /* grad[i] *= *gscalar for i < n, skipped entirely (no memory traffic) when *gscalar == 1.0f.
  * Used by the fused loss' backward: the upstream of `total = sup + fused_loss` is exactly 1. */
 DCT_API int dct_scale_if_not_one_f32(float* grad, int64_t n, const float* gscalar, void* stream);
+/* bfloat16 twin (grad: n bf16 elements, 2-byte aligned): grad[i] = RNE_bf16(float(grad[i]) * *gscalar), one fp32
+ * multiply and one rounding; skipped entirely when *gscalar == 1.0f.  How the bf16 loss gradients below apply an
+ * upstream that their launch did not know. */
+DCT_API int dct_scale_if_not_one_bf16(void* grad, int64_t n, const float* gscalar, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * KL family of the adversarial step.
@@ -542,7 +546,13 @@ DCT_API int dct_boundary_iou_i64(const int64_t* pred, const int64_t* labels, int
  * layout), gradients are written as bfloat16 (round-to-nearest-even); ALL arithmetic is fp32 in registers and the
  * map / sum outputs, labels, counts, flags and workspace are exactly as in the _f32 functions.  Only the TMA tile
  * pipeline serves these: HW % 8 == 0, 16-byte aligned tensors, C in {2,3,4,19}, K*C <= 80; any other shape
- * returns DCT_ERR_UNSUPPORTED with nothing launched and the caller converts to float32.
+ * (a 2-byte aligned bf16 tensor at an odd element offset included) returns DCT_ERR_UNSUPPORTED with nothing launched and
+ * the caller converts to float32.
+ * Gradient contract: each bf16 gradient element is the round-to-nearest-even bf16 of the fp32 value the _f32 kernel of
+ * the same tile shape computes (gconst / gscalar / gmap applied inside, before the rounding).  The Python wrappers apply
+ * an upstream the launch did not know afterwards, with dct_scale_if_not_one_bf16: one fp32 multiply of the stored value
+ * and one more rounding.  They accept an upstream map (gmap) at any 4-byte-aligned address, handing the launch a
+ * 16-byte-aligned copy when it is not aligned so.
  * Algorithmic traffic: 2*K*C*2 (+8 with labels) B/pixel for the JSD step, 3*C*2 for the adversarial KL.
  * ------------------------------------------------------------------------------------------ */
 
