@@ -106,8 +106,9 @@ inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, siz
 
 // Developer tracing (dct_dev_trace_begin / _end, include/dct_b200.h): while a trace buffer is registered every launch of a
 // traced kernel gets the next kTraceSlots * max_ctas words of it and its CTAs stamp %globaltimer there:
-// [0] after griddepcontrol.wait, [1] / [2] kernel-specific mid points, [3] at the CTA's end.  Null in the product.
-constexpr int kTraceSlots = 4;
+// [0] after griddepcontrol.wait, [1] / [2] kernel-specific mid points, [3] at the CTA's end, [4..6] kernel-specific points
+// of the CTA's end segment (include/dct_b200.h).  Null in the product.
+constexpr int kTraceSlots = 8;
 unsigned long long* trace_next(int grid);   // dct_abi.cu; nullptr when tracing is off or the buffer is exhausted
 
 inline bool aligned(const void* p, size_t a) { return (reinterpret_cast<uintptr_t>(p) % a) == 0; }
@@ -299,101 +300,116 @@ __device__ __forceinline__ long long warp_sum(long long v) {
     return v;
 }
 
-// Called by every thread of the CTA at the end of a tile-pipeline kernel.  `out` may be null.
-// Also re-arms the workspace header (ticket, tile counter, accumulators) when the last CTA is through.
-// SUM2: a second, independent sum (acc_fx2 / nonfinite2 -> ws->fx2_* -> *out2, nullable) with the same scheme.
+// End of a tile-pipeline kernel, in two parts.  `out` / `out2` may be null.
+// Part 1, tile_grid_add: the consumer threads [0, nsum) only -- every per-thread partial lives there -- as soon as their last
+// tile is done, while the producer warp still drains its stores: block reduction behind a named barrier of the consumers,
+// then thread 0's relaxed atomic adds to the workspace accumulators.
+// Part 2, tile_grid_finish: every thread, after a CTA-wide barrier (the producer's loop -- its last pool draw, its Dice-flag
+// acquire -- is then done).  Thread 0 draws the ticket with ONE acq_rel RMW (release: this CTA's adds and the producer's
+// accesses before it; every ticket RMW extends the release sequence, so the CTA that draws the last ticket acquires every
+// CTA's adds).  That CTA publishes the sums and re-arms the header (ticket, tile counter, Dice flag, accumulators).  The
+// re-armed header needs no fence: the next launch on this workspace reads it only after this grid has completed (stream
+// order, or its griddepcontrol.wait), and completion makes every write of the grid visible.
+// SUM2: a second, independent sum (acc_fx2 / nonfinite2 -> ws->fx2_* -> *out2) with the same scheme.
 // Each thread first carries its low sum's bits above 32 into the high sum; the (lo, hi) pair then holds the same value
 // with lo < 2^32 (for a sum that a single int64 held, exactly that int64's low and high halves).
-template <bool PUB = false, bool SUM2 = false>
-__device__ __forceinline__ void tile_grid_finish(const FxAcc& acc_fx, bool nonfinite, Workspace* ws, double* out, int num_ctas,
-                                                 const PeerPub* pub = nullptr, int pub_early = 0, const FxAcc& acc_fx2 = FxAcc{},
-                                                 bool nonfinite2 = false, double* out2 = nullptr) {
+template <bool SUM2 = false>
+__device__ __forceinline__ void tile_grid_add(const FxAcc& acc_fx, bool nonfinite, Workspace* ws, bool has_out, int nsum,
+                                              const FxAcc& acc_fx2 = FxAcc{}, bool nonfinite2 = false, bool has_out2 = false) {
     if (ws == nullptr) return;
-    __shared__ long long s_lo[SUM2 ? 40 : 20], s_hi[SUM2 ? 40 : 20];  // <= 17 warps per CTA (second sum at +20)
-    __shared__ int s_nf, s_nf2;
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = (blockDim.x + 31) >> 5;
-    if (out != nullptr) {
-        if (threadIdx.x == 0) s_nf = 0;
+    __shared__ long long s_lo[SUM2 ? 40 : 20], s_hi[SUM2 ? 40 : 20];  // <= 16 consumer warps (second sum at +20)
+    __shared__ int s_nf[SUM2 ? 40 : 20];
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = nsum >> 5;
+    if (has_out) {
         long long lo = (long long)(acc_fx.lo & 0xffffffffull), hi = acc_fx.hi + (long long)(acc_fx.lo >> 32);
         lo = warp_sum(lo);
         hi = warp_sum(hi);
         const bool wnf = __any_sync(0xffffffffu, nonfinite);
-        __syncthreads();
-        if (lane == 0) { s_lo[wid] = lo; s_hi[wid] = hi; if (wnf) s_nf = 1; }
+        if (lane == 0) { s_lo[wid] = lo; s_hi[wid] = hi; s_nf[wid] = wnf; }
     }
     if constexpr (SUM2) {
-        if (out2 != nullptr) {
-            if (threadIdx.x == 0) s_nf2 = 0;
+        if (has_out2) {
             long long lo = (long long)(acc_fx2.lo & 0xffffffffull), hi = acc_fx2.hi + (long long)(acc_fx2.lo >> 32);
             lo = warp_sum(lo);
             hi = warp_sum(hi);
             const bool wnf = __any_sync(0xffffffffu, nonfinite2);
-            __syncthreads();
-            if (lane == 0) { s_lo[20 + wid] = lo; s_hi[20 + wid] = hi; if (wnf) s_nf2 = 1; }
+            if (lane == 0) { s_lo[20 + wid] = lo; s_hi[20 + wid] = hi; s_nf[20 + wid] = wnf; }
         }
     }
-    __syncthreads();
+    asm volatile("bar.sync 1, %0;" ::"r"(nsum) : "memory");
     if (threadIdx.x == 0) {
         if constexpr (SUM2) {
-            if (out2 != nullptr) {
+            if (has_out2) {
                 long long lo = 0, hi = 0;
-                for (int w = 0; w < nw; ++w) { lo += s_lo[20 + w]; hi += s_hi[20 + w]; }
+                int nf = 0;
+                for (int w = 0; w < nw; ++w) { lo += s_lo[20 + w]; hi += s_hi[20 + w]; nf |= s_nf[20 + w]; }
                 atomicAdd(&ws->fx2_lo, (unsigned long long)lo);
                 atomicAdd(reinterpret_cast<unsigned long long*>(&ws->fx2_hi), (unsigned long long)hi);
-                if (s_nf2) atomicAdd(&ws->nonfinite2, 1u);
+                if (nf) atomicAdd(&ws->nonfinite2, 1u);
+            }
+        }
+        if (has_out) {
+            long long lo = 0, hi = 0;
+            int nf = 0;
+            for (int w = 0; w < nw; ++w) { lo += s_lo[w]; hi += s_hi[w]; nf |= s_nf[w]; }
+            atomicAdd(&ws->fx_lo, (unsigned long long)lo);
+            atomicAdd(reinterpret_cast<unsigned long long*>(&ws->fx_hi), (unsigned long long)hi);
+            if (nf) atomicAdd(&ws->nonfinite, 1u);
+        }
+    }
+}
+
+// `trace_ticket` (developer tracing, null in the product): thread 0 stamps %globaltimer there once its ticket has returned.
+template <bool PUB = false, bool SUM2 = false>
+__device__ __forceinline__ void tile_grid_finish(Workspace* ws, double* out, int num_ctas, unsigned long long* trace_ticket = nullptr,
+                                                 const PeerPub* pub = nullptr, int pub_early = 0, double* out2 = nullptr) {
+    if (ws == nullptr || threadIdx.x != 0) return;
+    unsigned int ticket;
+    asm volatile("atom.acq_rel.gpu.global.add.u32 %0, [%1], 1;" : "=r"(ticket) : "l"(&ws->ticket) : "memory");
+    // (conditional on the ticket: a volatile timer read is not hoisted above the branch, so it waits for the return)
+    if (trace_ticket != nullptr && ticket != ~0u) *trace_ticket = globaltimer_ns();
+    if constexpr (PUB) {
+        // Early publication: `pub->src` holds sums that were final BEFORE this launch started (the previous step's: every
+        // kernel that wrote them completed ahead of this grid's dependency wait).  The FIRST CTA to finish pushes them to
+        // the peers while the other CTAs are still working -- the CTAs of a launch end 3-4 us apart, so the ~2 us of the
+        // publication (counter and sums read back, remote stores) sit in the launch's own tail instead of between two
+        // launches of the stream.
+        if (pub_early && ticket == 0u)
+            peer_publish(pub->src, pub->seq, __ldcg(pub->seq), pub->n, pub->rank, pub->world, pub->nslots,
+                         pub->mailbox_table, nullptr, 0.0);
+    }
+    if (ticket == (unsigned int)num_ctas - 1u) {  // last CTA: publish the sums and re-arm the header
+        // every accumulator is loaded ahead of the first store (one round trip, not one per sum)
+        unsigned long long lo2 = 0ull, lo = 0ull;
+        long long hi2 = 0ll, hi = 0ll;
+        unsigned int nf2 = 0u, nf = 0u;
+        if constexpr (SUM2) {
+            if (out2 != nullptr) { lo2 = __ldcg(&ws->fx2_lo); hi2 = __ldcg(&ws->fx2_hi); nf2 = __ldcg(&ws->nonfinite2); }
+        }
+        if (out != nullptr) { lo = __ldcg(&ws->fx_lo); hi = __ldcg(&ws->fx_hi); nf = __ldcg(&ws->nonfinite); }
+        if constexpr (SUM2) {   // (ahead of `out`: a late publication below may carry this sum as well)
+            if (out2 != nullptr) {
+                const double total = ((double)hi2 * 4294967296.0 + (double)lo2) * (1.0 / 1099511627776.0);
+                *out2 = nf2 ? __longlong_as_double(0x7ff8000000000000ll) : total;
+                ws->fx2_lo = 0ull;
+                ws->fx2_hi = 0ll;
+                ws->nonfinite2 = 0u;
             }
         }
         if (out != nullptr) {
-            long long lo = 0, hi = 0;
-            for (int w = 0; w < nw; ++w) { lo += s_lo[w]; hi += s_hi[w]; }
-            atomicAdd(&ws->fx_lo, (unsigned long long)lo);
-            atomicAdd(reinterpret_cast<unsigned long long*>(&ws->fx_hi), (unsigned long long)hi);
-            if (s_nf) atomicAdd(&ws->nonfinite, 1u);
+            const double total = ((double)hi * 4294967296.0 + (double)lo) * (1.0 / 1099511627776.0);
+            const double fin = nf ? __longlong_as_double(0x7ff8000000000000ll) : total;
+            *out = fin;
+            if constexpr (PUB)  // the step's sums -> every rank's mailbox (NVLink)
+                if (!pub_early) peer_publish(pub->src, pub->seq, __ldcg(pub->seq), pub->n, pub->rank, pub->world, pub->nslots,
+                             pub->mailbox_table, out, fin);
+            ws->fx_lo = 0ull;
+            ws->fx_hi = 0ll;
+            ws->nonfinite = 0u;
         }
-        __threadfence();
-        const unsigned int ticket = atomicAdd(&ws->ticket, 1u);
-        if constexpr (PUB) {
-            // Early publication: `pub->src` holds sums that were final BEFORE this launch started (the previous step's: every
-            // kernel that wrote them completed ahead of this grid's dependency wait).  The FIRST CTA to finish pushes them to
-            // the peers while the other CTAs are still working -- the CTAs of a launch end 3-4 us apart, so the ~2 us of the
-            // publication (counter and sums read back, remote stores) sit in the launch's own tail instead of between two
-            // launches of the stream.
-            if (pub_early && ticket == 0u)
-                peer_publish(pub->src, pub->seq, __ldcg(pub->seq), pub->n, pub->rank, pub->world, pub->nslots,
-                             pub->mailbox_table, nullptr, 0.0);
-        }
-        if (ticket == (unsigned int)num_ctas - 1u) {  // last CTA: publish the sum and re-arm the header
-            __threadfence();
-            if constexpr (SUM2) {   // (ahead of `out`: a late publication below may carry this sum as well)
-                if (out2 != nullptr) {
-                    const unsigned long long lo = __ldcg(&ws->fx2_lo);
-                    const long long hi = __ldcg(&ws->fx2_hi);
-                    const double total = ((double)hi * 4294967296.0 + (double)lo) * (1.0 / 1099511627776.0);
-                    *out2 = __ldcg(&ws->nonfinite2) ? __longlong_as_double(0x7ff8000000000000ll) : total;
-                    ws->fx2_lo = 0ull;
-                    ws->fx2_hi = 0ll;
-                    ws->nonfinite2 = 0u;
-                }
-            }
-            if (out != nullptr) {
-                const unsigned long long lo = __ldcg(&ws->fx_lo);
-                const long long hi = __ldcg(&ws->fx_hi);
-                const unsigned int nf = __ldcg(&ws->nonfinite);
-                const double total = ((double)hi * 4294967296.0 + (double)lo) * (1.0 / 1099511627776.0);
-                const double fin = nf ? __longlong_as_double(0x7ff8000000000000ll) : total;
-                *out = fin;
-                if constexpr (PUB)  // the step's sums -> every rank's mailbox (NVLink)
-                    if (!pub_early) peer_publish(pub->src, pub->seq, __ldcg(pub->seq), pub->n, pub->rank, pub->world, pub->nslots,
-                                 pub->mailbox_table, out, fin);
-                ws->fx_lo = 0ull;
-                ws->fx_hi = 0ll;
-                ws->nonfinite = 0u;
-            }
-            ws->tile_counter = 0u;
-            ws->counts_zeroed = 0u;
-            __threadfence();
-            ws->ticket = 0u;
-        }
+        ws->tile_counter = 0u;
+        ws->counts_zeroed = 0u;
+        ws->ticket = 0u;
     }
 }
 

@@ -124,7 +124,8 @@ struct TileArgs {
     int pool_div;                  // developer switch (tools/kbench_*.cu): the tail pool is 1/pool_div of every CTA's range (0 = default 5)
     int prefetch;                  // tiles of this CTA's range whose rows are prefetched into L2 before the dependency wait
     int force_static;              // developer switch (tools/kbench_tile.cu): 1 = no tail pool (purely static contiguous ranges) even with a workspace
-    unsigned long long* trace;     // developer tracing: kTraceSlots words per CTA (start, first tile landed, -, end) in ns; null in the product
+    unsigned long long* trace;     // developer tracing: kTraceSlots words per CTA (start, first tile landed, -, end, tiles done,
+                                   // stores read out, ticket drawn) in ns; null in the product
     double* sum2;                  // SUM2 ops: grid sum of the second per-pixel value (nullable)
 };
 
@@ -535,10 +536,14 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
             }
             __syncwarp();
         }
+        if (a.trace != nullptr && lane == 0) a.trace[kTraceSlots * blockIdx.x + 4] = globaltimer_ns();   // tiles done
         if constexpr (NOUT > 0) {
-            if (lane == 0) tma::bulk_wait_all<0>();
+            // the CTA may exit once its stores have been read out of shared memory; their writes are complete and visible
+            // when the grid is (what the next grid's griddepcontrol.wait / stream order waits for)
+            if (lane == 0) tma::bulk_wait_read<0>();
         }
         if (a.trace != nullptr && lane == 0) {   // developer tracing: tiles this CTA processed, pool draws among them, its SM
+            a.trace[kTraceSlots * blockIdx.x + 5] = globaltimer_ns();
             unsigned int smid;
             asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
             const int pool_draws = draws > my_static ? draws - my_static : 0;
@@ -766,6 +771,12 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
                 if (lane == 0 && nbad_label != 0 && a.flags != nullptr) atomicAdd(&a.flags[DCT_FLAG_LABEL], nbad_label);
             }
         }
+        // this CTA's share of the loss sums goes to the workspace accumulators while the producer warp drains its stores
+        if constexpr (SUM2)
+            tile_grid_add<true>(acc_fx, nonfinite, a.ws, Op::HAS_MAP && a.sum != nullptr, CTHREADS, acc_fx2, nonfinite2,
+                                a.sum2 != nullptr);
+        else
+            tile_grid_add(acc_fx, nonfinite, a.ws, Op::HAS_MAP && a.sum != nullptr, CTHREADS);
     }
     // this CTA's tiles are done: the next kernel in the stream may be scheduled onto the SMs that drain first and run
     // its prologue; its pdl_wait() still holds it until this whole grid (epilogue below included) has completed
@@ -784,11 +795,10 @@ __global__ void __launch_bounds__(NCW * 32 + 32, MINB) tile_kernel(const TileArg
             if (bad) atomicAdd(&a.flags[DCT_FLAG_SIMPLEX], 1);
         }
     }
-    if constexpr (SUM2)
-        tile_grid_finish<PUB, true>(acc_fx, nonfinite, a.ws, Op::HAS_MAP ? a.sum : nullptr, gridDim.x, &a.pub, a.pub_early,
-                                    acc_fx2, nonfinite2, a.sum2);
-    else
-        tile_grid_finish<PUB>(acc_fx, nonfinite, a.ws, Op::HAS_MAP ? a.sum : nullptr, gridDim.x, &a.pub, a.pub_early);
+    __syncthreads();   // the producer's loop and thread 0's accumulator adds come before the ticket
+    unsigned long long* const trace_ticket = a.trace != nullptr ? a.trace + kTraceSlots * blockIdx.x + 6 : nullptr;
+    tile_grid_finish<PUB, SUM2>(a.ws, Op::HAS_MAP ? a.sum : nullptr, gridDim.x, trace_ticket, &a.pub, a.pub_early,
+                                SUM2 ? a.sum2 : nullptr);
     if (a.trace != nullptr && tid == 0) a.trace[kTraceSlots * blockIdx.x + 3] = globaltimer_ns();
 }
 

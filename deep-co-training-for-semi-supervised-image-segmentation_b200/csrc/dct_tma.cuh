@@ -66,10 +66,6 @@ template <int N>
 __device__ __forceinline__ void bulk_wait_read() {
     asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory");
 }
-template <int N>
-__device__ __forceinline__ void bulk_wait_all() {
-    asm volatile("cp.async.bulk.wait_group %0;" ::"n"(N) : "memory");
-}
 
 }  // namespace tma
 }  // namespace dct

@@ -139,6 +139,9 @@ l2_cluster_kernel(const L2Args a) {
 #pragma unroll
     for (int i = 0; i < CL / 4; ++i)   // lane l reads warp (l & 7) of CTAs (l >> 3) + 4 i, in a fixed order
         t += *cluster.map_shared_rank(&s_wsum[0][lane & 7], 4 * i + (lane >> 3));
+    // No CTA may exit (and free s_wsum) while a peer can still be reading it: this thread's peer reads are done -- it
+    // arrives here and waits at the exit, by when the stores below have normally given every peer time to arrive.
+    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
     t = warp_sum(t);
     if (a.trace != nullptr && threadIdx.x == 0) a.trace[kTraceSlots * blockIdx.x + 2] = globaltimer_ns();
     const L2Scale sc = l2_scales(t, a.passes, a.scale);
@@ -167,8 +170,9 @@ l2_cluster_kernel(const L2Args a) {
             }
         }
     }
+    if (a.trace != nullptr && threadIdx.x == 0) a.trace[kTraceSlots * blockIdx.x + 4] = globaltimer_ns();   // stores issued
     pdl_launch_dependents();
-    cluster.sync();  // no CTA may exit (and free s_wsum) while a peer can still be reading it
+    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
     if (a.trace != nullptr && threadIdx.x == 0) a.trace[kTraceSlots * blockIdx.x + 3] = globaltimer_ns();
 }
 

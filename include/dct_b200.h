@@ -580,10 +580,12 @@ DCT_API int dct_ce_fwdbwd_bf16(const void* logits, const int64_t* labels, int C,
 
 /* ------------------------------------------------------------------------------------------
  * Developer tracing (tools/step_trace.py; not used by the product).  Between _begin and _end every launch of the tile
- * pipeline and of the perturbation normalisation takes the next 4 * max_ctas uint64 words of `buf` (device memory, zeroed
+ * pipeline and of the perturbation normalisation takes the next 8 * max_ctas uint64 words of `buf` (device memory, zeroed
  * by the caller) and each of its CTAs stamps %globaltimer (ns) there: [0] after the programmatic-dependency wait,
  * [1] first tile landed / after the first per-sample exchange, [2] tile pipeline: (SM id << 32) | (pool draws << 16) | tiles
- * processed; normalisation: after the last exchange, [3] at its end.  _end returns the number of launches recorded.
+ * processed; normalisation: after the last exchange, [3] at its end.  End segments: tile pipeline [4] tiles done (last
+ * store issued), [5] stores read out of shared memory, [6] grid-sum ticket drawn; cluster normalisation [4] stores issued.
+ * _end returns the number of launches recorded.
  * Process-global state: do not trace from two host threads at once.
  * ------------------------------------------------------------------------------------------ */
 DCT_API int dct_dev_trace_begin(void* buf, int max_ctas, int max_launches);
